@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        # the reference algorithm (oracle port) on the host CPU
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's outputs as DIR/<name>.npy
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): PROOF/TEAM
 head fwd+bwd, 10 incremental tasks (C=20 classes, P=100 prompts, L=123 tokens), batch 1024
@@ -34,6 +35,7 @@ METRIC = "team_head_fwd_bwd_samples_per_sec"
 UNIT = "samples/s"
 NUM_TASKS = 10
 ROT = 64                         # rotating input slots: 64 x (2 x 2 MiB + cotangents 8 MiB) >> 126 MB L2
+DUMP_BYTES = 64 << 20            # --dump-outputs: size of all written arrays together
 
 
 def parse():
@@ -57,7 +59,16 @@ def parse():
     ap.add_argument("--comm", default="peer", choices=["peer", "nccl", "nccl-buckets"],
                     help="N>1 gradient exchange: own NVLink peer-memory kernel inside the step graph (default), one NCCL "
                          "all-reduce after the step, or three NCCL buckets overlapped with the backward")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed on rank 0 (feature outputs, "
+                         "classification logits and argmax, parameter gradients) as DIR/<name>.npy, so that two builds "
+                         "can be compared on the same seeded inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "team":
+        ap.error("--dump-outputs needs --impl team")
+    return a
 
 
 def ncu_dram_bytes_per_launch(kernel_prefix: str):
@@ -151,11 +162,45 @@ def workload_config(tasks: int, batch: int, world: int) -> dict:
             "alg_flops_per_sample_survey": 55.07e6 if tasks == 10 else None}
 
 
+def last_step_outputs(runner, budget: int = DUMP_BYTES) -> dict:
+    """Device copies of what the caller of `runner.step` receives from its last step: the four [B,512] feature outputs,
+    the classification logits and argmax (as float64) and the gradient of every trainable parameter.  When all of it would
+    exceed `budget` bytes, the per-sample arrays keep the same fixed, seeded sample of rows, listed in `sample_rows`.
+    Enqueued on the current stream, so later steps on that stream cannot overwrite them."""
+    import torch
+    rows = {"out_image": runner.outs[0], "out_text": runner.outs[1], "out_state": runner.outs[2],
+            "out_proto": runner.outs[3], "cls_logits": runner.logits, "cls_argmax": runner.argmax.double()}
+    grads = {"grad_" + k: v for k, v in runner.grad_views.items()}
+    fixed = sum(v.numel() * v.element_size() for v in grads.values())
+    per_row = sum(v[0].numel() * v.element_size() for v in rows.values())
+    if fixed + runner.B * per_row > budget:
+        k = (budget - fixed) // (per_row + 8)
+        if k < 1:
+            raise ValueError(f"--dump-outputs: the gradients alone ({fixed / 2**20:.1f} MiB) leave no room for a sample of "
+                             f"rows within {budget / 2**20:.0f} MiB")
+        idx = torch.randperm(runner.B, generator=torch.Generator().manual_seed(0))[:k].sort().values
+        rows = {n: v.index_select(0, idx.to(v.device)) for n, v in rows.items()}
+        rows["sample_rows"] = idx.double()
+    return {n: v.detach().clone() for n, v in {**rows, **grads}.items()}
+
+
+def write_outputs(arrays: dict, out_dir: str):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        v = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+        total += v.nbytes
+    print(f"[bench] wrote {len(arrays)} arrays of the last timed step ({total / 2**20:.1f} MiB) to {out_dir}",
+          file=sys.stderr, flush=True)
+
+
 def cpu_reference_step_fn(tasks: int, batch: int, nsets: int = 4):
     """One head step on the host CPU, same step definition as the GPU arm (no-grad classification logits +
     forward_tri_modal + VJP with fixed cotangents).  kind "reference": the UNMODIFIED reference modules
-    (utils/inc_net.py Proof_Net, models/proof.py Learner.forward_for_classification) loaded from baseline/_ref
-    (or /root/reference) through oracle/ref_loader.py, fake CLIP = identity on the 512-d features, eval mode.
+    (utils/inc_net.py Proof_Net, models/proof.py Learner.forward_for_classification) loaded from $TEAM_REFERENCE_ROOT
+    or oracle/_ref through oracle/ref_loader.py, fake CLIP = identity on the 512-d features, eval mode.
     kind "port": the oracle restatement (only when the reference tree is not there)."""
     import types
     import torch
@@ -168,7 +213,7 @@ def cpu_reference_step_fn(tasks: int, batch: int, nsets: int = 4):
     sets = [(synth.make_batch(batch, C, step=i), synth.make_cotangents(batch, step=i)) for i in range(nsets)]
     if ref_loader.available():
         net = ref_loader.build_reference_net(params, protos)
-        from models.proof import Learner                     # reference module (baseline/_ref)
+        from models.proof import Learner                     # reference module (oracle/ref_loader.py)
         fake = types.SimpleNamespace(_network=net, _device=torch.device("cpu"))
         sd = dict(net.named_parameters())
         train = [sd[n] for n in names]
@@ -211,7 +256,7 @@ def time_cpu(tasks: int, batch: int, steps: int, warmup: int, budget_s: float = 
         if budget_s > 0 and time.perf_counter() - t0 > budget_s:
             break
     dt = (time.perf_counter() - t0) / max(done, 1)
-    what = ("the unmodified reference (baseline/_ref: utils/inc_net.py Proof_Net.forward_tri_modal + models/proof.py "
+    what = ("the unmodified reference (utils/inc_net.py Proof_Net.forward_tri_modal + models/proof.py "
             "forward_for_classification + autograd), fake CLIP = identity" if kind == "reference"
             else "oracle port of the reference head")
     return {"value": batch / dt, "unit": UNIT, "cores": cores, "kind": kind,
@@ -225,8 +270,8 @@ def run_reference(a):
         return
     world = int(os.environ.get("WORLD_SIZE", "1"))
     warm = max(1, a.warmup)
-    # the same batch as the GPU arm (B per GPU); the whole run is bounded to a few minutes
-    cb, dt, done = time_cpu(a.tasks, a.batch, a.steps, warm, budget_s=240.0)
+    # the same batch as the GPU arm (B per GPU), exactly --steps timed steps
+    cb, dt, done = time_cpu(a.tasks, a.batch, a.steps, warm)
     # BASELINE configs[0], exactly: B=64, T=1, CPU fp32 (the reference's own CPU-runnable case)
     c1, dt1, n1 = time_cpu(1, 64, 10, 2, budget_s=30.0)
     line = {"metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
@@ -363,12 +408,15 @@ def run_team(a):
         e1.record(stream)
         barrier()
         ms = e0.elapsed_time(e1)
+        dump = last_step_outputs(runner) if a.dump_outputs and rank == 0 else None
         # the timed region of K steps can be shorter than one nvidia-smi period: keep replaying the same
         # steps (untimed) for 0.3 s so that the sampler sees the load the timed region ran under
         load(0.3)
         clocks = sampler.stop() if rank == 0 else None
         if clocks is not None:
             clocks["window"] = "timed region + 0.3 s of the same replayed steps (25 ms nvidia-smi period)"
+    if dump is not None:
+        write_outputs(dump, a.dump_outputs)
     if world > 1:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -2,7 +2,7 @@
 
     python oracle/gen_golden.py            # writes tests/golden/*.npz
 
-Imports ``/root/reference`` through ``oracle/ref_loader.py`` (stubbed timm / matplotlib /
+Imports the original project (``$TEAM_REFERENCE_ROOT`` or ``oracle/_ref``) through ``oracle/ref_loader.py`` (stubbed timm / matplotlib /
 open_clip), feeds it the seeded tensors of ``oracle/synth.py`` and stores the reference's
 outputs.  Inputs and parameters are NOT stored: tests rebuild them from the seeds in
 ``CASES`` (``oracle/cases.py``).  Large gradients are stored as a row subsample

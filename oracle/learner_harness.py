@@ -4,7 +4,7 @@
 Used twice with the same seeds:
   * `oracle/gen_golden.py` (build container, CPU): the reference learner with the reference `Proof_Net` and
     `AdaptiveStateDistanceMatrix` -> `tests/golden/learner_2tasks.npz`;
-  * `tests/test_gpu_learner_dropin.py` (GPU box, reference tree = `baseline/_ref`): the same learner code with the two
+  * `tests/test_gpu_learner_dropin.py` (reference tree = `$TEAM_REFERENCE_ROOT` or `oracle/_ref`): the same learner code with the two
     classes swapped for `team_b200.inc_net.Proof_Net` / `AdaptiveStateDistanceMatrix` - the two import lines
     `models/proof.py:8` and `:202` (INTEGRATION.md) - on `cuda:0`.
 SURVEY App. D: CLIP is the identity on pre-computed 512-d features ("images" ARE feature rows), the tokenizer maps a
