@@ -465,8 +465,6 @@ int team_gemm_bf16_group(const team_gemm_desc* descs, int32_t n, void* workspace
  * input buffers of a captured step (train.TrainStep.load): replaces four device-to-device copies between graph replays. */
 int team_copy_batch(const float* image, const float* text, const int64_t* state_ids, const int64_t* labels, int64_t batch,
                     float* d_image, float* d_text, int64_t* d_state_ids, int64_t* d_labels, void* stream);
-/* programmatic dependent launch for the library's kernels (default: env TEAM_PDL, else off) */
-int team_set_pdl(int on);
 /* debugging aid: if buf != NULL (32 x 1024 x 16 uint64) every GEMM CTA writes globaltimer stamps of its phases into the slot of its launch (tools/wave_stamps.py) */
 int team_gemm_debug_stamps(void* buf);
 /* fp32 [rows,cols] -> bf16 hi (and optional lo residual) */

@@ -116,8 +116,6 @@ def _declare(lib):
     if hasattr(lib, "team_gemm_bf16_group"):
         lib.team_gemm_bf16_group.restype = i32
         lib.team_gemm_bf16_group.argtypes = [C.POINTER(GemmDesc), C.c_int32, vp, sz, vp]
-        lib.team_set_pdl.restype = i32
-        lib.team_set_pdl.argtypes = [i32]
     if hasattr(lib, "team_gemm_bf16_nt"):
         lib.team_gemm_bf16_nt.restype = i32
         lib.team_gemm_bf16_nt.argtypes = [i64, i64, i64, vp, i64, vp, i64, vp, i64, vp]

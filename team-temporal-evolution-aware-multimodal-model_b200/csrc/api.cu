@@ -1,21 +1,11 @@
 // Error plumbing + device check for the C ABI (include/team_b200.h).
 #include <stdarg.h>
-#include <stdlib.h>
 #include <atomic>
 #include "common.cuh"
 
 namespace team {
 static std::atomic<long long> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
-static int g_pdl_state = -1;          // -1: read TEAM_PDL on first use (default on)
-bool pdl_enabled() {
-    if (g_pdl_state < 0) {
-        const char* e = getenv("TEAM_PDL");
-        g_pdl_state = (e != nullptr && e[0] == '0') ? 0 : 1;
-    }
-    return g_pdl_state != 0;
-}
-void pdl_set(bool on) { g_pdl_state = on ? 1 : 0; }
 static thread_local char g_err[512] = "";
 void set_error(const char* fmt, ...) {
     va_list ap;

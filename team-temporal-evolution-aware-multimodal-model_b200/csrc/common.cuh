@@ -43,8 +43,6 @@ void count_launch();
 // prologue (barrier init, TMEM alloc, parameter loads) of kernel N+1 overlap the tail of kernel N.
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-bool pdl_enabled();
-void pdl_set(bool on);
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t st, Args&&... args) {
@@ -57,7 +55,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned 
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<Args&&>(args)...);
 }
 // launch + count + status check (the kernel must start with pdl_trigger(); pdl_wait();)

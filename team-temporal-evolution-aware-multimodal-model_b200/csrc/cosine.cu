@@ -376,7 +376,7 @@ extern "C" int team_cosine_logits(const void* x, int x_dtype, int64_t n_rows, co
     // Small inputs (the classification logits of a 1 024-sample step): the tensor-pipe kernel is its prologue there (every CTA
     // normalises and hi/lo-splits the whole class table: 19 us on 8 CTAs at 1 024 rows, on the forward's critical path beside
     // the table rows) - the CUDA-core kernel takes 8 us on 64 CTAs.  From 8 192 rows the streaming rate decides.
-    if (getenv("TEAM_COSINE_V1") == nullptr && n_rows > 8192) {          // tensor-pipe contraction (3xTF32), see cosine_mma_kernel
+    if (n_rows > 8192) {          // tensor-pipe contraction (3xTF32), see cosine_mma_kernel
         const int nt = (int)((((num_classes < COS_CCHUNK ? num_classes : COS_CCHUNK)) + 7) / 8);
         const int64_t tiles = (n_rows + 15) / 16;
         int64_t gx2 = (tiles + COS2_WARPS - 1) / COS2_WARPS;

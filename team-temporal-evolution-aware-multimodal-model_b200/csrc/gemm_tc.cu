@@ -72,7 +72,6 @@ struct TcGroup {
     int stages;
     int cluster;                 // CTAs per cluster (1, 2, 4 or 8) = largest split count of the group
     unsigned long long* dbg;     // optional [cta][16] globaltimer stamps (tools/gemm_probe.py), else null
-    int diag;                    // TEAM_GEMM_DIAG (timing experiments only, results invalid): 1 = no global stores, 2 = no k-loop, 4 = no epilogue loop, 8 = no TMEM -> smem copy
 };
 __device__ __forceinline__ unsigned long long gtime() {
     unsigned long long t;
@@ -197,7 +196,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
     const int nkb0 = P.s[0].nkb;
     const int nkb = nkb0 + P.s[1].nkb;
     const int kb_begin = split * P.kb_per_split;
-    const int kb_end = (g.diag & 2) ? kb_begin : min(nkb, kb_begin + P.kb_per_split);
+    const int kb_end = min(nkb, kb_begin + P.kb_per_split);
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < nstages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
@@ -284,27 +283,25 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
     // TMEM -> padded smem tile (the operand ring is idle now); thread = one accumulator row
     float* stg = reinterpret_cast<float*>(smem);
     const int sld = bn + 4;
-    if (!(g.diag & 8)) {
-        float* my = stg + (size_t)(warp * 32 + lane) * sld;
-        const uint32_t tbase = tmem_base + ((uint32_t)(warp * 32) << 16);
-        int c = 0;
-        for (; c + 32 <= bn; c += 32) {              // two 16-column loads in flight per wait
-            uint32_t r[32];
-            tmem_ld16_nowait(tbase + (uint32_t)c, r);
-            tmem_ld16_nowait(tbase + (uint32_t)(c + 16), r + 16);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    float* my = stg + (size_t)(warp * 32 + lane) * sld;
+    const uint32_t tbase = tmem_base + ((uint32_t)(warp * 32) << 16);
+    int c = 0;
+    for (; c + 32 <= bn; c += 32) {              // two 16-column loads in flight per wait
+        uint32_t r[32];
+        tmem_ld16_nowait(tbase + (uint32_t)c, r);
+        tmem_ld16_nowait(tbase + (uint32_t)(c + 16), r + 16);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
-            for (int i = 0; i < 32; i += 4)
-                *reinterpret_cast<float4*>(my + c + i) = make_float4(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), __uint_as_float(r[i + 2]), __uint_as_float(r[i + 3]));
-        }
-        if (c < bn) {
-            uint32_t r[16];
-            tmem_ld16_nowait(tbase + (uint32_t)c, r);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        for (int i = 0; i < 32; i += 4)
+            *reinterpret_cast<float4*>(my + c + i) = make_float4(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), __uint_as_float(r[i + 2]), __uint_as_float(r[i + 3]));
+    }
+    if (c < bn) {
+        uint32_t r[16];
+        tmem_ld16_nowait(tbase + (uint32_t)c, r);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
-            for (int i = 0; i < 16; i += 4)
-                *reinterpret_cast<float4*>(my + c + i) = make_float4(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), __uint_as_float(r[i + 2]), __uint_as_float(r[i + 3]));
-        }
+        for (int i = 0; i < 16; i += 4)
+            *reinterpret_cast<float4*>(my + c + i) = make_float4(__uint_as_float(r[i]), __uint_as_float(r[i + 1]), __uint_as_float(r[i + 2]), __uint_as_float(r[i + 3]));
     }
     if (threadIdx.x == 64) TC_STAMP(8);
     // split-K: every CTA of the tile publishes its partial (cluster barrier), then owns rows [row0, row0 + nrow)
@@ -322,96 +319,94 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
         __syncthreads();
     }
     if (threadIdx.x == 64) TC_STAMP(9);
-    if (!(g.diag & 4)) {
-        const int M = P.M, N = P.N;
-        float* const C = (g.diag & 1) ? nullptr : P.C;
-        __nv_bfloat16* const Cb = (g.diag & 1) ? nullptr : P.Cb;
-        const long long ldc = P.ldc, ldcb = P.ldcb;
-        const bool vec_ok = (N % 4 == 0) && (C == nullptr || ((ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(C) & 15) == 0))) &&
-                            (Cb == nullptr || ((ldcb % 4 == 0) && ((reinterpret_cast<uintptr_t>(Cb) & 7) == 0)));
-        const float alpha = P.alpha, beta = P.beta;
-        const bool acc_c = beta != 0.f && C != nullptr;
-        const bool cb_f16 = P.cb_f16 != 0;
-        const float* bias = P.bias;
-        // thread -> (row offset r_off, float4 column c4): lanes run along the columns, rpp rows per pass
-        const int lpr = bn >> 2;                                   // float4 columns per row (4..32)
-        const int rpp = TC_THREADS / lpr;                          // rows per pass (4..32)
-        const int r_off = (int)threadIdx.x / lpr, c4 = (int)threadIdx.x - r_off * lpr;
-        const int col = n0 + 4 * c4;
-        if (r_off < rpp && col < N) {
-            float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (bias != nullptr) {
-                bv.x = __ldg(bias + col);
-                if (col + 1 < N) bv.y = __ldg(bias + col + 1);
-                if (col + 2 < N) bv.z = __ldg(bias + col + 2);
-                if (col + 3 < N) bv.w = __ldg(bias + col + 3);
-            }
-            // rows of this thread: row0 + r_off + q * rpp, q = 0 .. nq-1, clipped to the slice and to M
-            int nq = (nrow - r_off + rpp - 1) / rpp;
-            {
-                const int left = M - (m0 + row0 + r_off);
-                const int cap = left <= 0 ? 0 : (left + rpp - 1) / rpp;
-                if (cap < nq) nq = cap;
-            }
-            const uint32_t stg_addr = smem_u32(stg);
-            const uint32_t off0 = (uint32_t)(((row0 + r_off) * sld + 4 * c4) * 4), ostep = (uint32_t)(rpp * sld * 4);
-            const unsigned char* lp = reinterpret_cast<const unsigned char*>(stg) + off0;
-            uint32_t rbase[TC_MAX_SPLITS];
+    const int M = P.M, N = P.N;
+    float* const C = P.C;
+    __nv_bfloat16* const Cb = P.Cb;
+    const long long ldc = P.ldc, ldcb = P.ldcb;
+    const bool vec_ok = (N % 4 == 0) && (C == nullptr || ((ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(C) & 15) == 0))) &&
+                        (Cb == nullptr || ((ldcb % 4 == 0) && ((reinterpret_cast<uintptr_t>(Cb) & 7) == 0)));
+    const float alpha = P.alpha, beta = P.beta;
+    const bool acc_c = beta != 0.f && C != nullptr;
+    const bool cb_f16 = P.cb_f16 != 0;
+    const float* bias = P.bias;
+    // thread -> (row offset r_off, float4 column c4): lanes run along the columns, rpp rows per pass
+    const int lpr = bn >> 2;                                   // float4 columns per row (4..32)
+    const int rpp = TC_THREADS / lpr;                          // rows per pass (4..32)
+    const int r_off = (int)threadIdx.x / lpr, c4 = (int)threadIdx.x - r_off * lpr;
+    const int col = n0 + 4 * c4;
+    if (r_off < rpp && col < N) {
+        float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (bias != nullptr) {
+            bv.x = __ldg(bias + col);
+            if (col + 1 < N) bv.y = __ldg(bias + col + 1);
+            if (col + 2 < N) bv.z = __ldg(bias + col + 2);
+            if (col + 3 < N) bv.w = __ldg(bias + col + 3);
+        }
+        // rows of this thread: row0 + r_off + q * rpp, q = 0 .. nq-1, clipped to the slice and to M
+        int nq = (nrow - r_off + rpp - 1) / rpp;
+        {
+            const int left = M - (m0 + row0 + r_off);
+            const int cap = left <= 0 ? 0 : (left + rpp - 1) / rpp;
+            if (cap < nq) nq = cap;
+        }
+        const uint32_t stg_addr = smem_u32(stg);
+        const uint32_t off0 = (uint32_t)(((row0 + r_off) * sld + 4 * c4) * 4), ostep = (uint32_t)(rpp * sld * 4);
+        const unsigned char* lp = reinterpret_cast<const unsigned char*>(stg) + off0;
+        uint32_t rbase[TC_MAX_SPLITS];
 #pragma unroll
-            for (int z = 0; z < TC_MAX_SPLITS; ++z) rbase[z] = z < splits ? map_to_cta(stg_addr + off0, rank0 + (uint32_t)z) : 0u;
-            float* cp = C != nullptr ? C + (long long)(m0 + row0 + r_off) * ldc + col : nullptr;
-            __nv_bfloat16* bp = Cb != nullptr ? Cb + (long long)(m0 + row0 + r_off) * ldcb + col : nullptr;
-            const long long cstep = (long long)rpp * ldc, bstep = (long long)rpp * ldcb;
-            constexpr int UN = 8;                                  // rows in flight per thread
-            for (int q0 = 0; q0 < nq; q0 += UN) {
-                float4 v[UN], o[UN];
-                if (splits == 1) {
+        for (int z = 0; z < TC_MAX_SPLITS; ++z) rbase[z] = z < splits ? map_to_cta(stg_addr + off0, rank0 + (uint32_t)z) : 0u;
+        float* cp = C != nullptr ? C + (long long)(m0 + row0 + r_off) * ldc + col : nullptr;
+        __nv_bfloat16* bp = Cb != nullptr ? Cb + (long long)(m0 + row0 + r_off) * ldcb + col : nullptr;
+        const long long cstep = (long long)rpp * ldc, bstep = (long long)rpp * ldcb;
+        constexpr int UN = 8;                                  // rows in flight per thread
+        for (int q0 = 0; q0 < nq; q0 += UN) {
+            float4 v[UN], o[UN];
+            if (splits == 1) {
+#pragma unroll
+                for (int j = 0; j < UN; ++j)
+                    if (q0 + j < nq) v[j] = *reinterpret_cast<const float4*>(lp + (size_t)(q0 + j) * ostep);
+            } else {
+#pragma unroll
+                for (int j = 0; j < UN; ++j)
+                    if (q0 + j < nq) v[j] = ld_cluster_f4(rbase[0] + (uint32_t)(q0 + j) * ostep);
+#pragma unroll
+                for (int z = 1; z < TC_MAX_SPLITS; ++z) {      // fixed order: deterministic
+                    if (z >= splits) break;
+                    float4 a[UN];
 #pragma unroll
                     for (int j = 0; j < UN; ++j)
-                        if (q0 + j < nq) v[j] = *reinterpret_cast<const float4*>(lp + (size_t)(q0 + j) * ostep);
+                        if (q0 + j < nq) a[j] = ld_cluster_f4(rbase[z] + (uint32_t)(q0 + j) * ostep);
+#pragma unroll
+                    for (int j = 0; j < UN; ++j)
+                        if (q0 + j < nq) { v[j].x += a[j].x; v[j].y += a[j].y; v[j].z += a[j].z; v[j].w += a[j].w; }
+                }
+            }
+            if (acc_c && vec_ok) {
+#pragma unroll
+                for (int j = 0; j < UN; ++j)
+                    if (q0 + j < nq) o[j] = *reinterpret_cast<const float4*>(cp + (q0 + j) * cstep);
+            }
+#pragma unroll
+            for (int j = 0; j < UN; ++j) {
+                if (q0 + j >= nq) continue;
+                float4 x = make_float4(fmaf(alpha, v[j].x, bv.x), fmaf(alpha, v[j].y, bv.y), fmaf(alpha, v[j].z, bv.z), fmaf(alpha, v[j].w, bv.w));
+                if (vec_ok) {
+                    if (acc_c) { x.x = fmaf(beta, o[j].x, x.x); x.y = fmaf(beta, o[j].y, x.y); x.z = fmaf(beta, o[j].z, x.z); x.w = fmaf(beta, o[j].w, x.w); }
+                    if (cp != nullptr) *reinterpret_cast<float4*>(cp + (q0 + j) * cstep) = x;
+                    if (bp != nullptr) *reinterpret_cast<uint2*>(bp + (q0 + j) * bstep) = pack_h16x4(x, cb_f16);
                 } else {
+                    // ragged N / unaligned outputs: element-wise with guards
+                    const float xs[4] = {x.x, x.y, x.z, x.w};
 #pragma unroll
-                    for (int j = 0; j < UN; ++j)
-                        if (q0 + j < nq) v[j] = ld_cluster_f4(rbase[0] + (uint32_t)(q0 + j) * ostep);
-#pragma unroll
-                    for (int z = 1; z < TC_MAX_SPLITS; ++z) {      // fixed order: deterministic
-                        if (z >= splits) break;
-                        float4 a[UN];
-#pragma unroll
-                        for (int j = 0; j < UN; ++j)
-                            if (q0 + j < nq) a[j] = ld_cluster_f4(rbase[z] + (uint32_t)(q0 + j) * ostep);
-#pragma unroll
-                        for (int j = 0; j < UN; ++j)
-                            if (q0 + j < nq) { v[j].x += a[j].x; v[j].y += a[j].y; v[j].z += a[j].z; v[j].w += a[j].w; }
-                    }
-                }
-                if (acc_c && vec_ok) {
-#pragma unroll
-                    for (int j = 0; j < UN; ++j)
-                        if (q0 + j < nq) o[j] = *reinterpret_cast<const float4*>(cp + (q0 + j) * cstep);
-                }
-#pragma unroll
-                for (int j = 0; j < UN; ++j) {
-                    if (q0 + j >= nq) continue;
-                    float4 x = make_float4(fmaf(alpha, v[j].x, bv.x), fmaf(alpha, v[j].y, bv.y), fmaf(alpha, v[j].z, bv.z), fmaf(alpha, v[j].w, bv.w));
-                    if (vec_ok) {
-                        if (acc_c) { x.x = fmaf(beta, o[j].x, x.x); x.y = fmaf(beta, o[j].y, x.y); x.z = fmaf(beta, o[j].z, x.z); x.w = fmaf(beta, o[j].w, x.w); }
-                        if (cp != nullptr) *reinterpret_cast<float4*>(cp + (q0 + j) * cstep) = x;
-                        if (bp != nullptr) *reinterpret_cast<uint2*>(bp + (q0 + j) * bstep) = pack_h16x4(x, cb_f16);
-                    } else {
-                        // ragged N / unaligned outputs: element-wise with guards
-                        const float xs[4] = {x.x, x.y, x.z, x.w};
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            if (col + i >= N) continue;
-                            float y = xs[i];
-                            if (cp != nullptr) {
-                                float* dst = cp + (q0 + j) * cstep + i;
-                                if (acc_c) y = fmaf(beta, *dst, y);
-                                *dst = y;
-                            }
-                            if (bp != nullptr) reinterpret_cast<unsigned short*>(bp)[(q0 + j) * bstep + i] = pack_h16(y, cb_f16);
+                    for (int i = 0; i < 4; ++i) {
+                        if (col + i >= N) continue;
+                        float y = xs[i];
+                        if (cp != nullptr) {
+                            float* dst = cp + (q0 + j) * cstep + i;
+                            if (acc_c) y = fmaf(beta, *dst, y);
+                            *dst = y;
                         }
+                        if (bp != nullptr) reinterpret_cast<unsigned short*>(bp)[(q0 + j) * bstep + i] = pack_h16(y, cb_f16);
                     }
                 }
             }
@@ -819,9 +814,6 @@ static std::once_flag g_encode_once;
 static unsigned long long* g_dbg = nullptr;
 static int g_dbg_launch = 0;      // launch slot inside the stamp buffer (32 slots x 1024 CTAs x 16 stamps)
 
-void tc_set_pdl(bool on) { pdl_set(on); }
-bool tc_pdl() { return pdl_enabled(); }
-
 static int get_encode() {
     std::call_once(g_encode_once, [] {
         void* fn = nullptr;
@@ -880,11 +872,9 @@ static int tc_launch(cudaStream_t st, const TcGroup& grp, int total_ctas, double
         at[na].val.clusterDim.x = (unsigned)grp.cluster; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
         ++na;
     }
-    if (pdl_enabled()) {
-        at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
+    at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
     cfg.attrs = at;
     cfg.numAttrs = na;
     const cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_bf16_tcgen05_kernel, grp);
@@ -994,7 +984,7 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     const cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_bf16_persistent_kernel, out);
     count_launch();
     if (e != cudaSuccess) return cuda_fail(e, "gemm_bf16_persistent_kernel");
@@ -1020,28 +1010,10 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
     return TEAM_OK;
 }
 
-// co-resident CTA budget of a launch whose cluster size is `cluster` (TEAM_GEMM_CTAS_C2 / _C4 / _C8 override)
+// co-resident CTA budget of a launch whose cluster size is `cluster`
 static int tc_target_ctas(int cluster) {
-    static int cap[4] = {-1, -1, -1, -1};
-    if (cap[0] < 0) {
-        const char* names[4] = {nullptr, "TEAM_GEMM_CTAS_C2", "TEAM_GEMM_CTAS_C4", "TEAM_GEMM_CTAS_C8"};
-        const int defaults[4] = {TC_TARGET_CTAS, TC_TARGET_CTAS, 272, 240};      // measured at B = 1024: -2 % step time
-        for (int i = 3; i >= 0; --i) {
-            const char* e = names[i] != nullptr ? getenv(names[i]) : nullptr;
-            cap[i] = e != nullptr ? atoi(e) : defaults[i];
-        }
-    }
+    static constexpr int cap[4] = {TC_TARGET_CTAS, TC_TARGET_CTAS, 272, 240};      // measured at B = 1024: -2 % step time
     return cap[cluster >= 8 ? 3 : cluster >= 4 ? 2 : cluster >= 2 ? 1 : 0];
-}
-
-static int pk_min_tiles() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("TEAM_GEMM_PERSIST_MIN_TILES");
-        v = e != nullptr ? atoi(e) : 2 * NUM_SMS;
-        if (v < 0) v = 0;
-    }
-    return v;
 }
 
 // Plans tiles / splits for ops[0..n) and launches them in chunks of TC_MAXP problems.
@@ -1073,7 +1045,7 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
         }
         if (np == 0) continue;
         {   // large launches: persistent kernel (128 x 256 tiles, overlapped epilogue)
-            bool ok = tiles128 >= pk_min_tiles();
+            bool ok = tiles128 >= 2 * NUM_SMS;
             for (int i = 0; i < np && ok; ++i) ok = pk_eligible(*sel[i]);
             if (ok) {
                 if ((rc = pk_launch_group(st, sel, np, ws, ws_bytes))) return rc;
@@ -1124,8 +1096,7 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
         // split-K by doubling: always the problem with the most k-blocks per CTA, while two CTAs per SM can hold the launch
         int total = 0;
         for (int i = 0; i < np; ++i) total += tiles[i];
-        const bool allow_split = getenv("TEAM_NO_SPLITK") == nullptr;
-        while (allow_split) {
+        for (;;) {
             int best = -1, best_kb = 10;
             for (int i = 0; i < np; ++i) {
                 const int s = grp.p[i].splits;
@@ -1158,7 +1129,6 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
         grp.cluster = cluster;
         grp.stages = cta <= NUM_SMS ? TC_MAX_STAGES : TC_STAGES;
         grp.dbg = g_dbg != nullptr ? g_dbg + (size_t)(g_dbg_launch++ % 32) * 1024 * 16 : nullptr;
-        { const char* dg = getenv("TEAM_GEMM_DIAG"); grp.diag = dg != nullptr ? atoi(dg) : 0; }
         if ((rc = tc_launch(st, grp, cta, flops, bytes))) return rc;
     }
     return TEAM_OK;
@@ -1238,10 +1208,5 @@ extern "C" int team_f32_to_bf16(const float* src, int64_t lds, int64_t rows, int
 extern "C" int team_gemm_debug_stamps(void* buf) {
     g_dbg = reinterpret_cast<unsigned long long*>(buf);
     g_dbg_launch = 0;
-    return TEAM_OK;
-}
-
-extern "C" int team_set_pdl(int on) {
-    tc_set_pdl(on != 0);
     return TEAM_OK;
 }

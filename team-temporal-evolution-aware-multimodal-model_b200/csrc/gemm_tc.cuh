@@ -36,8 +36,6 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
 int gemm_bf16_tc(cudaStream_t st, const TcGemm& g, void* ws, size_t ws_bytes);
 size_t tc_workspace_bytes(size_t partial_bytes);
 int tc_workspace_init(cudaStream_t st, void* ws, size_t ws_bytes);
-void tc_set_pdl(bool on);
-bool tc_pdl();
 // fp32 [rows,cols] (lds) -> bf16 hi (+ optional lo = bf16(x - hi)) with leading dimension ldd
 int to_bf16(cudaStream_t st, const float* src, int64_t lds, int64_t rows, int cols, void* hi, void* lo, int64_t ldd);
 

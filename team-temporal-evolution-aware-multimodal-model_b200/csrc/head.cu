@@ -1,7 +1,6 @@
 // Host orchestration + C ABI of the fusion head: team_head_tri_fwd / team_head_tri_bwd /
 // team_head_encode (include/team_b200.h).  Every launch goes to the caller's stream, there is
 // no synchronisation and no allocation, so a whole step can be captured into a CUDA graph.
-#include <stdlib.h>
 #include "head_proof_kernels.cuh"
 #include "head_table_kernels.cuh"
 #include "head_table_gram.cuh"
@@ -266,7 +265,7 @@ static int record_ready(cudaStream_t st, void* ev) {
 // ---- fork / join onto a per-thread side stream, so that independent kernels of one call run concurrently (under
 // stream capture the side stream joins the capture and the kernels become parallel branches of the graph).
 // Resources are created lazily per host thread and device; if that fails (e.g. creation refused during a capture)
-// the call simply stays on the caller's stream.  TEAM_NO_FORK=1 disables it (A/B runs).
+// the call simply stays on the caller's stream.
 struct SideStream {                 // one lane: a stream and its fork / join events
     cudaStream_t st = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr;
@@ -277,9 +276,6 @@ struct SideLanes {
 };
 static SideStream* side_stream(int lane) {
     static thread_local SideLanes tab[16];
-    static int off = -1;
-    if (off < 0) off = getenv("TEAM_NO_FORK") != nullptr ? 1 : 0;
-    if (off) return nullptr;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return nullptr;
     SideLanes& t = tab[dev];
@@ -319,31 +315,18 @@ static int join_side(cudaStream_t main, SideStream* s) {
     return TEAM_OK;
 }
 
-// second-generation table-row kernels unless the head is too large for them or TEAM_TABLE_V1 is set (A/B runs)
+// second-generation table-row kernels unless the head is too large for them
 static bool use_table2(const HeadDims& d) {
-    static int v1 = -1;
-    if (v1 < 0) v1 = getenv("TEAM_TABLE_V1") != nullptr ? 1 : 0;
-    return v1 == 0 && table2_supported(d) && table2_bwd_smem_floats(d) * sizeof(float) <= 227 * 1024;
+    return table2_supported(d) && table2_bwd_smem_floats(d) * sizeof(float) <= 227 * 1024;
 }
 
-// Gram formulation of the table-query rows (head_table_gram.cuh) for batches of at least TEAM_TABLE_GRAM_MIN_B samples
-// (default 16384).  Measured (profiles/EXPERIMENTS.md round 2): its kernels are 1.5 - 1.9x faster than the second
-// generation in isolation at 65 536 samples, but the step gains only 2 % there (both generations fill the register file,
-// so the side-lane kernels no longer overlap) and loses below ~16 384 samples, where its two extra step-level launches
-// sit on the critical path.  TEAM_TABLE_V2 / TEAM_TABLE_V1 force the older kernels.  Read per call (tests flip it).
+// Gram formulation of the table-query rows (head_table_gram.cuh) for batches of at least TABLE_GRAM_MIN_B samples.
+// Measured (profiles/EXPERIMENTS.md round 2): its kernels are 1.5 - 1.9x faster than the second generation in isolation
+// at 65 536 samples, but the step gains only 2 % there (both generations fill the register file, so the side-lane kernels
+// no longer overlap) and loses below ~16 384 samples, where its two extra step-level launches sit on the critical path.
+constexpr int TABLE_GRAM_MIN_B = 16384;
 static bool use_table_gram(const HeadDims& d) {
-    if (getenv("TEAM_TABLE_V2") != nullptr || getenv("TEAM_TABLE_V1") != nullptr) return false;
-    const char* e = getenv("TEAM_TABLE_GRAM_MIN_B");
-    const int min_b = e != nullptr ? atoi(e) : 16384;
-    return d.B >= min_b && table_gram_supported(d);
-}
-// warps per CTA of the Gram kernels (TEAM_TG_FW / TEAM_TG_BW override, A/B runs)
-static int tg_warps_of(const HeadDims& d, const char* env, int dflt) {
-    const char* e = getenv(env);
-    int nw = e != nullptr ? atoi(e) : dflt;
-    if (nw != 8 && nw != 16) nw = dflt;
-    (void)d;
-    return nw;
+    return d.B >= TABLE_GRAM_MIN_B && table_gram_supported(d);
 }
 
 static void norm_add(NormList& nl, int& blocks, const float* Z, float* X, __nv_bfloat16* Xh, float* inv, int64_t rows) {
@@ -497,7 +480,7 @@ extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t 
     }
     if (use_table_gram(d)) {      // Gram formulation: scalar LayerNorm algebra per (sample, row), vector outputs as coefficient sums
         if ((rc = join_side(cx.st, gram_side))) return rc;          // table_gram_prep_kernel
-        const int nw = tg_warps_of(d, "TEAM_TG_FW", tg_warps(d)), groups = (d.B + nw - 1) / nw;
+        const int nw = tg_warps(d), groups = (d.B + nw - 1) / nw;
         const size_t tsm = tg_fwd_smem_floats(d) * sizeof(float);
         TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_gram_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
         TEAM_LAUNCH(table_gram_fwd_kernel, groups < NUM_SMS ? groups : NUM_SMS, nw * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.VFs.f + (size_t)d.Nsp * D, w.GT, w.W0, w.VFo.f, w.VFs.f, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state, w.xs, w.xst, w.RS);
@@ -549,7 +532,7 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
     // ---- table-query rows (prototype / state outputs)
     int tgrid;
     if (use_table_gram(d)) {      // Gram formulation (head_table_gram.cuh); needs W0 / GT / xs / xst / RS of the matching forward
-        const int nw = tg_warps_of(d, "TEAM_TG_BW", 8), groups = (d.B + nw - 1) / nw;
+        const int nw = 8, groups = (d.B + nw - 1) / nw;
         tgrid = groups < NUM_SMS ? groups : NUM_SMS;
         // LayerNorm gamma / beta gradients of the table rows: own kernel on the side lane (fields dgam / dbet of the records)
         TEAM_LAUNCH(table_dgamma_kernel, tgrid, 256, 0, own_side != nullptr ? own_side->st : cx.st, d, g_proto, g_state, w.xs, w.xst, w.tab_partials);

@@ -138,7 +138,7 @@ static int bgemm(cudaStream_t st, bool ta, bool tb, int64_t batch, int M, int N,
         cudaLaunchAttribute at[1];
         at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at; cfg.numAttrs = pdl_enabled() ? 1 : 0;
+        cfg.attrs = at; cfg.numAttrs = 1;
         cudaError_t e;
         if (!ta && tb) e = cudaLaunchKernelEx(&cfg, bgemm_f32_kernel<false, true>, M, N, K, alpha, Ab, lda, sA, Bb, ldb, sB, beta, Cb, ldc, sC);
         else if (!ta && !tb) e = cudaLaunchKernelEx(&cfg, bgemm_f32_kernel<false, false>, M, N, K, alpha, Ab, lda, sA, Bb, ldb, sB, beta, Cb, ldc, sC);

@@ -551,9 +551,8 @@ static SgPlan sg_plan(int64_t n_rows, int64_t K) {
 // ... and bf16 rows with few keys from 64 K rows on: the shared-memory kernel is issue-bound on 1 KB rows (45 % of the copy peak
 // at 4 M rows), the gather is not
 static bool sg_wanted(int64_t n_rows, int64_t K, bool bf16_rows = false) {
-    if (getenv("TEAM_SEGSUM_V2") != nullptr || getenv("TEAM_SEGSUM_V1") != nullptr) return false;
     const bool many_keys = K > 100 && n_rows >= 4096;
-    const bool narrow_rows = bf16_rows && n_rows >= 65536 && getenv("TEAM_SEGSUM_BF16_V2") == nullptr;
+    const bool narrow_rows = bf16_rows && n_rows >= 65536;
     return (many_keys || narrow_rows) && K < (1 << 20) && n_rows < (1ll << 31) && (size_t)(K + 1) * 32 * sizeof(int) <= 200 * 1024;
 }
 
@@ -686,7 +685,7 @@ static void seg_plan(int64_t n_rows, int64_t K, int* n_clusters, int* n_slabs, i
 // second generation: columns per CTA (128 x 4 floats for K <= 100, 256 x 1 for K <= 200, 128 x 1 for K <= 400), n_chunks row
 // chunks; returns false when the first generation must run
 static bool seg2_plan(int64_t n_rows, int64_t K, bool norm, int* width, int* n_chunks, int64_t* rows_per_cta) {
-    if (getenv("TEAM_SEGSUM_V1") != nullptr || K > 400 || (norm && K > 100)) return false;
+    if (K > 400 || (norm && K > 100)) return false;
     const int w = K <= 100 ? 512 : (K <= 200 ? 256 : 128);
     const size_t smem = (size_t)K * w * sizeof(float) + 8192;
     int occ = (int)((size_t)(220 * 1024) / smem);

@@ -70,6 +70,8 @@ def test_cosine_linear_vs_golden(golden):
     (4099, 20, True, False, torch.float32), (65536, 20, False, True, torch.float32),
     (30001, 20, True, False, torch.bfloat16), (5000, 70, False, False, torch.float32),
     (70001, 20, True, False, torch.bfloat16), (66000, 6, False, True, torch.bfloat16),      # bf16 rows, few keys: key-partitioned path
+    (3000, 50, False, False, torch.float32), (2500, 30, True, True, torch.float32),          # first generation below 4 096 rows: K > 400; K > 100 normalised
+    (20000, 170, True, False, torch.bfloat16),                                               # first generation: K >= 1 600 keys
 ])
 def test_keyed_sums_vs_oracle(n, C, zipf, norm, dtype):
     from team_b200 import ops
@@ -110,12 +112,11 @@ def test_keyed_sums_empty_and_out_of_range():
     assert counts0.cpu().tolist() == [0, 0, 0, 0] and float(sums0.abs().sum()) == 0.0
 
 
-@pytest.mark.parametrize("n", [4096, 10007, 300000])
+@pytest.mark.parametrize("n", [3000, 4096, 10007, 300000])
 def test_keyed_sums_many_keys_foreign_rows(n):
-    """The key-partitioned path (K > 100: rows sorted by key, then summed from HBM): labels outside the class window, states
-    outside [0, 10), keys that own no row, a key that owns nearly every row; equals the shared-memory path bit for bit in
-    the counts and to round-off in the sums."""
-    import os
+    """Labels outside the class window, states outside [0, 10), keys that own no row, a key that owns nearly every row, on
+    the key-partitioned path (K > 100 from 4 096 rows: rows sorted by key, then summed from HBM) and below 4 096 rows on the
+    column-partitioned shared-memory path: exact counts, sums to round-off."""
     from team_b200 import ops
     g = torch.Generator().manual_seed(n)
     x = torch.randn(n, 512, generator=g)
@@ -132,17 +133,14 @@ def test_keyed_sums_many_keys_foreign_rows(n):
     assert int(counts[80:90].sum()) == 0 and float(sums[80:90].abs().sum()) == 0.0
     again, _ = ops.keyed_sums(x.cuda(), y.cuda(), s.cuda(), class_base=3, num_classes=20, num_states=10)
     assert torch.equal(sums, again)
-    os.environ["TEAM_SEGSUM_V2"] = "1"                       # the column-partitioned shared-memory path
-    try:
-        old, cold = ops.keyed_sums(x.cuda(), y.cuda(), s.cuda(), class_base=3, num_classes=20, num_states=10)
-    finally:
-        del os.environ["TEAM_SEGSUM_V2"]
-    assert torch.equal(cold, counts) and rel(old, ref) < 1e-5
 
 
 @pytest.mark.parametrize("n,C,dtype", [(1, 2, torch.float32), (1025, 20, torch.float32),
                                        (4096, 32, torch.float32), (999, 50, torch.float32),
-                                       (2048, 20, torch.bfloat16)])
+                                       (2048, 20, torch.bfloat16),
+                                       # more than 8 192 rows: the tensor-pipe kernel (C = 50: two class chunks)
+                                       (8193, 20, torch.float32), (70001, 50, torch.float32),
+                                       (8193, 50, torch.bfloat16), (70001, 20, torch.bfloat16)])
 def test_cosine_logits_vs_oracle(n, C, dtype):
     from team_b200 import ops
     x, y, _ = synth.make_prototype_build_inputs(n, max(C, 2), seed=5 + n, normalize=False)

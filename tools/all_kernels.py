@@ -1,7 +1,7 @@
 """Launches every kernel family of libteam_b200.so once (after a warm-up pass) between cudaProfilerStart/Stop, for
     ncu --set full --profile-from-start off ... python tools/all_kernels.py
-Sizes: the headline head step (B = 1024, T = 10, bf16), an 8192-sample step for the persistent GEMM + Gram table-row
-kernels (TEAM_TABLE_GRAM_MIN_B=4096), 512 K rows (1 GB) for the HBM kernels, the 200-class graph.  Kept small on purpose: ncu saves
+Sizes: the headline head step (B = 1024, T = 10, bf16), a 16384-sample step for the persistent GEMM + Gram table-row
+kernels (the smallest batch that selects them), 512 K rows (1 GB) for the HBM kernels, the 200-class graph.  Kept small on purpose: ncu saves
 and restores device memory around every replay pass.  Peer all-reduce needs > 1 GPU and is not covered here."""
 import os
 import sys
@@ -24,7 +24,7 @@ b = {k: v.to(dev) for k, v in synth.make_batch(B, C, step=0).items()}
 cots = [c.to(dev).reshape(B, 512) for c in synth.make_cotangents(B, step=0)]
 ONLY = os.environ.get("ALLK_ONLY", "")            # "graph": only the graph / state-distance kernels (a short second capture)
 gen = torch.Generator(device=dev).manual_seed(0)
-big = 8 if ONLY == "graph" else int(os.environ.get('ALLK_BIG', '8192'))   # run with TEAM_TABLE_GRAM_MIN_B <= this to reach the Gram table-row kernels
+big = 8 if ONLY == "graph" else int(os.environ.get('ALLK_BIG', '16384'))   # >= 16384 samples select the Gram table-row kernels
 bigx = [torch.nn.functional.normalize(torch.randn(big, 512, generator=gen, device=dev), dim=-1) for _ in range(2)]
 bigs = torch.randint(1, 5, (big,), generator=gen, device=dev)
 bigc = [torch.randn(big, 512, generator=gen, device=dev) for _ in range(4)]
