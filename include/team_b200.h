@@ -470,9 +470,6 @@ int team_gemm_debug_stamps(void* buf);
 /* fp32 [rows,cols] -> bf16 hi (and optional lo residual) */
 int team_f32_to_bf16(const float* src, int64_t lds, int64_t rows, int64_t cols, void* hi, void* lo,
                      int64_t ldd, void* stream);
-/* C[M,N] fp32 = A[M,K] (bf16, K-major) * B[N,K]^T (bf16, K-major). */
-int team_gemm_bf16_nt(int64_t M, int64_t N, int64_t K, const void* A, int64_t lda,
-                      const void* B, int64_t ldb, float* C, int64_t ldc, void* stream);
 
 #ifdef __cplusplus
 }

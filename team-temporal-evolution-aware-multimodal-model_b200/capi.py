@@ -116,9 +116,6 @@ def _declare(lib):
     if hasattr(lib, "team_gemm_bf16_group"):
         lib.team_gemm_bf16_group.restype = i32
         lib.team_gemm_bf16_group.argtypes = [C.POINTER(GemmDesc), C.c_int32, vp, sz, vp]
-    if hasattr(lib, "team_gemm_bf16_nt"):
-        lib.team_gemm_bf16_nt.restype = i32
-        lib.team_gemm_bf16_nt.argtypes = [i64, i64, i64, vp, i64, vp, i64, vp, i64, vp]
     if hasattr(lib, "team_head_workspace_bytes"):
         lib.team_head_workspace_bytes.restype = sz
         lib.team_head_workspace_bytes.argtypes = [i64, C.c_int32, C.c_int32, C.c_int32, i32]

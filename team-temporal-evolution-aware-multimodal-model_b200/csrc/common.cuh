@@ -2,7 +2,6 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
-#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -98,25 +97,6 @@ __device__ __forceinline__ uint2 pack_bf16x4(float4 v) {
     o.x = *reinterpret_cast<const uint32_t*>(&a);
     o.y = *reinterpret_cast<const uint32_t*>(&b);
     return o;
-}
-
-// IEEE half (1+5+10) variants: forward ACTIVATIONS of the head keep 11 significant bits in their 16-bit GEMM
-// shadows (bounded values: normalised rows, probabilities, q/k/v of unit rows); inputs, weights and everything the
-// backward produces (gradients: unbounded range) stay bf16.  tcgen05 kind::f16 takes the A and B formats separately.
-__device__ __forceinline__ uint2 pack_f16x4(float4 v) {
-    const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
-    uint2 o;
-    o.x = *reinterpret_cast<const uint32_t*>(&a);
-    o.y = *reinterpret_cast<const uint32_t*>(&b);
-    return o;
-}
-__device__ __forceinline__ uint2 pack_h16x4(float4 v, bool f16) { return f16 ? pack_f16x4(v) : pack_bf16x4(v); }
-__device__ __forceinline__ unsigned short pack_h16(float v, bool f16) {
-    return f16 ? __half_as_ushort(__float2half_rn(v)) : __bfloat16_as_ushort(__float2bfloat16_rn(v));
-}
-__device__ __forceinline__ float4 unpack_f16x4(uint2 u) {
-    const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
-    return make_float4(a.x, a.y, b.x, b.y);
 }
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }

@@ -54,7 +54,7 @@ static_assert(TC_BM * (TC_MAX_BN + 4) * 4 <= TC_STAGES * TC_STAGE_BYTES, "epilog
 
 struct alignas(64) TcSegDev {
     CUtensorMap ma, mb;
-    int K, nkb, a_mn, b_mn, a_f16, b_f16;
+    int K, nkb, a_mn, b_mn;
 };
 struct alignas(64) TcProb {
     TcSegDev s[2];            // K-segments accumulated into the same TMEM tile (s[1].nkb == 0: single segment)
@@ -64,7 +64,7 @@ struct alignas(64) TcProb {
     long long ldc, ldcb;
     float alpha, beta;
     int M, N;
-    int bn, tiles_n, n_tiles, cta_begin, splits, kb_per_split, cb_f16;
+    int bn, tiles_n, n_tiles, cta_begin, splits, kb_per_split;
 };
 struct TcGroup {
     TcProb p[TC_MAXP];
@@ -161,9 +161,9 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo_bytes
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
            ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46) | (2ull << 61);
 }
-// instruction descriptor, kind::f16: D=f32, A / B format (0 = f16, 1 = bf16) @7 / @10, majors, N>>3 @17, M>>4 @24
-__host__ __device__ inline uint32_t umma_idesc(int M, int N, int a_mn, int b_mn, int a_f16 = 0, int b_f16 = 0) {
-    return (1u << 4) | ((a_f16 ? 0u : 1u) << 7) | ((b_f16 ? 0u : 1u) << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
+// instruction descriptor, kind::f16: D=f32, A / B format bf16 (1) @7 / @10, majors, N>>3 @17, M>>4 @24
+__host__ __device__ inline uint32_t umma_idesc(int M, int N, int a_mn, int b_mn) {
+    return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
            ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
@@ -251,8 +251,8 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
         TC_STAMP(3);
     } else if (threadIdx.x == 32) {
         // ===================== MMA issuer (one thread) =====================
-        const uint32_t idesc0 = umma_idesc(TC_BM, bn, P.s[0].a_mn, P.s[0].b_mn, P.s[0].a_f16, P.s[0].b_f16);
-        const uint32_t idesc1 = umma_idesc(TC_BM, bn, P.s[1].a_mn, P.s[1].b_mn, P.s[1].a_f16, P.s[1].b_f16);
+        const uint32_t idesc0 = umma_idesc(TC_BM, bn, P.s[0].a_mn, P.s[0].b_mn);
+        const uint32_t idesc1 = umma_idesc(TC_BM, bn, P.s[1].a_mn, P.s[1].b_mn);
         int stage = 0; uint32_t phase = 0;
         for (int kb = kb_begin; kb < kb_end; ++kb) {
             const int si = kb >= nkb0 ? 1 : 0;
@@ -327,7 +327,6 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
                         (Cb == nullptr || ((ldcb % 4 == 0) && ((reinterpret_cast<uintptr_t>(Cb) & 7) == 0)));
     const float alpha = P.alpha, beta = P.beta;
     const bool acc_c = beta != 0.f && C != nullptr;
-    const bool cb_f16 = P.cb_f16 != 0;
     const float* bias = P.bias;
     // thread -> (row offset r_off, float4 column c4): lanes run along the columns, rpp rows per pass
     const int lpr = bn >> 2;                                   // float4 columns per row (4..32)
@@ -393,7 +392,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
                 if (vec_ok) {
                     if (acc_c) { x.x = fmaf(beta, o[j].x, x.x); x.y = fmaf(beta, o[j].y, x.y); x.z = fmaf(beta, o[j].z, x.z); x.w = fmaf(beta, o[j].w, x.w); }
                     if (cp != nullptr) *reinterpret_cast<float4*>(cp + (q0 + j) * cstep) = x;
-                    if (bp != nullptr) *reinterpret_cast<uint2*>(bp + (q0 + j) * bstep) = pack_h16x4(x, cb_f16);
+                    if (bp != nullptr) *reinterpret_cast<uint2*>(bp + (q0 + j) * bstep) = pack_bf16x4(x);
                 } else {
                     // ragged N / unaligned outputs: element-wise with guards
                     const float xs[4] = {x.x, x.y, x.z, x.w};
@@ -406,7 +405,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ TcGroup g) {
                             if (acc_c) y = fmaf(beta, *dst, y);
                             *dst = y;
                         }
-                        if (bp != nullptr) reinterpret_cast<unsigned short*>(bp)[(q0 + j) * bstep + i] = pack_h16(y, cb_f16);
+                        if (bp != nullptr) bp[(q0 + j) * bstep + i] = __float2bfloat16_rn(y);
                     }
                 }
             }
@@ -458,7 +457,7 @@ struct alignas(64) PkProb {
     long long ldc, ldcb;
     float alpha, beta;
     int M, N;
-    int bn, tiles_n, n_tiles, item_begin, splits, kb_per_split, cb_f16;
+    int bn, tiles_n, n_tiles, item_begin, splits, kb_per_split;
     float* partials;              // [n_tiles][splits][128][bn] fp32 (splits > 1): summed by pk_fixup_kernel
 };
 struct PkGroup {
@@ -583,8 +582,8 @@ gemm_bf16_persistent_kernel(const __grid_constant__ PkGroup g) {
                 mbar_wait(&acc_empty[buf], accph ^ 1);              // epilogue has drained this accumulator
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint32_t d_tmem = tmem_base + (uint32_t)(buf * PK_BN_MAX);
-                const uint32_t idesc0 = umma_idesc(TC_BM, it.bn, P.s[0].a_mn, P.s[0].b_mn, P.s[0].a_f16, P.s[0].b_f16);
-                const uint32_t idesc1 = umma_idesc(TC_BM, it.bn, P.s[1].a_mn, P.s[1].b_mn, P.s[1].a_f16, P.s[1].b_f16);
+                const uint32_t idesc0 = umma_idesc(TC_BM, it.bn, P.s[0].a_mn, P.s[0].b_mn);
+                const uint32_t idesc1 = umma_idesc(TC_BM, it.bn, P.s[1].a_mn, P.s[1].b_mn);
                 for (int kb = it.kb_begin; kb < it.kb_end; ++kb) {
                     const int si = kb >= it.nkb0 ? 1 : 0;
                     const int a_mn = P.s[si].a_mn, b_mn = P.s[si].b_mn;
@@ -711,7 +710,7 @@ gemm_bf16_persistent_kernel(const __grid_constant__ PkGroup g) {
                         if (bp != nullptr) {
 #pragma unroll
                             for (int j = 0; j < 8; ++j)
-                                if (j < nj) *reinterpret_cast<uint2*>(bp + j * bstep) = pack_h16x4(v[j], P.cb_f16 != 0);
+                                if (j < nj) *reinterpret_cast<uint2*>(bp + j * bstep) = pack_bf16x4(v[j]);
                         }
                     }
                 }
@@ -737,7 +736,7 @@ struct PkFixProb {
     const float* bias;
     long long ldc, ldcb;
     float alpha, beta;
-    int M, N, bn, tiles_n, n_tiles, splits, blk_begin, cb_f16;
+    int M, N, bn, tiles_n, n_tiles, splits, blk_begin;
 };
 struct PkFix {
     PkFixProb p[TC_MAXP];
@@ -780,7 +779,7 @@ pk_fixup_kernel(const __grid_constant__ PkFix f) {
             x.x = fmaf(P.beta, o.x, x.x); x.y = fmaf(P.beta, o.y, x.y); x.z = fmaf(P.beta, o.z, x.z); x.w = fmaf(P.beta, o.w, x.w);
         }
         if (P.C != nullptr) *reinterpret_cast<float4*>(P.C + (long long)row * P.ldc + col) = x;
-        if (P.Cb != nullptr) *reinterpret_cast<uint2*>(P.Cb + (long long)row * P.ldcb + col) = pack_h16x4(x, P.cb_f16 != 0);
+        if (P.Cb != nullptr) *reinterpret_cast<uint2*>(P.Cb + (long long)row * P.ldcb + col) = pack_bf16x4(x);
     }
 }
 
@@ -846,10 +845,6 @@ static int make_map(CUtensorMap* map, const void* base, int64_t inner, int64_t o
     return TEAM_OK;
 }
 
-// split-K no longer goes through global memory: the workspace arguments are kept for ABI stability only
-size_t tc_workspace_bytes(size_t) { return 256; }
-int tc_workspace_init(cudaStream_t, void*, size_t) { return TEAM_OK; }
-
 static int tc_launch(cudaStream_t st, const TcGroup& grp, int total_ctas, double flops, double bytes) {
     // per device (a process may drive several GPUs) and cheap enough to skip a lock: a racing second call only repeats it
     static bool attr_set[64] = {};
@@ -884,7 +879,7 @@ static int tc_launch(cudaStream_t st, const TcGroup& grp, int total_ctas, double
     return TEAM_OK;
 }
 
-// ---- persistent path: planning + launch of one group (<= TC_MAXP problems).  ws = [tickets | split-K partials].
+// ---- persistent path: planning + launch of one group (<= TC_MAXP problems).  ws holds the split-K partials.
 static bool pk_eligible(const TcGemm& g) {
     if (g.N % 4 != 0) return false;
     if (g.C != nullptr && (g.ldc % 4 != 0 || (reinterpret_cast<uintptr_t>(g.C) & 15) != 0)) return false;
@@ -950,7 +945,7 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
         const TcGemm& g = *sel[i];
         PkProb& p = out.p[o];
         p.partials = grp.p[i].partials;
-        p.C = g.C; p.ldc = g.ldc; p.Cb = reinterpret_cast<__nv_bfloat16*>(g.Cb); p.ldcb = g.ldcb; p.bias = g.bias; p.cb_f16 = g.cb_f16 ? 1 : 0;
+        p.C = g.C; p.ldc = g.ldc; p.Cb = reinterpret_cast<__nv_bfloat16*>(g.Cb); p.ldcb = g.ldcb; p.bias = g.bias;
         p.alpha = g.alpha; p.beta = g.beta; p.M = (int)g.M; p.N = (int)g.N;
         p.bn = bn_[i]; p.tiles_n = tiles_n_[i]; p.n_tiles = tiles_[i]; p.splits = splits_[i]; p.kb_per_split = kbps_[i];
         p.item_begin = item;
@@ -959,7 +954,7 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
         for (int q = 0; q < g.nseg; ++q) {
             const TcSeg& sg = g.s[q];
             TcSegDev& sd = p.s[q];
-            sd.K = (int)sg.K; sd.a_mn = sg.a_mn ? 1 : 0; sd.b_mn = sg.b_mn ? 1 : 0; sd.a_f16 = sg.a_f16 ? 1 : 0; sd.b_f16 = sg.b_f16 ? 1 : 0;
+            sd.K = (int)sg.K; sd.a_mn = sg.a_mn ? 1 : 0; sd.b_mn = sg.b_mn ? 1 : 0;
             sd.nkb = (int)((sg.K + TC_BK - 1) / TC_BK);
             if (!sg.a_mn) rc = make_map(&sd.ma, sg.A, sg.K, g.M, sg.lda, TC_BK, TC_BM); else rc = make_map(&sd.ma, sg.A, g.M, sg.K, sg.lda, 64, TC_BK);
             if (rc) return rc;
@@ -1001,7 +996,7 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
             if (p.splits <= 1) continue;
             PkFixProb& q = fx.p[fx.n++];
             q.partials = p.partials; q.C = p.C; q.Cb = p.Cb; q.bias = p.bias; q.ldc = p.ldc; q.ldcb = p.ldcb;
-            q.alpha = p.alpha; q.beta = p.beta; q.M = p.M; q.N = p.N; q.bn = p.bn; q.tiles_n = p.tiles_n; q.cb_f16 = p.cb_f16;
+            q.alpha = p.alpha; q.beta = p.beta; q.M = p.M; q.N = p.N; q.bn = p.bn; q.tiles_n = p.tiles_n;
             q.n_tiles = p.n_tiles; q.splits = p.splits; q.blk_begin = blocks;
             blocks += 16 * p.n_tiles;
         }
@@ -1073,13 +1068,13 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
             p.tiles_n = (int)((g.N + bn - 1) / bn);
             p.M = (int)g.M; p.N = (int)g.N;
             p.alpha = g.alpha; p.beta = g.beta;
-            p.C = g.C; p.ldc = g.ldc; p.Cb = reinterpret_cast<__nv_bfloat16*>(g.Cb); p.ldcb = g.ldcb; p.bias = g.bias; p.cb_f16 = g.cb_f16 ? 1 : 0;
+            p.C = g.C; p.ldc = g.ldc; p.Cb = reinterpret_cast<__nv_bfloat16*>(g.Cb); p.ldcb = g.ldcb; p.bias = g.bias;
             nkbs[i] = 0;
             kflops[i] = 0;
             for (int q = 0; q < g.nseg; ++q) {
                 const TcSeg& sg = g.s[q];
                 TcSegDev& sd = p.s[q];
-                sd.K = (int)sg.K; sd.a_mn = sg.a_mn ? 1 : 0; sd.b_mn = sg.b_mn ? 1 : 0; sd.a_f16 = sg.a_f16 ? 1 : 0; sd.b_f16 = sg.b_f16 ? 1 : 0;
+                sd.K = (int)sg.K; sd.a_mn = sg.a_mn ? 1 : 0; sd.b_mn = sg.b_mn ? 1 : 0;
                 sd.nkb = (int)((sg.K + TC_BK - 1) / TC_BK);
                 // K-major operand [rows,K]: inner = K, box {64, tile rows};  MN-major operand [K,rows]: inner = rows, box {64, 64}
                 if (!sg.a_mn) rc = make_map(&sd.ma, sg.A, sg.K, g.M, sg.lda, TC_BK, TC_BM); else rc = make_map(&sd.ma, sg.A, g.M, sg.K, sg.lda, 64, TC_BK);
@@ -1134,19 +1129,6 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
     return TEAM_OK;
 }
 
-int gemm_bf16_tc(cudaStream_t st, const TcGemm& g, void* ws, size_t ws_bytes) {
-    if (g.A2 == nullptr) return gemm_bf16_group(st, &g, 1, ws, ws_bytes);
-    TEAM_REQUIRE(g.nseg == 1, "gemm_bf16: the two-term A split takes a single K-segment");
-    // two-term split of A: C = alpha (A_hi + A_lo) B + ... as two accumulating passes
-    TcGemm a = g, b = g;
-    a.A2 = nullptr;
-    int rc = gemm_bf16_group(st, &a, 1, ws, ws_bytes);
-    if (rc) return rc;
-    b.s[0].A = g.A2; b.A2 = nullptr; b.beta = 1.f; b.bias = nullptr;
-    TEAM_REQUIRE(g.C != nullptr && g.Cb == nullptr, "gemm_bf16: the two-term A split needs an fp32 output");
-    return gemm_bf16_group(st, &b, 1, ws, ws_bytes);
-}
-
 int to_bf16(cudaStream_t st, const float* src, int64_t lds, int64_t rows, int cols, void* hi, void* lo, int64_t ldd) {
     TEAM_REQUIRE(cols % 4 == 0 && lds % 4 == 0 && ldd % 4 == 0, "to_bf16: cols/ld must be multiples of 4");
     const int64_t n = rows * (cols / 4);
@@ -1167,10 +1149,14 @@ extern "C" int team_gemm_bf16(int a_mn, int b_mn, int64_t M, int64_t N, int64_t 
     memset(&g, 0, sizeof(g));
     g.M = M; g.N = N; g.nseg = 1; g.alpha = alpha; g.beta = beta;
     g.s[0].a_mn = a_mn != 0; g.s[0].b_mn = b_mn != 0; g.s[0].K = K;
-    g.s[0].A = A; g.A2 = A_lo; g.s[0].lda = lda; g.s[0].B = B; g.s[0].ldb = ldb; g.C = C; g.ldc = ldc; g.bias = bias;
-    int rc = tc_workspace_init((cudaStream_t)stream, workspace, workspace_bytes);
-    if (rc) return rc;
-    return gemm_bf16_tc((cudaStream_t)stream, g, workspace, workspace_bytes);
+    g.s[0].A = A; g.s[0].lda = lda; g.s[0].B = B; g.s[0].ldb = ldb; g.C = C; g.ldc = ldc; g.bias = bias;
+    const cudaStream_t st = (cudaStream_t)stream;
+    int rc = gemm_bf16_group(st, &g, 1, workspace, workspace_bytes);
+    if (rc || A_lo == nullptr) return rc;
+    // two-term split of A: C = alpha (A_hi + A_lo) B + ... as two passes, the second accumulating into the fp32 output
+    TEAM_REQUIRE(C != nullptr, "gemm_bf16: the two-term A split needs an fp32 output");
+    g.s[0].A = A_lo; g.beta = 1.f; g.bias = nullptr;
+    return gemm_bf16_group(st, &g, 1, workspace, workspace_bytes);
 }
 
 extern "C" int team_gemm_bf16_group(const team_gemm_desc* descs, int32_t n, void* workspace, size_t workspace_bytes,
@@ -1190,14 +1176,7 @@ extern "C" int team_gemm_bf16_group(const team_gemm_desc* descs, int32_t n, void
         g.C = d.C; g.ldc = d.ldc; g.Cb = d.C_bf16; g.ldcb = d.ldc_bf16;
         g.bias = d.bias;
     }
-    int rc = tc_workspace_init((cudaStream_t)stream, workspace, workspace_bytes);
-    if (rc) return rc;
     return gemm_bf16_group((cudaStream_t)stream, ops, n, workspace, workspace_bytes);
-}
-
-extern "C" int team_gemm_bf16_nt(int64_t M, int64_t N, int64_t K, const void* A, int64_t lda, const void* B,
-                                 int64_t ldb, float* C, int64_t ldc, void* stream) {
-    return team_gemm_bf16(0, 0, M, N, K, 1.f, A, nullptr, lda, B, ldb, 0.f, C, ldc, nullptr, nullptr, 0, stream);
 }
 
 extern "C" int team_f32_to_bf16(const float* src, int64_t lds, int64_t rows, int64_t cols, void* hi, void* lo,

@@ -12,7 +12,6 @@ struct TcSeg {
     int64_t lda;
     const void* B;            // bf16
     int64_t ldb;
-    bool a_f16, b_f16;        // operand holds IEEE half instead of bf16 (tcgen05 kind::f16 formats are per operand)
 };
 
 // C[M,N] = alpha * sum_s op(A_s) op(B_s) (+ bias[N]) (+ beta * C): up to two K-segments accumulate into the
@@ -22,20 +21,15 @@ struct TcGemm {
     int nseg;                 // 1 or 2
     TcSeg s[2];
     float alpha, beta;
-    const void* A2;           // optional bf16 "lo" half of s[0].A (same layout), single-problem entry only
     float* C;                 // fp32 [M,N] output (and beta input), may be null if Cb is set
     int64_t ldc;
     void* Cb;                 // bf16 [M,N] copy of the output, may be null
     int64_t ldcb;
-    bool cb_f16;              // write Cb as IEEE half instead of bf16
     const float* bias;        // fp32 [N] or null
 };
 
-// one launch per TC_MAXP problems; ws = [tickets | split-K partials] (tc_workspace_init zeroes the tickets)
+// one launch per TC_MAXP problems; ws holds the split-K partials of the persistent path
 int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t ws_bytes);
-int gemm_bf16_tc(cudaStream_t st, const TcGemm& g, void* ws, size_t ws_bytes);
-size_t tc_workspace_bytes(size_t partial_bytes);
-int tc_workspace_init(cudaStream_t st, void* ws, size_t ws_bytes);
 // fp32 [rows,cols] (lds) -> bf16 hi (+ optional lo = bf16(x - hi)) with leading dimension ldd
 int to_bf16(cudaStream_t st, const float* src, int64_t lds, int64_t rows, int cols, void* hi, void* lo, int64_t ldd);
 

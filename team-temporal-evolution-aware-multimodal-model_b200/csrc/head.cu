@@ -25,15 +25,13 @@ void head_plan(const HeadDims& d, int mode, void* base, HeadWS* w) {
     };
     auto take = [&](size_t n_floats) -> float* { return reinterpret_cast<float*>(take_bytes(n_floats * sizeof(float))); };
     // fp32 matrix [rows, cols] and, in BF16 mode, its bf16 shadow
-    auto mat = [&](size_t rows, size_t cols, bool want_f = true, bool act = false) -> Mat {
+    auto mat = [&](size_t rows, size_t cols, bool want_f = true) -> Mat {
         Mat m;
         m.f = want_f ? take(rows * cols) : nullptr;
         m.h = bf ? reinterpret_cast<__nv_bfloat16*>(take_bytes(rows * cols * 2)) : nullptr;
         m.ld = (int64_t)cols;
-        m.f16 = act && ACT_F16;          // forward activation: IEEE-half shadow (head_kernels.cuh)
         return m;
     };
-    const bool ACT = true;
     const size_t B2 = d.B2, Nsp = d.Nsp, Rt = d.Rt, Bn = d.B;
     for (int i = 0; i < 3; ++i) { w->Wsum[i] = mat(D, D); w->bsum[i] = take(D); }
     w->Wqkv = mat(3 * D, D);
@@ -41,14 +39,14 @@ void head_plan(const HeadDims& d, int mode, void* base, HeadWS* w) {
     w->protos = mat(d.C, D, false); w->E = mat(10, D, false);
     w->img = mat(Bn, D, false); w->txt = mat(Bn, D, false);
     w->Ztab = take(Rt * D);
-    w->S = mat(Nsp, D, true, ACT); w->invS = take(Nsp);
-    w->QKVs = mat(Nsp, 3 * D, true, ACT);
-    w->VFs = mat(Nsp + 2 * TG_RP, D, true, ACT);    // + the table rows (s, n) of the Gram GEMM (head_table_gram.cuh)
-    w->TT = take(Nsp * Nsp); w->mt = take(Nsp); w->Zt = take(Nsp); w->Pt = mat(Nsp, Nsp, true, ACT); w->NFt = take(Nsp * D);
-    w->Xo = mat(B2, D, true, ACT); w->invo = take(B2);
-    w->QKVo = mat(B2, 3 * D, true, ACT); w->VFo = mat(B2, D, true, ACT);
-    w->SQ = mat(B2, Nsp); w->SK = take(B2 * Nsp);                 // SQ.h later holds dS (a gradient): bf16
-    w->Aext = mat(B2, Nsp, true, ACT); w->aown = take(B2 * 2);
+    w->S = mat(Nsp, D); w->invS = take(Nsp);
+    w->QKVs = mat(Nsp, 3 * D);
+    w->VFs = mat(Nsp + 2 * TG_RP, D);    // + the table rows (s, n) of the Gram GEMM (head_table_gram.cuh)
+    w->TT = take(Nsp * Nsp); w->mt = take(Nsp); w->Zt = take(Nsp); w->Pt = mat(Nsp, Nsp); w->NFt = take(Nsp * D);
+    w->Xo = mat(B2, D); w->invo = take(B2);
+    w->QKVo = mat(B2, 3 * D); w->VFo = mat(B2, D);
+    w->SQ = mat(B2, Nsp); w->SK = take(B2 * Nsp);
+    w->Aext = mat(B2, Nsp); w->aown = take(B2 * 2);
     w->Ybo = take(B2 * D);
     w->dYo = mat(B2, D); w->rowdot = take(B2); w->dsown = take(B2 * 2);
     w->dSK = mat(B2, Nsp); w->dVFo = mat(B2, D); w->dVFo_own = take(B2 * D);
@@ -137,9 +135,8 @@ static int run_wave(HeadCtx& cx, Wave& wv) {
                 TEAM_REQUIRE(o.s[q].A.h != nullptr && o.s[q].B.h != nullptr, "head: GEMM operand without bf16 shadow (wave op %d)", i);
                 g.s[q].a_mn = o.s[q].a_mn; g.s[q].b_mn = o.s[q].b_mn; g.s[q].K = o.s[q].K;
                 g.s[q].A = o.s[q].A.h; g.s[q].lda = o.s[q].A.ld; g.s[q].B = o.s[q].B.h; g.s[q].ldb = o.s[q].B.ld;
-                g.s[q].a_f16 = o.s[q].A.f16; g.s[q].b_f16 = o.s[q].B.f16;
             }
-            g.C = o.C.f; g.ldc = o.C.ld; g.Cb = o.C.h; g.ldcb = o.C.ld; g.bias = o.bias; g.cb_f16 = o.C.f16;
+            g.C = o.C.f; g.ldc = o.C.ld; g.Cb = o.C.h; g.ldcb = o.C.ld; g.bias = o.bias;
         }
         rc = gemm_bf16_group(cx.st, t, nt, cx.w.gemm_ws, cx.w.gemm_ws_bytes);
         wv.n = 0;
@@ -177,10 +174,10 @@ static PtrList plist(const float* const* p, int n) {
     return l;
 }
 
-static void conv_add(ConvList& cl, int& blocks, const float* src, float* dstf, __nv_bfloat16* dsth, int64_t n_floats, bool act = false) {
+static void conv_add(ConvList& cl, int& blocks, const float* src, float* dstf, __nv_bfloat16* dsth, int64_t n_floats) {
     if (n_floats <= 0 || (dstf == nullptr && dsth == nullptr)) return;
     ConvSeg& s = cl.s[cl.n++];
-    s.src = src; s.dstf = dstf; s.dsth = dsth; s.n4 = n_floats / 4; s.blk0 = blocks; s.act = act ? 1 : 0;
+    s.src = src; s.dstf = dstf; s.dsth = dsth; s.n4 = n_floats / 4; s.blk0 = blocks;
     blocks += (int)((s.n4 + 255) / 256);
 }
 
@@ -407,10 +404,9 @@ extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t 
     if ((rc = prologue(cx, hw, 3, image_feat, text_feat, want_cls ? text_cls : nullptr, batch))) return rc;
     SideStream* fill_side = side;        // joined before wave 2 (the first reader of the prompt rows): wave 1 chains straight behind the prologue
     Wave wv;
-    const Mat none{nullptr, nullptr, 0};
     auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
     // outputs that are only ever GEMM operands: in BF16 mode the fp32 copy is not written at all
-    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld, m.f16} : m; };
+    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; };
     // ---- wave 1: every projection of the step (prototype rows, state table, image rows, text rows, class text)
     seg(wv.add(d.C, D, 0.f, fonly(w.Ztab, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
     seg(wv.add(10, D, 0.f, fonly(w.Ztab + (size_t)d.C * D, D), w.bsum[2]), false, w.E, false, w.Wsum[2], D);
@@ -495,7 +491,6 @@ extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t 
     }
     if ((rc = join_side(cx.st, side))) return rc;
     if ((rc = join_side(cx.st, cls_side))) return rc;
-    (void)none;
     return TEAM_OK;
 }
 
@@ -517,7 +512,7 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
     const TabOff to = tab_offsets(d);
     auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
     const bool bf = cx.mode == TEAM_MODE_BF16;
-    auto honly = [&](const Mat& m) { return bf ? Mat{nullptr, m.h, m.ld, m.f16} : m; };
+    auto honly = [&](const Mat& m) { return bf ? Mat{nullptr, m.h, m.ld} : m; };
     // ---- own query rows: independent of the table-query rows -> side lane, beside them (its dVF part goes to dVFo_own)
     int ogrid = (d.B + 7) / 8;
     if (ogrid > NUM_SMS) ogrid = NUM_SMS;
@@ -736,14 +731,14 @@ extern "C" int team_head_proof_fwd(const team_head_weights* hw, int mode, int64_
         ConvList cl;
         memset(&cl, 0, sizeof(cl));
         int blocks = 0;
-        conv_add(cl, blocks, image_feat, w.Xo.f, w.Xo.h, batch * D, true);
-        conv_add(cl, blocks, text_feat, w.S.f, w.S.h, (int64_t)Tn * D, true);
+        conv_add(cl, blocks, image_feat, w.Xo.f, w.Xo.h, batch * D);
+        conv_add(cl, blocks, text_feat, w.S.f, w.S.h, (int64_t)Tn * D);
         TEAM_LAUNCH(prep_kernel, blocks, 256, 0, cx.st, ps, cl);
     }
     TEAM_LAUNCH(fill_prompt_rows_kernel, P + (d.Nsp - M), 128, 0, cx.st, plist(hw->prompts, hw->num_tasks), hw->prompts_per_task > 0 ? hw->prompts_per_task : 1, R, M, d.Nsp, w.S.f, w.S.h);
     Wave wv;
     auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
-    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld, m.f16} : m; };
+    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; };
     // ---- wave 1: projections (class-text rows, prototype rows, image rows)
     if (!inputs_encoded) seg(wv.add(Tn, D, 0.f, fonly(w.Ztab, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
     seg(wv.add(C, D, 0.f, fonly(w.Ztab + (size_t)Tn * D, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
@@ -827,7 +822,7 @@ extern "C" int team_head_tri_classtext_fwd(const team_head_weights* hw, int mode
     }
     Wave wv;
     auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
-    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld, m.f16} : m; };
+    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; };
     // ---- wave 1: projections (class-text rows, prototype rows, state table, image rows)
     seg(wv.add(Tn, D, 0.f, fonly(w.Ztab, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
     seg(wv.add(C, D, 0.f, fonly(w.Ztab + (size_t)Tn * D, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);

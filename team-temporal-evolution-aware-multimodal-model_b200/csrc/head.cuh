@@ -26,20 +26,16 @@ constexpr int NRM_MAX_PARTIALS = 64;     // per-segment column-sum partials of n
 // head is a Mat: the fp32 side feeds the CUDA-core kernels and the F32 mode, the bf16 side feeds tcgen05.
 // The shadow is written by whoever produces the fp32 values (GEMM epilogue or row kernel) - there is no
 // separate conversion pass except for the caller's inputs and weights (prep_kernel).
-// f16: the shadow holds IEEE half (forward activations: 11 significant bits, bounded range) instead of bf16
-// (inputs, weights, every gradient) - the tcgen05 instruction descriptor takes the format per operand.
 struct Mat {
     float* f;
     __nv_bfloat16* h;
     int64_t ld;
-    bool f16 = false;
 };
 inline Mat sub(const Mat& m, int64_t r0, int64_t c0) {
     Mat o;
     o.f = m.f ? m.f + r0 * m.ld + c0 : nullptr;
     o.h = m.h ? m.h + r0 * m.ld + c0 : nullptr;
     o.ld = m.ld;
-    o.f16 = m.f16;
     return o;
 }
 

@@ -496,8 +496,8 @@ own_own_bwd_kernel(HeadDims d, const float* __restrict__ QKVo, const __nv_bfloat
     const size_t r0 = (size_t)b * 3 * D, r1 = (size_t)(d.B + b) * 3 * D;
     float4 q0[4], q1[4], k0[4], k1[4], t[4];
     const bool hq = QKVoh != nullptr;
-    ld_row_any_act(QKVo + r0, hq ? QKVoh + r0 : nullptr, lane, q0); ld_row_any_act(QKVo + r1, hq ? QKVoh + r1 : nullptr, lane, q1);
-    ld_row_any_act(QKVo + r0 + D, hq ? QKVoh + r0 + D : nullptr, lane, k0); ld_row_any_act(QKVo + r1 + D, hq ? QKVoh + r1 + D : nullptr, lane, k1);
+    ld_row_any(QKVo + r0, hq ? QKVoh + r0 : nullptr, lane, q0); ld_row_any(QKVo + r1, hq ? QKVoh + r1 : nullptr, lane, q1);
+    ld_row_any(QKVo + r0 + D, hq ? QKVoh + r0 + D : nullptr, lane, k0); ld_row_any(QKVo + r1 + D, hq ? QKVoh + r1 + D : nullptr, lane, k1);
     const float s00 = dsown[2 * b], s01 = dsown[2 * b + 1];
     const float s10 = dsown[2 * (d.B + b)], s11 = dsown[2 * (d.B + b) + 1];
     (void)dQKVoh;

@@ -28,7 +28,6 @@ struct ConvSeg {
     __nv_bfloat16* dsth;       // optional bf16 shadow
     int64_t n4;                // float4 count (rows * cols / 4; both sides contiguous)
     int blk0;                  // first conversion block of this segment
-    int act;                   // shadow is a forward-activation buffer (IEEE half when ACT_F16), else bf16
 };
 constexpr int PREP_MAX_SEGS = 12;
 struct ConvList {
@@ -82,7 +81,7 @@ prep_kernel(const __grid_constant__ PrepSum ps, const __grid_constant__ ConvList
     if (i >= sg.n4) return;
     const float4 v = __ldg(reinterpret_cast<const float4*>(sg.src) + i);
     if (sg.dstf != nullptr) reinterpret_cast<float4*>(sg.dstf)[i] = v;
-    if (sg.dsth != nullptr) reinterpret_cast<uint2*>(sg.dsth)[i] = pack_h16x4(v, sg.act != 0 && ACT_F16);
+    if (sg.dsth != nullptr) reinterpret_cast<uint2*>(sg.dsth)[i] = pack_bf16x4(v);
 }
 
 // ------------------------------------------------------------------ row L2-normalise (F.normalize)
@@ -121,7 +120,7 @@ rows_normalize_kernel(const __grid_constant__ NormList nl) {
         scale_row(v, s);
     }
     st_row(sg.X + r * D, lane, v);
-    st_row_act(sg.Xh != nullptr ? sg.Xh + r * D : nullptr, lane, v);
+    st_row_h(sg.Xh != nullptr ? sg.Xh + r * D : nullptr, lane, v);
     if (sg.inv != nullptr && lane == 0) sg.inv[r] = s;
 }
 
@@ -155,7 +154,7 @@ fill_prompt_rows_kernel(PtrList prompts, int ppt, int C, int Ns, int Nsp, float*
         dst = Ns + (r - P);
     }
     reinterpret_cast<float4*>(S + (size_t)dst * D)[threadIdx.x] = v;
-    if (Sh != nullptr) reinterpret_cast<uint2*>(Sh + (size_t)dst * D)[threadIdx.x] = pack_h16x4(v, ACT_F16);
+    if (Sh != nullptr) reinterpret_cast<uint2*>(Sh + (size_t)dst * D)[threadIdx.x] = pack_bf16x4(v);
 }
 
 // ------------------------------------------------------------------ per-step softmax partials of step-row queries
@@ -187,10 +186,10 @@ table_prep_kernel(const float* __restrict__ TT, int M, int Nsp, float* __restric
                 add_row(v, b);
             } else {
                 st_row(Xf + (size_t)(xrows + x) * D, lane, v);
-                st_row_act(Xh != nullptr ? Xh + (size_t)(xrows + x) * D : nullptr, lane, v);
+                st_row_h(Xh != nullptr ? Xh + (size_t)(xrows + x) * D : nullptr, lane, v);
             }
             st_row(Xf + (size_t)x * D, lane, v);
-            st_row_act(Xh != nullptr ? Xh + (size_t)x * D : nullptr, lane, v);
+            st_row_h(Xh != nullptr ? Xh + (size_t)x * D : nullptr, lane, v);
             return;
         }
         return;
@@ -203,7 +202,7 @@ table_prep_kernel(const float* __restrict__ TT, int M, int Nsp, float* __restric
         float p = 0.f;
         if (j < M) { p = expf(TT[(size_t)r * Nsp + j] * INV_TAU - mx); z += p; }
         Pt[(size_t)r * Nsp + j] = p;
-        if (Pth != nullptr) st_act(Pth + (size_t)r * Nsp + j, p);
+        if (Pth != nullptr) Pth[(size_t)r * Nsp + j] = __float2bfloat16_rn(p);
     }
     z = warp_sum(z);
     if (lane == 0) { mt[r] = mx; Zt[r] = z; }
@@ -258,7 +257,7 @@ table_nf_kernel(const float* __restrict__ TT, int M, int Nsp, int C, const float
         const float4 o = part[c4];
         acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
         reinterpret_cast<float4*>(Xn + (size_t)tr * D)[c4] = acc;
-        if (Xnh != nullptr) reinterpret_cast<uint2*>(Xnh + (size_t)tr * D)[c4] = pack_h16x4(acc, ACT_F16);
+        if (Xnh != nullptr) reinterpret_cast<uint2*>(Xnh + (size_t)tr * D)[c4] = pack_bf16x4(acc);
     }
 }
 
@@ -277,10 +276,10 @@ attn_own_kernel(HeadDims d, const float* __restrict__ SQ, const float* __restric
     const int scol = d.M + clamp_state(state_ids[b]);
     float4 q[4], k[4];
     const bool hq = QKVoh != nullptr;
-    ld_row_any_act(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
-    ld_row_any_act(QKVo + (size_t)b * 3 * D + D, hq ? QKVoh + (size_t)b * 3 * D + D : nullptr, lane, k);
+    ld_row_any(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
+    ld_row_any(QKVo + (size_t)b * 3 * D + D, hq ? QKVoh + (size_t)b * 3 * D + D : nullptr, lane, k);
     const float s_img = warp_sum(dot_part(q, k)) * INV_TAU;
-    ld_row_any_act(QKVo + (size_t)(d.B + b) * 3 * D + D, hq ? QKVoh + (size_t)(d.B + b) * 3 * D + D : nullptr, lane, k);
+    ld_row_any(QKVo + (size_t)(d.B + b) * 3 * D + D, hq ? QKVoh + (size_t)(d.B + b) * 3 * D + D : nullptr, lane, k);
     const float s_txt = warp_sum(dot_part(q, k)) * INV_TAU;
     float mx = fmaxf(s_img, s_txt);
     for (int j = lane; j < d.Nsp; j += 32)
@@ -298,7 +297,7 @@ attn_own_kernel(HeadDims d, const float* __restrict__ SQ, const float* __restric
     for (int j = lane; j < d.Nsp; j += 32) {
         const float a = Aext[(size_t)row * d.Nsp + j] * iz;
         Aext[(size_t)row * d.Nsp + j] = a;
-        if (Aexth != nullptr) st_act(Aexth + (size_t)row * d.Nsp + j, a);
+        if (Aexth != nullptr) Aexth[(size_t)row * d.Nsp + j] = __float2bfloat16_rn(a);
     }
     if (lane == 0) { aown[2 * row] = p_img * iz; aown[2 * row + 1] = p_txt * iz; }
 }

@@ -41,26 +41,6 @@ __device__ __forceinline__ void st_row_h(__nv_bfloat16* p, int lane, const float
 #pragma unroll
     for (int i = 0; i < 4; ++i) reinterpret_cast<uint2*>(p)[lane + 32 * i] = pack_bf16x4(v[i]);
 }
-// Forward ACTIVATION shadows (S, Xo, q/k/v, VF, softmax probabilities) may be kept as IEEE half (11 significant bits)
-// instead of bf16.  One switch so that writers, readers and the GEMM operand formats (head.cu) cannot disagree.
-// OFF: measured on B200 (profiles/EXPERIMENTS.md, round 2) tcgen05.mma kind::f16 raises "illegal instruction" when the
-// A and B formats differ (f16 x bf16), and every backward GEMM multiplies a bf16 gradient with a forward activation;
-// all-f16 operands work, so the switch only becomes usable with a second (bf16) shadow of every activation.
-constexpr bool ACT_F16 = false;
-__device__ __forceinline__ void ld_row_any_act(const float* f, const __nv_bfloat16* h, int lane, float4 (&v)[4]) {
-    if (h != nullptr && ACT_F16) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) v[i] = unpack_f16x4(reinterpret_cast<const uint2*>(h)[lane + 32 * i]);
-    } else {
-        ld_row_any(f, h, lane, v);
-    }
-}
-__device__ __forceinline__ void st_row_act(__nv_bfloat16* p, int lane, const float4 (&v)[4]) {
-    if (p == nullptr) return;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) reinterpret_cast<uint2*>(p)[lane + 32 * i] = pack_h16x4(v[i], ACT_F16);
-}
-__device__ __forceinline__ void st_act(__nv_bfloat16* p, float v) { *reinterpret_cast<unsigned short*>(p) = pack_h16(v, ACT_F16); }
 // ---- 512-wide row arithmetic on packed fp32 pairs (sm_100 FFMA2 / FADD2 / FMUL2: one instruction per two
 // lanes of a float4, rounding identical to the scalar fmaf / add / mul)
 __device__ __forceinline__ float2 xy(const float4& v) { return make_float2(v.x, v.y); }

@@ -21,8 +21,8 @@ proof_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const
     if (row >= B) return;
     float4 q[4], k[4];
     const bool hq = QKVoh != nullptr;
-    ld_row_any_act(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
-    ld_row_any_act(QKVo + (size_t)row * 3 * D + D, hq ? QKVoh + (size_t)row * 3 * D + D : nullptr, lane, k);
+    ld_row_any(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
+    ld_row_any(QKVo + (size_t)row * 3 * D + D, hq ? QKVoh + (size_t)row * 3 * D + D : nullptr, lane, k);
     const float s_own = warp_sum(dot_part(q, k)) * INV_TAU;
     float mx = s_own;
     for (int j = lane; j < M; j += 32) mx = fmaxf(mx, SQ[(size_t)row * Nsp + j] * INV_TAU);
@@ -39,7 +39,7 @@ proof_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const
     for (int j = lane; j < Nsp; j += 32) {
         const float a = Aext[(size_t)row * Nsp + j] * iz;
         Aext[(size_t)row * Nsp + j] = a;
-        if (Aexth != nullptr) st_act(Aexth + (size_t)row * Nsp + j, a);
+        if (Aexth != nullptr) Aexth[(size_t)row * Nsp + j] = __float2bfloat16_rn(a);
     }
     if (lane == 0) aown[row] = p_own * iz;
 }
@@ -154,8 +154,8 @@ ct_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const fl
     const int scol = M + clamp_state(state_ids[row]);
     float4 q[4], k[4];
     const bool hq = QKVoh != nullptr;
-    ld_row_any_act(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
-    ld_row_any_act(QKVo + (size_t)row * 3 * D + D, hq ? QKVoh + (size_t)row * 3 * D + D : nullptr, lane, k);
+    ld_row_any(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
+    ld_row_any(QKVo + (size_t)row * 3 * D + D, hq ? QKVoh + (size_t)row * 3 * D + D : nullptr, lane, k);
     const float s_own = warp_sum(dot_part(q, k)) * INV_TAU;
     float mx = s_own;
     for (int j = lane; j < Nsp; j += 32)
@@ -173,7 +173,7 @@ ct_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const fl
     for (int j = lane; j < Nsp; j += 32) {
         const float a = Aext[(size_t)row * Nsp + j] * iz;
         Aext[(size_t)row * Nsp + j] = a;
-        if (Aexth != nullptr) st_act(Aexth + (size_t)row * Nsp + j, a);
+        if (Aexth != nullptr) Aexth[(size_t)row * Nsp + j] = __float2bfloat16_rn(a);
     }
     if (lane == 0) aown[row] = p_own * iz;
 }

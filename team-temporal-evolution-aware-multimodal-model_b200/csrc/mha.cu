@@ -357,7 +357,7 @@ __global__ void __launch_bounds__(256) mean_mid_bwd_kernel(const float* __restri
 struct Dense {
     cudaStream_t st;
     int mode;
-    void* gws; size_t gws_bytes;           // split-K / ticket workspace of the engine
+    void* gws; size_t gws_bytes;           // split-K workspace of the engine
     __nv_bfloat16 *ha, *hb;                // bf16 staging of the two operands (mode BF16)
 };
 static int dense(const Dense& e, bool ta, bool tb, int64_t M, int64_t N, int64_t K, const float* A, int64_t lda, const float* B, int64_t ldb,
@@ -375,7 +375,7 @@ static int dense(const Dense& e, bool ta, bool tb, int64_t M, int64_t N, int64_t
     g.s[0].a_mn = ta; g.s[0].b_mn = !tb; g.s[0].K = K;
     g.s[0].A = e.ha; g.s[0].lda = lda; g.s[0].B = e.hb; g.s[0].ldb = ldb;
     g.alpha = 1.f; g.beta = beta; g.C = C; g.ldc = ldc; g.bias = bias;
-    return gemm_bf16_tc(e.st, g, e.gws, e.gws_bytes);
+    return gemm_bf16_group(e.st, &g, 1, e.gws, e.gws_bytes);
 }
 
 struct MhaPlan {
@@ -407,9 +407,8 @@ static MhaPlan mha_plan(int64_t B, int64_t Lq, int64_t Lk, void* base) {
     const int64_t rmax = p.Rq > p.Rk ? p.Rq : p.Rk;
     p.ha = (__nv_bfloat16*)take((size_t)(rmax > D ? rmax : D) * D * 2);
     p.hb = (__nv_bfloat16*)take((size_t)(rmax > D ? rmax : D) * D * 2);
-    size_t g1 = gemm_f32_workspace_bytes(D, D, rmax);                      // weight gradients: K = rows (split-K)
-    size_t g2 = tc_workspace_bytes((size_t)64 << 20);
-    p.gws_bytes = align_up(g1 > g2 ? g1 : g2, 256);
+    const size_t g = gemm_f32_workspace_bytes(D, D, rmax);                 // weight gradients: K = rows (split-K)
+    p.gws_bytes = align_up(g > 256 ? g : 256, 256);                       // floor: keeps team_mha_workspace_bytes as callers size it
     p.gws = take(p.gws_bytes);
     p.total = off;
     return p;
@@ -462,7 +461,6 @@ extern "C" int team_mha_fwd(int mode, int64_t batch, int64_t len_q, int64_t len_
     if (workspace_bytes < p.total) { set_error("mha fwd: workspace %zu < %zu bytes", workspace_bytes, p.total); return TEAM_EWORKSPACE; }
     const cudaStream_t st = (cudaStream_t)stream;
     const int Lq = (int)len_q, Lk = (int)len_k;
-    if (mode == TEAM_MODE_BF16 && (rc = tc_workspace_init(st, p.gws, p.gws_bytes))) return rc;
     const Dense e{st, mode, p.gws, p.gws_bytes, p.ha, p.hb};
     if ((rc = dense(e, false, true, p.Rq, D, D, q_in, D, w_q, D, 0.f, p.Q, D, nullptr))) return rc;
     if ((rc = dense(e, false, true, p.Rk, D, D, k_in, D, w_k, D, 0.f, p.K, D, nullptr))) return rc;
@@ -495,7 +493,6 @@ extern "C" int team_mha_bwd(int mode, int64_t batch, int64_t len_q, int64_t len_
     if (workspace_bytes < p.total) { set_error("mha bwd: workspace %zu < %zu bytes", workspace_bytes, p.total); return TEAM_EWORKSPACE; }
     const cudaStream_t st = (cudaStream_t)stream;
     const int Lq = (int)len_q, Lk = (int)len_k;
-    if (mode == TEAM_MODE_BF16 && (rc = tc_workspace_init(st, p.gws, p.gws_bytes))) return rc;
     const Dense e{st, mode, p.gws, p.gws_bytes, p.ha, p.hb};
     // LayerNorm backward (+ residual branch), b_fc / gamma / beta gradients
     TEAM_LAUNCH(mha_ln_bwd_kernel, p.ln_ctas, MHA_LNB_WARPS * 32, 0, st, g_out, p.XH, p.rstd, ln_g, p.dPre, p.partial, p.Rq, p.ln_rows_per_cta,
