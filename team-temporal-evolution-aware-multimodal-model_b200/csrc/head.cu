@@ -1,6 +1,9 @@
-// Host orchestration + C ABI of the fusion head: team_head_tri_fwd / team_head_tri_bwd /
-// team_head_encode (include/team_b200.h).  Every launch goes to the caller's stream, there is
-// no synchronisation and no allocation, so a whole step can be captured into a CUDA graph.
+// Host orchestration + C ABI of the fusion head (include/team_b200.h): the tri-modal forward and backward
+// (team_head_tri_fwd / team_head_tri_bwd), the two forwards whose text rows are shared by the whole batch
+// (team_head_tri_classtext_fwd, team_head_proof_fwd: shared_rows_fwd), the projections alone and their backward
+// (team_head_encode, team_head_encode_bwd, team_head_encode_rows_bwd) and the workspace queries.  Every launch goes to
+// the caller's stream or a side lane joined before the call returns; there is no synchronisation and no allocation,
+// so a whole step can be captured into a CUDA graph.
 #include "head_proof_kernels.cuh"
 #include "head_table_kernels.cuh"
 #include "head_table_gram.cuh"
@@ -118,6 +121,9 @@ static GOp& seg(GOp& o, bool a_mn, const Mat& A, bool b_mn, const Mat& B, int64_
     g.a_mn = a_mn; g.b_mn = b_mn; g.K = K; g.A = A; g.B = B;
     return o;
 }
+static Mat fonly(float* p, int64_t ld) { return Mat{p, nullptr, ld}; }
+// outputs that are only ever GEMM operands: in BF16 mode the fp32 copy is not written at all
+static Mat honly(const Mat& m, int mode) { return mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; }
 
 static int run_wave(HeadCtx& cx, Wave& wv) {
     if (wv.n == 0) return TEAM_OK;
@@ -155,6 +161,12 @@ static int run_wave(HeadCtx& cx, Wave& wv) {
     wv.n = 0;
     return TEAM_OK;
 }
+
+#define RUN(wave)                                     \
+    do {                                              \
+        int _rc = run_wave(cx, wave);                 \
+        if (_rc != TEAM_OK) return _rc;               \
+    } while (0)
 
 static int validate(const team_head_weights* hw, int mode, int64_t batch) {
     TEAM_REQUIRE(hw != nullptr, "head: null weights");
@@ -234,16 +246,19 @@ static void bind_inputs(HeadCtx& cx, const team_head_weights* hw, const float* i
     w.tcls.f = const_cast<float*>(text_cls);
 }
 
-static int setup(HeadCtx& cx, const team_head_weights* hw, int mode, int64_t batch, int Tc, void* workspace,
-                 size_t workspace_bytes, void* stream) {
+// Checks the weights and the workspace and lays the workspace out.  The "class" block of the step rows is the
+// text_rows class-text rows followed by the C prototype rows (text_rows = 0 outside shared_rows_fwd); Tc is the
+// number of class-text rows staged by the prologue.  who names the caller in the workspace error.
+static int setup(HeadCtx& cx, const char* who, const team_head_weights* hw, int mode, int64_t batch, int text_rows, int Tc,
+                 void* workspace, size_t workspace_bytes, void* stream) {
     int rc = validate(hw, mode, batch);
     if (rc) return rc;
     cx.st = (cudaStream_t)stream;
     cx.mode = mode;
-    cx.d = head_dims(batch, hw->num_classes, hw->num_tasks * hw->prompts_per_task, Tc);
+    cx.d = head_dims(batch, text_rows + hw->num_classes, hw->num_tasks * hw->prompts_per_task, Tc);
     head_plan(cx.d, mode, workspace, &cx.w);
     if (workspace == nullptr || workspace_bytes < cx.w.total_bytes) {
-        set_error("head: workspace %zu < %zu bytes", workspace_bytes, cx.w.total_bytes);
+        set_error("%s: workspace %zu < %zu bytes", who, workspace_bytes, cx.w.total_bytes);
         return TEAM_EWORKSPACE;
     }
     TEAM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "head: workspace must be 256-byte aligned");
@@ -333,6 +348,91 @@ static void norm_add(NormList& nl, int& blocks, const float* Z, float* X, __nv_b
     blocks += (int)((rows + 7) / 8);
 }
 
+// GEMM waves 2 and 3 of every forward: q/k/v of the step rows and of the `own` own rows, then fc folded into V and
+// every score matrix.  VFo: the own-row fc values, with the bf16 shadow only where a later kernel reads it.
+static int qkv_score_waves(HeadCtx& cx, int64_t own, const Mat& VFo) {
+    const HeadDims& d = cx.d;
+    HeadWS& w = cx.w;
+    Wave wv;
+    // ---- wave 2: q/k/v of the step rows and of the own rows against the packed [3D, D] weight
+    seg(wv.add(d.Nsp, 3 * D, 0.f, honly(w.QKVs, cx.mode)), false, w.S, false, w.Wqkv, D);
+    seg(wv.add(own, 3 * D, 0.f, honly(w.QKVo, cx.mode)), false, w.Xo, false, w.Wqkv, D);
+    RUN(wv);
+    // ---- wave 3: fc folded into V, and every score matrix
+    const Mat Qs = sub(w.QKVs, 0, 0), Ks = sub(w.QKVs, 0, D), Vs = sub(w.QKVs, 0, 2 * D);
+    const Mat Qo = sub(w.QKVo, 0, 0), Ko = sub(w.QKVo, 0, D), Vo = sub(w.QKVo, 0, 2 * D);
+    seg(wv.add(d.Nsp, D, 0.f, w.VFs), false, Vs, false, w.Wfc, D);
+    seg(wv.add(own, D, 0.f, VFo), false, Vo, false, w.Wfc, D);
+    seg(wv.add(d.Nsp, d.Nsp, 0.f, fonly(w.TT, d.Nsp)), false, Qs, false, Ks, D);
+    seg(wv.add(own, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, Qo, false, Ks, D);
+    seg(wv.add(own, d.Nsp, 0.f, fonly(w.SK, d.Nsp)), false, Ko, false, Qs, D);
+    RUN(wv);
+    return TEAM_OK;
+}
+
+// Forward of the two layouts whose Tn text rows are shared by the whole batch, up to the image-row outputs: step rows
+// [Tn text | C prototypes | P prompts | 10 state rows], own rows = the B image rows (head_proof_kernels.cuh).
+// Class-text form of forward_tri_modal: state_ids given, the state table fills the 10 state rows and the sample's
+// state row is one more key of its image query.  PROOF: state_ids = nullptr, the state rows stay zero and unseen;
+// with inputs_encoded the image / text rows arrive projected and normalised.  cx comes from setup(text_rows = Tn).
+static int shared_rows_fwd(HeadCtx& cx, const team_head_weights* hw, const float* image_feat, const float* text_feat,
+                           int Tn, const int64_t* state_ids, int inputs_encoded, float* out_image) {
+    const HeadDims& d = cx.d;
+    HeadWS& w = cx.w;
+    const bool states = state_ids != nullptr;
+    const int C = hw->num_classes, R = Tn + C, M = d.M, B = d.B;
+    int rc;
+    bind_inputs(cx, hw, image_feat, nullptr, text_feat);
+    {
+        team_head_weights staged = *hw;
+        if (!states) staged.state_emb = nullptr;
+        if ((rc = prologue(cx, &staged, states ? 3 : 2, inputs_encoded ? nullptr : image_feat, nullptr,
+                           inputs_encoded ? nullptr : text_feat, B))) return rc;
+    }
+    if (inputs_encoded) {                                  // rows arrive projected + normalised: straight into Xo / S
+        PrepSum ps;
+        memset(&ps, 0, sizeof(ps));
+        ConvList cl;
+        memset(&cl, 0, sizeof(cl));
+        int blocks = 0;
+        conv_add(cl, blocks, image_feat, w.Xo.f, w.Xo.h, (int64_t)B * D);
+        conv_add(cl, blocks, text_feat, w.S.f, w.S.h, (int64_t)Tn * D);
+        TEAM_LAUNCH(prep_kernel, blocks, 256, 0, cx.st, ps, cl);
+    }
+    // prompt rows [R, M), then zeros up to Nsp: from Ns with a state table, from M without (the state rows are zero)
+    const int zero_from = states ? d.Ns : M;
+    const int fill_rows = d.P + (d.Nsp - zero_from);
+    if (fill_rows > 0)
+        TEAM_LAUNCH(fill_prompt_rows_kernel, fill_rows, 128, 0, cx.st, plist(hw->prompts, hw->num_tasks), hw->prompts_per_task > 0 ? hw->prompts_per_task : 1, R, zero_from, d.Nsp, w.S.f, w.S.h);
+    Wave wv;
+    // ---- wave 1: projections (class-text rows, prototype rows, state table, image rows)
+    if (!inputs_encoded) seg(wv.add(Tn, D, 0.f, fonly(w.Ztab, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
+    seg(wv.add(C, D, 0.f, fonly(w.Ztab + (size_t)Tn * D, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
+    if (states) seg(wv.add(10, D, 0.f, fonly(w.Ztab + (size_t)R * D, D), w.bsum[2]), false, w.E, false, w.Wsum[2], D);
+    if (!inputs_encoded) seg(wv.add(B, D, 0.f, fonly(w.Xo.f, D), w.bsum[0]), false, w.img, false, w.Wsum[0], D);
+    RUN(wv);
+    {   // L2-normalise: projected text and prototype rows -> S[0,R), state table -> S[M,M+10), image rows in place
+        NormList nl;
+        memset(&nl, 0, sizeof(nl));
+        nl.do_normalize = 1;
+        int blocks = 0;
+        const int r0 = inputs_encoded ? Tn : 0;
+        norm_add(nl, blocks, w.Ztab + (size_t)r0 * D, w.S.f + (size_t)r0 * D, w.S.h ? w.S.h + (size_t)r0 * D : nullptr, w.invS + r0, R - r0);
+        if (states) norm_add(nl, blocks, w.Ztab + (size_t)R * D, w.S.f + (size_t)M * D, w.S.h ? w.S.h + (size_t)M * D : nullptr, w.invS + M, 10);
+        if (!inputs_encoded) norm_add(nl, blocks, w.Xo.f, w.Xo.f, w.Xo.h, w.invo, B);
+        TEAM_LAUNCH(rows_normalize_kernel, blocks, 256, 0, cx.st, nl);
+    }
+    if ((rc = qkv_score_waves(cx, B, fonly(w.VFo.f, D)))) return rc;
+    TEAM_LAUNCH(table_prep_kernel, (d.Nsp + 7) / 8, 256, 0, cx.st, w.TT, M, d.Nsp, w.mt, w.Zt, w.Pt.f, w.Pt.h, (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, (const __nv_bfloat16*)nullptr, 0, 0, (float*)nullptr, (__nv_bfloat16*)nullptr);
+    TEAM_LAUNCH(image_attn_own_kernel, (B + 7) / 8, 256, 0, cx.st, B, M, d.Nsp, w.SQ.f, w.QKVo.f, cx.mode == TEAM_MODE_BF16 ? w.QKVo.h : nullptr, state_ids, w.Aext.f, w.Aext.h, w.aown);
+    // ---- wave 4: probabilities x (fc-space) values
+    seg(wv.add(d.Nsp, D, 0.f, fonly(w.NFt, D)), false, w.Pt, true, w.VFs, d.Nsp);
+    seg(wv.add(B, D, 0.f, fonly(w.Ybo, D)), false, w.Aext, true, w.VFs, d.Nsp);
+    RUN(wv);
+    TEAM_LAUNCH(proof_ln_own_fwd_kernel, (B + 7) / 8, 256, 0, cx.st, B, w.Ybo, w.aown, w.VFo.f, w.Xo.f, hw->b_fc, hw->ln_g, hw->ln_b, out_image);
+    return TEAM_OK;
+}
+
 }  // namespace team
 
 using namespace team;
@@ -373,12 +473,6 @@ extern "C" size_t team_head_own_rows_offset(int64_t batch, int32_t num_classes, 
     return (size_t)(reinterpret_cast<uintptr_t>(w.Xo.f) - 256);
 }
 
-#define RUN(wave)                                     \
-    do {                                              \
-        int _rc = run_wave(cx, wave);                 \
-        if (_rc != TEAM_OK) return _rc;               \
-    } while (0)
-
 // Forward: 13 launches (prologue, prompt rows, 4 GEMM waves, 7 row kernels; three short side-lane branches) - see
 // DESIGN.md section 4.
 extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t batch, const float* image_feat,
@@ -387,7 +481,7 @@ extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t 
                                  float* out_proto, float* cls_logits, int64_t* cls_argmax, void* workspace,
                                  size_t workspace_bytes, void* stream) {
     HeadCtx cx;
-    int rc = setup(cx, hw, mode, batch, (int)(text_cls ? num_text_cls : 0), workspace, workspace_bytes, stream);
+    int rc = setup(cx, "head", hw, mode, batch, 0, (int)(text_cls ? num_text_cls : 0), workspace, workspace_bytes, stream);
     if (rc) return rc;
     TEAM_REQUIRE(image_feat && text_feat && state_ids && out_image && out_text && out_state && out_proto, "head fwd: null pointer");
     TEAM_REQUIRE(hw->w_q && hw->w_k && hw->w_v && hw->w_fc && hw->b_fc && hw->ln_g && hw->ln_b && hw->state_emb && hw->prototypes, "head fwd: null weight");
@@ -404,9 +498,6 @@ extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t 
     if ((rc = prologue(cx, hw, 3, image_feat, text_feat, want_cls ? text_cls : nullptr, batch))) return rc;
     SideStream* fill_side = side;        // joined before wave 2 (the first reader of the prompt rows): wave 1 chains straight behind the prologue
     Wave wv;
-    auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
-    // outputs that are only ever GEMM operands: in BF16 mode the fp32 copy is not written at all
-    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; };
     // ---- wave 1: every projection of the step (prototype rows, state table, image rows, text rows, class text)
     seg(wv.add(d.C, D, 0.f, fonly(w.Ztab, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
     seg(wv.add(10, D, 0.f, fonly(w.Ztab + (size_t)d.C * D, D), w.bsum[2]), false, w.E, false, w.Wsum[2], D);
@@ -425,19 +516,8 @@ extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t 
         TEAM_LAUNCH(rows_normalize_kernel, blocks, 256, 0, cx.st, nl);
     }
     if ((rc = join_side(cx.st, fill_side))) return rc;
-    // ---- wave 2: q/k/v of the step rows and of the own rows against the packed [3D, D] weight
-    seg(wv.add(d.Nsp, 3 * D, 0.f, honly(w.QKVs)), false, w.S, false, w.Wqkv, D);
-    seg(wv.add(d.B2, 3 * D, 0.f, honly(w.QKVo)), false, w.Xo, false, w.Wqkv, D);
-    RUN(wv);
-    // ---- wave 3: fc folded into V, and every score matrix
-    const Mat Qs = sub(w.QKVs, 0, 0), Ks = sub(w.QKVs, 0, D), Vs = sub(w.QKVs, 0, 2 * D);
-    const Mat Qo = sub(w.QKVo, 0, 0), Ko = sub(w.QKVo, 0, D), Vo = sub(w.QKVo, 0, 2 * D);
-    seg(wv.add(d.Nsp, D, 0.f, w.VFs), false, Vs, false, w.Wfc, D);
-    seg(wv.add(d.B2, D, 0.f, w.VFo), false, Vo, false, w.Wfc, D);
-    seg(wv.add(d.Nsp, d.Nsp, 0.f, fonly(w.TT, d.Nsp)), false, Qs, false, Ks, D);
-    seg(wv.add(d.B2, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, Qo, false, Ks, D);
-    seg(wv.add(d.B2, d.Nsp, 0.f, fonly(w.SK, d.Nsp)), false, Ko, false, Qs, D);
-    RUN(wv);
+    // waves 2 and 3; VFo keeps its bf16 shadow (GEMM operand of the backward and of the Gram table rows)
+    if ((rc = qkv_score_waves(cx, d.B2, w.VFo))) return rc;
     SideStream* gram_side = nullptr;
     {   // the two softmax kernels (step-row table, own rows) are independent
         const cudaStream_t tst = fork_side(cx.st, &side);
@@ -501,7 +581,7 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
                                  const float* g_text, const float* g_state, const float* g_proto,
                                  const team_head_grads* gr, void* workspace, size_t workspace_bytes, void* stream) {
     HeadCtx cx;
-    int rc = setup(cx, hw, mode, batch, 0, workspace, workspace_bytes, stream);
+    int rc = setup(cx, "head", hw, mode, batch, 0, 0, workspace, workspace_bytes, stream);
     if (rc) return rc;
     TEAM_REQUIRE(gr && g_image && g_text && g_state && image_feat && text_feat && state_ids, "head bwd: null pointer");
     TEAM_REQUIRE(gr->w_img && gr->b_img && gr->w_text && gr->b_text && gr->w_state && gr->b_state && gr->state_emb &&
@@ -510,9 +590,7 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
     HeadWS& w = cx.w;
     bind_inputs(cx, hw, image_feat, text_feat, nullptr);
     const TabOff to = tab_offsets(d);
-    auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
     const bool bf = cx.mode == TEAM_MODE_BF16;
-    auto honly = [&](const Mat& m) { return bf ? Mat{nullptr, m.h, m.ld} : m; };
     // ---- own query rows: independent of the table-query rows -> side lane, beside them (its dVF part goes to dVFo_own)
     int ogrid = (d.B + 7) / 8;
     if (ogrid > NUM_SMS) ogrid = NUM_SMS;
@@ -590,10 +668,10 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
     const Mat& dS = w.SQ;
     // ---- wave 7: score gradients -> dQ/dK, fc folded into V, dWfc
     seg(wv.add(d.B2, D, 1.f, dQo), false, dS, true, Ks, d.Nsp);                                                                     // dQo = dS Ks + the own x own part
-    seg(seg(wv.add(d.Nsp, D, 0.f, honly(dKs)), true, dS, true, Qo, d.B2), true, w.dTT, true, Qs, d.Nsp);                  // dKs = dS^T Qo + dTT^T Qs
-    seg(seg(wv.add(d.Nsp, D, 0.f, honly(dQs)), true, w.dSK, true, Ko, d.B2), false, w.dTT, true, Ks, d.Nsp);              // dQs = dSK^T Ko + dTT Ks
-    seg(wv.add(d.B2, D, 0.f, honly(dVo)), false, w.dVFo, true, w.Wfc, D);                                                 // dVo = dVFo Wfc
-    seg(wv.add(d.Nsp, D, 0.f, honly(dVs)), false, w.dVFs, true, w.Wfc, D);
+    seg(seg(wv.add(d.Nsp, D, 0.f, honly(dKs, cx.mode)), true, dS, true, Qo, d.B2), true, w.dTT, true, Qs, d.Nsp);                  // dKs = dS^T Qo + dTT^T Qs
+    seg(seg(wv.add(d.Nsp, D, 0.f, honly(dQs, cx.mode)), true, w.dSK, true, Ko, d.B2), false, w.dTT, true, Ks, d.Nsp);              // dQs = dSK^T Ko + dTT Ks
+    seg(wv.add(d.B2, D, 0.f, honly(dVo, cx.mode)), false, w.dVFo, true, w.Wfc, D);                                                 // dVo = dVFo Wfc
+    seg(wv.add(d.Nsp, D, 0.f, honly(dVs, cx.mode)), false, w.dVFs, true, w.Wfc, D);
     seg(seg(wv.add(D, D, 0.f, fonly(gr->w_fc, D)), true, w.dVFo, true, Vo, d.B2), true, w.dVFs, true, Vs, d.Nsp);  // dWfc = dVFo^T Vo + dVFs^T Vs
     RUN(wv);
     if ((rc = record_ready(cx.st, gr->ev_w_fc))) return rc;
@@ -699,84 +777,17 @@ extern "C" int team_head_proof_fwd(const team_head_weights* hw, int mode, int64_
                                    const float* text_feat, int64_t num_text, int inputs_encoded, float* out_image,
                                    float* out_text, float* out_proto, void* workspace, size_t workspace_bytes,
                                    void* stream) {
-    HeadCtx cx;
-    int rc = validate(hw, mode, batch);
-    if (rc) return rc;
     TEAM_REQUIRE(image_feat && text_feat && out_image && out_text && out_proto, "head proof fwd: null pointer");
     TEAM_REQUIRE(num_text >= 1 && num_text <= 2048, "head proof fwd: num_text %lld out of range", (long long)num_text);
+    const int Tn = (int)num_text;
+    HeadCtx cx;
+    int rc = setup(cx, "head proof fwd", hw, mode, batch, Tn, Tn, workspace, workspace_bytes, stream);
+    if (rc) return rc;
     TEAM_REQUIRE(hw->w_q && hw->w_k && hw->w_v && hw->w_fc && hw->b_fc && hw->ln_g && hw->ln_b && hw->prototypes, "head proof fwd: null weight");
-    const int Tn = (int)num_text, C = hw->num_classes, P = hw->num_tasks * hw->prompts_per_task;
-    const int R = Tn + C;                                  // shared rows whose outputs are returned (batch means)
-    cx.st = (cudaStream_t)stream;
-    cx.mode = mode;
-    cx.d = head_dims(batch, R, P, Tn);                     // "classes" of the layout = text rows + prototype rows
-    head_plan(cx.d, mode, workspace, &cx.w);
-    if (workspace == nullptr || workspace_bytes < cx.w.total_bytes) {
-        set_error("head proof fwd: workspace %zu < %zu bytes", workspace_bytes, cx.w.total_bytes);
-        return TEAM_EWORKSPACE;
-    }
-    TEAM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "head: workspace must be 256-byte aligned");
+    if ((rc = shared_rows_fwd(cx, hw, image_feat, text_feat, Tn, nullptr, inputs_encoded, out_image))) return rc;
     const HeadDims& d = cx.d;
     HeadWS& w = cx.w;
-    const int M = d.M, B = d.B;                            // M = Tn + C + P shared keys; the 10 state rows of the layout stay zero
-    bind_inputs(cx, hw, image_feat, nullptr, text_feat);
-    {
-        team_head_weights tmp = *hw;
-        tmp.state_emb = nullptr;
-        if ((rc = prologue(cx, &tmp, 2, inputs_encoded ? nullptr : image_feat, nullptr, inputs_encoded ? nullptr : text_feat, batch))) return rc;
-    }
-    if (inputs_encoded) {                                  // rows arrive projected + normalised: straight into Xo / S
-        PrepSum ps;
-        memset(&ps, 0, sizeof(ps));
-        ConvList cl;
-        memset(&cl, 0, sizeof(cl));
-        int blocks = 0;
-        conv_add(cl, blocks, image_feat, w.Xo.f, w.Xo.h, batch * D);
-        conv_add(cl, blocks, text_feat, w.S.f, w.S.h, (int64_t)Tn * D);
-        TEAM_LAUNCH(prep_kernel, blocks, 256, 0, cx.st, ps, cl);
-    }
-    TEAM_LAUNCH(fill_prompt_rows_kernel, P + (d.Nsp - M), 128, 0, cx.st, plist(hw->prompts, hw->num_tasks), hw->prompts_per_task > 0 ? hw->prompts_per_task : 1, R, M, d.Nsp, w.S.f, w.S.h);
-    Wave wv;
-    auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
-    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; };
-    // ---- wave 1: projections (class-text rows, prototype rows, image rows)
-    if (!inputs_encoded) seg(wv.add(Tn, D, 0.f, fonly(w.Ztab, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
-    seg(wv.add(C, D, 0.f, fonly(w.Ztab + (size_t)Tn * D, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
-    if (!inputs_encoded) seg(wv.add(B, D, 0.f, fonly(w.Xo.f, D), w.bsum[0]), false, w.img, false, w.Wsum[0], D);
-    RUN(wv);
-    {
-        NormList nl;
-        memset(&nl, 0, sizeof(nl));
-        nl.do_normalize = 1;
-        int blocks = 0;
-        if (!inputs_encoded) {
-            norm_add(nl, blocks, w.Ztab, w.S.f, w.S.h, w.invS, R);
-            norm_add(nl, blocks, w.Xo.f, w.Xo.f, w.Xo.h, w.invo, B);
-        } else {
-            norm_add(nl, blocks, w.Ztab + (size_t)Tn * D, w.S.f + (size_t)Tn * D, w.S.h ? w.S.h + (size_t)Tn * D : nullptr, w.invS + Tn, C);
-        }
-        TEAM_LAUNCH(rows_normalize_kernel, blocks, 256, 0, cx.st, nl);
-    }
-    // ---- wave 2: q/k/v of the shared rows and of the image rows
-    seg(wv.add(d.Nsp, 3 * D, 0.f, honly(w.QKVs)), false, w.S, false, w.Wqkv, D);
-    seg(wv.add(B, 3 * D, 0.f, honly(w.QKVo)), false, w.Xo, false, w.Wqkv, D);
-    RUN(wv);
-    // ---- wave 3: fc folded into V; score matrices
-    const Mat Qs = sub(w.QKVs, 0, 0), Ks = sub(w.QKVs, 0, D), Vs = sub(w.QKVs, 0, 2 * D);
-    const Mat Qo = sub(w.QKVo, 0, 0), Ko = sub(w.QKVo, 0, D), Vo = sub(w.QKVo, 0, 2 * D);
-    seg(wv.add(d.Nsp, D, 0.f, w.VFs), false, Vs, false, w.Wfc, D);
-    seg(wv.add(B, D, 0.f, fonly(w.VFo.f, D)), false, Vo, false, w.Wfc, D);
-    seg(wv.add(d.Nsp, d.Nsp, 0.f, fonly(w.TT, d.Nsp)), false, Qs, false, Ks, D);
-    seg(wv.add(B, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, Qo, false, Ks, D);
-    seg(wv.add(B, d.Nsp, 0.f, fonly(w.SK, d.Nsp)), false, Ko, false, Qs, D);
-    RUN(wv);
-    TEAM_LAUNCH(table_prep_kernel, (d.Nsp + 7) / 8, 256, 0, cx.st, w.TT, M, d.Nsp, w.mt, w.Zt, w.Pt.f, w.Pt.h, (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, (const __nv_bfloat16*)nullptr, 0, 0, (float*)nullptr, (__nv_bfloat16*)nullptr);
-    TEAM_LAUNCH(proof_attn_own_kernel, (B + 7) / 8, 256, 0, cx.st, B, M, d.Nsp, w.SQ.f, w.QKVo.f, cx.mode == TEAM_MODE_BF16 ? w.QKVo.h : nullptr, w.Aext.f, w.Aext.h, w.aown);
-    // ---- wave 4: probabilities x (fc-space) values
-    seg(wv.add(d.Nsp, D, 0.f, fonly(w.NFt, D)), false, w.Pt, true, w.VFs, d.Nsp);
-    seg(wv.add(B, D, 0.f, fonly(w.Ybo, D)), false, w.Aext, true, w.VFs, d.Nsp);
-    RUN(wv);
-    TEAM_LAUNCH(proof_ln_own_fwd_kernel, (B + 7) / 8, 256, 0, cx.st, B, w.Ybo, w.aown, w.VFo.f, w.Xo.f, hw->b_fc, hw->ln_g, hw->ln_b, out_image);
+    const int R = Tn + hw->num_classes, B = d.B;           // shared rows whose outputs are returned (batch means)
     // ---- shared-row queries: per-CTA sums over a contiguous sample block, then the fixed-order batch mean
     int per_cta = (B + 2 * NUM_SMS - 1) / (2 * NUM_SMS);
     if (per_cta < 4) per_cta = 4;
@@ -794,69 +805,17 @@ extern "C" int team_head_tri_classtext_fwd(const team_head_weights* hw, int mode
                                            const float* text_feat, int64_t num_text, const int64_t* state_ids,
                                            float* out_image, float* out_text, float* out_state, float* out_proto,
                                            void* workspace, size_t workspace_bytes, void* stream) {
-    HeadCtx cx;
-    int rc = validate(hw, mode, batch);
-    if (rc) return rc;
     TEAM_REQUIRE(image_feat && text_feat && state_ids && out_image && out_text && out_state && out_proto, "head classtext fwd: null pointer");
     TEAM_REQUIRE(num_text >= 1 && num_text <= 2048, "head classtext fwd: num_text %lld out of range", (long long)num_text);
+    const int Tn = (int)num_text;
+    HeadCtx cx;
+    int rc = setup(cx, "head classtext fwd", hw, mode, batch, Tn, Tn, workspace, workspace_bytes, stream);
+    if (rc) return rc;
     TEAM_REQUIRE(hw->w_q && hw->w_k && hw->w_v && hw->w_fc && hw->b_fc && hw->ln_g && hw->ln_b && hw->prototypes && hw->state_emb, "head classtext fwd: null weight");
-    const int Tn = (int)num_text, C = hw->num_classes, P = hw->num_tasks * hw->prompts_per_task;
-    const int R = Tn + C;
-    cx.st = (cudaStream_t)stream;
-    cx.mode = mode;
-    cx.d = head_dims(batch, R, P, Tn);           // step rows: [Tn text | C prototypes | P prompts | 10 state-table rows]
-    head_plan(cx.d, mode, workspace, &cx.w);
-    if (workspace == nullptr || workspace_bytes < cx.w.total_bytes) {
-        set_error("head classtext fwd: workspace %zu < %zu bytes", workspace_bytes, cx.w.total_bytes);
-        return TEAM_EWORKSPACE;
-    }
-    TEAM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "head: workspace must be 256-byte aligned");
+    if ((rc = shared_rows_fwd(cx, hw, image_feat, text_feat, Tn, state_ids, 0, out_image))) return rc;
     const HeadDims& d = cx.d;
     HeadWS& w = cx.w;
-    const int M = d.M, B = d.B;
-    bind_inputs(cx, hw, image_feat, nullptr, text_feat);
-    if ((rc = prologue(cx, hw, 3, image_feat, nullptr, text_feat, batch))) return rc;
-    const int fill_rows = P + (d.Nsp - d.Ns);
-    if (fill_rows > 0) {
-        TEAM_LAUNCH(fill_prompt_rows_kernel, fill_rows, 128, 0, cx.st, plist(hw->prompts, hw->num_tasks), hw->prompts_per_task > 0 ? hw->prompts_per_task : 1, R, d.Ns, d.Nsp, w.S.f, w.S.h);
-    }
-    Wave wv;
-    auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
-    auto honly = [&](const Mat& m) { return cx.mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; };
-    // ---- wave 1: projections (class-text rows, prototype rows, state table, image rows)
-    seg(wv.add(Tn, D, 0.f, fonly(w.Ztab, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
-    seg(wv.add(C, D, 0.f, fonly(w.Ztab + (size_t)Tn * D, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
-    seg(wv.add(10, D, 0.f, fonly(w.Ztab + (size_t)R * D, D), w.bsum[2]), false, w.E, false, w.Wsum[2], D);
-    seg(wv.add(B, D, 0.f, fonly(w.Xo.f, D), w.bsum[0]), false, w.img, false, w.Wsum[0], D);
-    RUN(wv);
-    {
-        NormList nl;
-        memset(&nl, 0, sizeof(nl));
-        nl.do_normalize = 1;
-        int blocks = 0;
-        norm_add(nl, blocks, w.Ztab, w.S.f, w.S.h, w.invS, R);
-        norm_add(nl, blocks, w.Ztab + (size_t)R * D, w.S.f + (size_t)M * D, w.S.h ? w.S.h + (size_t)M * D : nullptr, w.invS + M, 10);
-        norm_add(nl, blocks, w.Xo.f, w.Xo.f, w.Xo.h, w.invo, B);
-        TEAM_LAUNCH(rows_normalize_kernel, blocks, 256, 0, cx.st, nl);
-    }
-    seg(wv.add(d.Nsp, 3 * D, 0.f, honly(w.QKVs)), false, w.S, false, w.Wqkv, D);
-    seg(wv.add(B, 3 * D, 0.f, honly(w.QKVo)), false, w.Xo, false, w.Wqkv, D);
-    RUN(wv);
-    const Mat Qs = sub(w.QKVs, 0, 0), Ks = sub(w.QKVs, 0, D), Vs = sub(w.QKVs, 0, 2 * D);
-    const Mat Qo = sub(w.QKVo, 0, 0), Ko = sub(w.QKVo, 0, D), Vo = sub(w.QKVo, 0, 2 * D);
-    seg(wv.add(d.Nsp, D, 0.f, w.VFs), false, Vs, false, w.Wfc, D);
-    seg(wv.add(B, D, 0.f, fonly(w.VFo.f, D)), false, Vo, false, w.Wfc, D);
-    seg(wv.add(d.Nsp, d.Nsp, 0.f, fonly(w.TT, d.Nsp)), false, Qs, false, Ks, D);
-    seg(wv.add(B, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, Qo, false, Ks, D);
-    seg(wv.add(B, d.Nsp, 0.f, fonly(w.SK, d.Nsp)), false, Ko, false, Qs, D);
-    RUN(wv);
-    TEAM_LAUNCH(table_prep_kernel, (d.Nsp + 7) / 8, 256, 0, cx.st, w.TT, M, d.Nsp, w.mt, w.Zt, w.Pt.f, w.Pt.h, (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, (const __nv_bfloat16*)nullptr, 0, 0, (float*)nullptr, (__nv_bfloat16*)nullptr);
-    TEAM_LAUNCH(ct_attn_own_kernel, (B + 7) / 8, 256, 0, cx.st, B, M, d.Nsp, w.SQ.f, w.QKVo.f, cx.mode == TEAM_MODE_BF16 ? w.QKVo.h : nullptr, state_ids, w.Aext.f, w.Aext.h, w.aown);
-    seg(wv.add(d.Nsp, D, 0.f, fonly(w.NFt, D)), false, w.Pt, true, w.VFs, d.Nsp);
-    seg(wv.add(B, D, 0.f, fonly(w.Ybo, D)), false, w.Aext, true, w.VFs, d.Nsp);
-    RUN(wv);
-    TEAM_LAUNCH(proof_ln_own_fwd_kernel, (B + 7) / 8, 256, 0, cx.st, B, w.Ybo, w.aown, w.VFo.f, w.Xo.f, hw->b_fc, hw->ln_g, hw->ln_b, out_image);
-    TEAM_LAUNCH(ct_table_rows_fwd_kernel, (B + 7) / 8, 256, 0, cx.st, B, Tn, C, M, d.Nsp, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_text, out_state, out_proto);
+    TEAM_LAUNCH(ct_table_rows_fwd_kernel, (d.B + 7) / 8, 256, 0, cx.st, d.B, Tn, hw->num_classes, d.M, d.Nsp, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_text, out_state, out_proto);
     return TEAM_OK;
 }
 
@@ -867,7 +826,7 @@ extern "C" int team_head_encode(const team_head_weights* hw, int mode, int which
     TEAM_REQUIRE(which >= 0 && which <= 3 && out != nullptr && n_rows >= 0, "head encode: bad args");
     if (which == 3 && hw != nullptr) n_rows = hw->num_classes;
     if (n_rows == 0) return TEAM_OK;
-    int rc = setup(cx, hw, mode, which <= 1 ? n_rows : 1, 0, workspace, workspace_bytes, stream);
+    int rc = setup(cx, "head", hw, mode, which <= 1 ? n_rows : 1, 0, 0, workspace, workspace_bytes, stream);
     if (rc) return rc;
     HeadWS& w = cx.w;
     const float* xf = which <= 1 ? reinterpret_cast<const float*>(x) : nullptr;
@@ -882,7 +841,6 @@ extern "C" int team_head_encode(const team_head_weights* hw, int mode, int which
         if (which != 2) tmp.state_emb = nullptr;
         if ((rc = prologue(cx, &tmp, 3, xf, nullptr, nullptr, which <= 1 ? n_rows : 0))) return rc;
     }
-    auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
     const int k = which == 3 ? 0 : which;
     Wave wv;
     NormList nl;
@@ -928,7 +886,7 @@ extern "C" int team_head_encode_rows_bwd(const team_head_weights* hw, int mode, 
     HeadCtx cx;
     TEAM_REQUIRE(which >= 0 && which <= 2 && x != nullptr && g_out != nullptr && g_w != nullptr && g_b != nullptr && n_rows >= 1,
                  "head encode bwd: bad args");
-    int rc = setup(cx, hw, mode, n_rows, 0, workspace, workspace_bytes, stream);
+    int rc = setup(cx, "head", hw, mode, n_rows, 0, 0, workspace, workspace_bytes, stream);
     if (rc) return rc;
     HeadWS& w = cx.w;
     bind_inputs(cx, hw, x, nullptr, nullptr);
@@ -938,7 +896,6 @@ extern "C" int team_head_encode_rows_bwd(const team_head_weights* hw, int mode, 
         tmp.prototypes = nullptr; tmp.state_emb = nullptr;
         if ((rc = prologue(cx, &tmp, 3, x, nullptr, nullptr, n_rows))) return rc;
     }
-    auto fonly = [](float* p, int64_t ld) { return Mat{p, nullptr, ld}; };
     Wave wv;
     if (normalize) {
         seg(wv.add(n_rows, D, 0.f, fonly(w.Xo.f, D), w.bsum[which]), false, w.img, false, w.Wsum[which], D);

@@ -1,36 +1,44 @@
-// Kernels of the PROOF fusion forward (Proof_Net.forward / forward_transformer, utils/inc_net.py:436-492):
-// tokens of sample b = [image_b | Tn class-text rows | C prototype rows | P prompt rows].  Only the image row is
-// per sample; the Tn + C + P other rows are the same for every sample, so - exactly as in the tri-modal head -
-// they are projected once per step, their softmax over the shared keys is a per-step partial (m_r, Z_r, NF_r)
-// and the only per-sample key they see is the image key of the sample.  Outputs: the image row of every sample,
-// and the BATCH MEANS of the text / prototype rows (utils/inc_net.py:458-459).
+// Kernels of the two forwards whose text rows are shared by the whole batch (head.cu: shared_rows_fwd).  Step rows:
+// [Tn class-text rows | C prototype rows | P prompt rows | 10 state-table rows]; only the image row is per sample.
+//  - PROOF fusion (Proof_Net.forward / forward_transformer, utils/inc_net.py:436-492): tokens of sample b =
+//    [image_b | Tn text | C prototypes | P prompts]; the state rows stay zero and no query sees them.  Outputs: the
+//    image row of every sample and the BATCH MEANS of the text / prototype rows (utils/inc_net.py:458-459).
+//  - class-text form of forward_tri_modal (utils/inc_net.py:528-580 with text rows != batch): tokens of sample b =
+//    [image_b | Tn text | state_b | C prototypes | P prompts]; the state-table row of the sample (column M + sid) is
+//    one more per-sample key.  Outputs per sample: image row, MEAN over the Tn text rows, state row, MEAN over the C
+//    prototype rows.
+// As in the tri-modal head, the shared rows are projected once per step, their softmax over the M = Tn + C + P shared
+// keys is a per-step partial (m_r, Z_r, NF_r), and the only per-sample keys they see are those of the sample.
 #pragma once
 #include "head_bwd_kernels.cuh"
 
 namespace team {
 
-// softmax of the own (image) query of every sample over the M shared keys and its own key
+// softmax of the own (image) query over the M shared keys, the sample's state key (column M + sid; none when
+// state_ids is null) and its own key
 __global__ void __launch_bounds__(256)
-proof_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const float* __restrict__ QKVo,
-                      const __nv_bfloat16* __restrict__ QKVoh, float* __restrict__ Aext,
-                      __nv_bfloat16* __restrict__ Aexth, float* __restrict__ aown) {
+image_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const float* __restrict__ QKVo,
+                      const __nv_bfloat16* __restrict__ QKVoh, const int64_t* __restrict__ state_ids,
+                      float* __restrict__ Aext, __nv_bfloat16* __restrict__ Aexth, float* __restrict__ aown) {
     pdl_trigger();
     pdl_wait();
     const int lane = threadIdx.x & 31;
     const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
     if (row >= B) return;
+    const int scol = state_ids != nullptr ? M + clamp_state(state_ids[row]) : -1;
     float4 q[4], k[4];
     const bool hq = QKVoh != nullptr;
     ld_row_any(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
     ld_row_any(QKVo + (size_t)row * 3 * D + D, hq ? QKVoh + (size_t)row * 3 * D + D : nullptr, lane, k);
     const float s_own = warp_sum(dot_part(q, k)) * INV_TAU;
     float mx = s_own;
-    for (int j = lane; j < M; j += 32) mx = fmaxf(mx, SQ[(size_t)row * Nsp + j] * INV_TAU);
+    for (int j = lane; j < Nsp; j += 32)
+        if (j < M || j == scol) mx = fmaxf(mx, SQ[(size_t)row * Nsp + j] * INV_TAU);
     mx = warp_max(mx);
     float z = 0.f;
     for (int j = lane; j < Nsp; j += 32) {
         float p = 0.f;
-        if (j < M) { p = expf(SQ[(size_t)row * Nsp + j] * INV_TAU - mx); z += p; }
+        if (j < M || j == scol) { p = expf(SQ[(size_t)row * Nsp + j] * INV_TAU - mx); z += p; }
         Aext[(size_t)row * Nsp + j] = p;
     }
     const float p_own = expf(s_own - mx);
@@ -133,49 +141,6 @@ proof_finalize_kernel(const float* __restrict__ partials, int nparts, int R, int
         float* dst = r < Tn ? out_text + (size_t)r * D : out_proto + (size_t)(r - Tn) * D;
         reinterpret_cast<float4*>(dst)[c] = t;
     }
-}
-
-// ------------------------------------------------------------------ class-text form of forward_tri_modal
-// (utils/inc_net.py:528-580 with text rows != batch): tokens of sample b = [image_b | Tn class-text rows | state_b |
-// C prototype rows | P prompt rows].  Own row: the image.  Shared keys: the M = Tn + C + P text / prototype / prompt
-// rows; per-sample keys: the own image key and the state-table row of the sample (column M + sid).  Returned:
-// image row, MEAN over the Tn text rows, state row, MEAN over the C prototype rows - all per sample.
-
-// softmax of the own (image) query over the M shared keys, the sample's state key and its own key
-__global__ void __launch_bounds__(256)
-ct_attn_own_kernel(int B, int M, int Nsp, const float* __restrict__ SQ, const float* __restrict__ QKVo,
-                   const __nv_bfloat16* __restrict__ QKVoh, const int64_t* __restrict__ state_ids,
-                   float* __restrict__ Aext, __nv_bfloat16* __restrict__ Aexth, float* __restrict__ aown) {
-    pdl_trigger();
-    pdl_wait();
-    const int lane = threadIdx.x & 31;
-    const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
-    if (row >= B) return;
-    const int scol = M + clamp_state(state_ids[row]);
-    float4 q[4], k[4];
-    const bool hq = QKVoh != nullptr;
-    ld_row_any(QKVo + (size_t)row * 3 * D, hq ? QKVoh + (size_t)row * 3 * D : nullptr, lane, q);
-    ld_row_any(QKVo + (size_t)row * 3 * D + D, hq ? QKVoh + (size_t)row * 3 * D + D : nullptr, lane, k);
-    const float s_own = warp_sum(dot_part(q, k)) * INV_TAU;
-    float mx = s_own;
-    for (int j = lane; j < Nsp; j += 32)
-        if (j < M || j == scol) mx = fmaxf(mx, SQ[(size_t)row * Nsp + j] * INV_TAU);
-    mx = warp_max(mx);
-    float z = 0.f;
-    for (int j = lane; j < Nsp; j += 32) {
-        float p = 0.f;
-        if (j < M || j == scol) { p = expf(SQ[(size_t)row * Nsp + j] * INV_TAU - mx); z += p; }
-        Aext[(size_t)row * Nsp + j] = p;
-    }
-    const float p_own = expf(s_own - mx);
-    z = warp_sum(z) + p_own;
-    const float iz = 1.0f / z;
-    for (int j = lane; j < Nsp; j += 32) {
-        const float a = Aext[(size_t)row * Nsp + j] * iz;
-        Aext[(size_t)row * Nsp + j] = a;
-        if (Aexth != nullptr) Aexth[(size_t)row * Nsp + j] = __float2bfloat16_rn(a);
-    }
-    if (lane == 0) aown[row] = p_own * iz;
 }
 
 // table-query rows of one sample (warp per sample): Tn text rows, C prototype rows, the state row.
