@@ -29,7 +29,7 @@
 #include <cudaTypedefs.h>
 #include <mutex>
 #include <stdlib.h>
-#include "gemm_tc.cuh"
+#include "gemm.cuh"
 #include "prof.cuh"
 
 namespace team {
@@ -46,7 +46,6 @@ constexpr int TC_B_BYTES = TC_MAX_BN * TC_BK * 2;      // 16 KB
 constexpr int TC_STAGE_BYTES = TC_A_BYTES + TC_B_BYTES;
 constexpr int tc_smem_bytes(int stages) { return stages * TC_STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/; }   // 3 stages: 97.25 KB -> 2 CTAs / SM
 constexpr uint32_t TC_TMEM_COLS = 128;
-constexpr int TC_MAXP = 8;           // problems per launch (kernel parameter space: 8 * 768 B; CUDA >= 12.1 allows 32 KB)
 constexpr int TC_MAX_SPLITS = 8;     // = largest portable cluster size
 constexpr int TC_TARGET_CTAS = 2 * NUM_SMS;
 
@@ -845,26 +844,70 @@ static int make_map(CUtensorMap* map, const void* base, int64_t inner, int64_t o
     return TEAM_OK;
 }
 
-static int tc_launch(cudaStream_t st, const TcGroup& grp, int total_ctas, double flops, double bytes) {
-    // per device (a process may drive several GPUs) and cheap enough to skip a lock: a racing second call only repeats it
-    static bool attr_set[64] = {};
+// The device K-segments of problem g (sd[1] is left alone when g has one segment), with B's tensor map for an N tile
+// of bn columns.  *ksum: the problem's K summed over its segments.
+static int fill_segs(TcSegDev* sd, const TcGemm& g, int bn, double* ksum) {
+    int rc;
+    *ksum = 0;
+    for (int q = 0; q < g.nseg; ++q) {
+        const TcSeg& sg = g.s[q];
+        TcSegDev& d = sd[q];
+        d.K = (int)sg.K; d.a_mn = sg.a_mn ? 1 : 0; d.b_mn = sg.b_mn ? 1 : 0;
+        d.nkb = (int)((sg.K + TC_BK - 1) / TC_BK);
+        // K-major operand [rows,K]: inner = K, box {64, tile rows};  MN-major operand [K,rows]: inner = rows, box {64, 64}
+        if (!sg.a_mn) rc = make_map(&d.ma, sg.A, sg.K, g.M, sg.lda, TC_BK, TC_BM); else rc = make_map(&d.ma, sg.A, g.M, sg.K, sg.lda, 64, TC_BK);
+        if (rc) return rc;
+        if (!sg.b_mn) rc = make_map(&d.mb, sg.B, sg.K, g.N, sg.ldb, TC_BK, bn); else rc = make_map(&d.mb, sg.B, g.N, sg.K, sg.ldb, 64, TC_BK);
+        if (rc) return rc;
+        *ksum += (double)sg.K;
+    }
+    return TEAM_OK;
+}
+
+// the profiler's estimate of one problem: 2 M N K flops; bf16 operands read once, fp32 / bf16 output written once
+static void add_cost(double& flops, double& bytes, const TcGemm& g, double ksum) {
+    const int M = (int)g.M, N = (int)g.N;
+    flops += 2.0 * M * N * ksum;
+    bytes += 2.0 * ((double)M + (double)N) * ksum + (g.C ? 4.0 : 0.0) * M * N + (g.Cb ? 2.0 : 0.0) * M * N;
+}
+
+// this launch's slot of the globaltimer stamp buffer (team_gemm_debug_stamps), or null
+static unsigned long long* next_dbg() { return g_dbg != nullptr ? g_dbg + (size_t)(g_dbg_launch++ % 32) * 1024 * 16 : nullptr; }
+
+// raises a kernel's dynamic shared memory limit once per device (a process may drive several GPUs); cheap enough
+// to skip a lock: a racing second call only repeats it
+static int set_smem_once(bool (&done)[64], const void* kernel, int bytes) {
     int dev = 0;
     TEAM_CUDA_CHECK(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(gemm_bf16_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem_bytes(TC_MAX_STAGES)));
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
+    if (dev < 0 || dev >= 64 || !done[dev]) {
+        TEAM_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        if (dev >= 0 && dev < 64) done[dev] = true;
     }
-    const int pslot = prof_enabled() ? prof_begin(st, 1, flops, bytes) : -1;
+    return TEAM_OK;
+}
+
+// one profiler record (prof.cuh) from construction to the end of the scope
+struct ProfScope {
+    cudaStream_t st;
+    int slot;
+    ProfScope(cudaStream_t s, double flops, double bytes) : st(s), slot(prof_enabled() ? prof_begin(s, 1, flops, bytes) : -1) {}
+    ~ProfScope() { if (slot >= 0) prof_end(st, slot); }
+};
+
+// launch with programmatic stream serialization and, for cluster > 1, a cluster dimension; counts the launch
+template <typename Group>
+static int tc_launch(cudaStream_t st, void (*kernel)(Group), const Group& g, const char* name, int grid, int threads,
+                     int smem, int cluster) {
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)total_ctas, 1, 1);
-    cfg.blockDim = dim3(TC_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = tc_smem_bytes(grp.stages);
+    cfg.gridDim = dim3((unsigned)grid, 1, 1);
+    cfg.blockDim = dim3((unsigned)threads, 1, 1);
+    cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute at[2];
     int na = 0;
-    if (grp.cluster > 1) {
+    if (cluster > 1) {
         at[na].id = cudaLaunchAttributeClusterDimension;
-        at[na].val.clusterDim.x = (unsigned)grp.cluster; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
+        at[na].val.clusterDim.x = (unsigned)cluster; at[na].val.clusterDim.y = 1; at[na].val.clusterDim.z = 1;
         ++na;
     }
     at[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -872,10 +915,9 @@ static int tc_launch(cudaStream_t st, const TcGroup& grp, int total_ctas, double
     ++na;
     cfg.attrs = at;
     cfg.numAttrs = na;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_bf16_tcgen05_kernel, grp);
-    if (pslot >= 0) prof_end(st, pslot);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, g);
     count_launch();
-    if (e != cudaSuccess) return cuda_fail(e, "gemm_bf16_tcgen05_kernel");
+    if (e != cudaSuccess) return cuda_fail(e, name);
     return TEAM_OK;
 }
 
@@ -889,19 +931,14 @@ static bool pk_eligible(const TcGemm& g) {
 }
 
 static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, void* ws, size_t ws_bytes) {
-    static bool attr_set[64] = {};
-    int dev = 0;
-    TEAM_CUDA_CHECK(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(gemm_bf16_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PK_SMEM_BYTES));
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-    PkGroup grp;
-    memset(&grp, 0, sizeof(grp));
+    static bool smem_set[64] = {};
+    int rc = set_smem_once(smem_set, (const void*)gemm_bf16_persistent_kernel, PK_SMEM_BYTES);
+    if (rc) return rc;
     const bool have_ws = ws != nullptr && ws_bytes > 4096 && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
     char* part_base = have_ws ? reinterpret_cast<char*>(ws) : nullptr;
     size_t part_cap = have_ws ? ws_bytes : 0, part_off = 0;
-    int order[TC_MAXP], bn_[TC_MAXP], tiles_n_[TC_MAXP], tiles_[TC_MAXP], nkb_[TC_MAXP], splits_[TC_MAXP], kbps_[TC_MAXP];
+    int order[TC_MAXP], bn_[TC_MAXP], tiles_n_[TC_MAXP], tiles_[TC_MAXP], splits_[TC_MAXP], kbps_[TC_MAXP];
+    float* partials[TC_MAXP];
     bool any_split = false;
     for (int i = 0; i < np; ++i) {
         const TcGemm& g = *sel[i];
@@ -923,12 +960,12 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
         }
         int kbps = (nkb + splits - 1) / splits;
         splits = (nkb + kbps - 1) / kbps;                 // every split owns at least one k-block
-        bn_[i] = bn; tiles_n_[i] = tiles_n; tiles_[i] = tiles; nkb_[i] = nkb; splits_[i] = splits; kbps_[i] = kbps;
+        bn_[i] = bn; tiles_n_[i] = tiles_n; tiles_[i] = tiles; splits_[i] = splits; kbps_[i] = kbps;
         order[i] = i;
+        partials[i] = nullptr;
         if (splits > 1) {
             any_split = true;
-            PkProb& p = grp.p[i];
-            p.partials = reinterpret_cast<float*>(part_base + part_off);
+            partials[i] = reinterpret_cast<float*>(part_base + part_off);
             part_off += align_up((size_t)tiles * splits * TC_BM * bn * 4, 256);
         }
     }
@@ -938,55 +975,30 @@ static int pk_launch_group(cudaStream_t st, const TcGemm* const* sel, int np, vo
             if (kbps_[order[b]] > kbps_[order[a]]) { const int t = order[a]; order[a] = order[b]; order[b] = t; }
     PkGroup out;
     memset(&out, 0, sizeof(out));
-    int item = 0, rc;
+    int item = 0;
     double flops = 0, bytes = 0;
     for (int o = 0; o < np; ++o) {
         const int i = order[o];
         const TcGemm& g = *sel[i];
         PkProb& p = out.p[o];
-        p.partials = grp.p[i].partials;
+        p.partials = partials[i];
         p.C = g.C; p.ldc = g.ldc; p.Cb = reinterpret_cast<__nv_bfloat16*>(g.Cb); p.ldcb = g.ldcb; p.bias = g.bias;
         p.alpha = g.alpha; p.beta = g.beta; p.M = (int)g.M; p.N = (int)g.N;
         p.bn = bn_[i]; p.tiles_n = tiles_n_[i]; p.n_tiles = tiles_[i]; p.splits = splits_[i]; p.kb_per_split = kbps_[i];
         p.item_begin = item;
         item += tiles_[i] * splits_[i];
-        double ksum = 0;
-        for (int q = 0; q < g.nseg; ++q) {
-            const TcSeg& sg = g.s[q];
-            TcSegDev& sd = p.s[q];
-            sd.K = (int)sg.K; sd.a_mn = sg.a_mn ? 1 : 0; sd.b_mn = sg.b_mn ? 1 : 0;
-            sd.nkb = (int)((sg.K + TC_BK - 1) / TC_BK);
-            if (!sg.a_mn) rc = make_map(&sd.ma, sg.A, sg.K, g.M, sg.lda, TC_BK, TC_BM); else rc = make_map(&sd.ma, sg.A, g.M, sg.K, sg.lda, 64, TC_BK);
-            if (rc) return rc;
-            if (!sg.b_mn) rc = make_map(&sd.mb, sg.B, sg.K, g.N, sg.ldb, TC_BK, p.bn); else rc = make_map(&sd.mb, sg.B, g.N, sg.K, sg.ldb, 64, TC_BK);
-            if (rc) return rc;
-            ksum += (double)sg.K;
-        }
-        if (g.nseg == 1) { out.p[o].s[1] = out.p[o].s[0]; out.p[o].s[1].nkb = 0; out.p[o].s[1].K = 0; }   // valid (unused) maps
-        flops += 2.0 * p.M * p.N * ksum;
-        bytes += 2.0 * ((double)p.M + (double)p.N) * ksum + (p.C ? 4.0 : 0.0) * p.M * p.N + (p.Cb ? 2.0 : 0.0) * p.M * p.N;
+        double ksum;
+        if ((rc = fill_segs(p.s, g, p.bn, &ksum))) return rc;
+        if (g.nseg == 1) { p.s[1] = p.s[0]; p.s[1].nkb = 0; p.s[1].K = 0; }   // valid (unused) maps
+        add_cost(flops, bytes, g, ksum);
     }
     out.n = np;
     out.total_items = item;
-    out.dbg = g_dbg != nullptr ? g_dbg + (size_t)(g_dbg_launch++ % 32) * 1024 * 16 : nullptr;
-    const int pslot = prof_enabled() ? prof_begin(st, 1, flops, bytes) : -1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(item < NUM_SMS ? item : NUM_SMS), 1, 1);
-    cfg.blockDim = dim3(PK_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = PK_SMEM_BYTES;
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_bf16_persistent_kernel, out);
-    count_launch();
-    if (e != cudaSuccess) return cuda_fail(e, "gemm_bf16_persistent_kernel");
-    struct ProfEnd {                     // the fix-up kernel is part of the timed GEMM
-        cudaStream_t st; int slot;
-        ~ProfEnd() { if (slot >= 0) prof_end(st, slot); }
-    } prof_guard{st, pslot};
+    out.dbg = next_dbg();
+    ProfScope prof(st, flops, bytes);    // the fix-up kernel is part of the timed GEMM
+    if ((rc = tc_launch(st, gemm_bf16_persistent_kernel, out, "gemm_bf16_persistent_kernel", item < NUM_SMS ? item : NUM_SMS,
+                        PK_THREADS, PK_SMEM_BYTES, 1)))
+        return rc;
     if (any_split) {
         PkFix fx;
         memset(&fx, 0, sizeof(fx));
@@ -1017,6 +1029,7 @@ static int tc_target_ctas(int cluster) {
 //     split further (2 / 4 / 8 ways), so that a [512,512] weight gradient over K = 2B rows does not run as 16 long CTAs
 //     next to hundreds of short ones.  The largest split count is the cluster size of the launch.
 int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t ws_bytes) {
+    static bool smem_set[64] = {};
     int rc = get_encode();
     if (rc) return rc;
     for (int base = 0; base < n; base += TC_MAXP) {
@@ -1049,7 +1062,7 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
         }
         const bool narrow = tiles128 < NUM_SMS;
         int tiles[TC_MAXP], nkbs[TC_MAXP];
-        double kflops[TC_MAXP];
+        double ksums[TC_MAXP];
         for (int i = 0; i < np; ++i) {
             const TcGemm& g = *sel[i];
             bool any_b_mn = false;
@@ -1069,21 +1082,8 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
             p.M = (int)g.M; p.N = (int)g.N;
             p.alpha = g.alpha; p.beta = g.beta;
             p.C = g.C; p.ldc = g.ldc; p.Cb = reinterpret_cast<__nv_bfloat16*>(g.Cb); p.ldcb = g.ldcb; p.bias = g.bias;
-            nkbs[i] = 0;
-            kflops[i] = 0;
-            for (int q = 0; q < g.nseg; ++q) {
-                const TcSeg& sg = g.s[q];
-                TcSegDev& sd = p.s[q];
-                sd.K = (int)sg.K; sd.a_mn = sg.a_mn ? 1 : 0; sd.b_mn = sg.b_mn ? 1 : 0;
-                sd.nkb = (int)((sg.K + TC_BK - 1) / TC_BK);
-                // K-major operand [rows,K]: inner = K, box {64, tile rows};  MN-major operand [K,rows]: inner = rows, box {64, 64}
-                if (!sg.a_mn) rc = make_map(&sd.ma, sg.A, sg.K, g.M, sg.lda, TC_BK, TC_BM); else rc = make_map(&sd.ma, sg.A, g.M, sg.K, sg.lda, 64, TC_BK);
-                if (rc) return rc;
-                if (!sg.b_mn) rc = make_map(&sd.mb, sg.B, sg.K, g.N, sg.ldb, TC_BK, bn); else rc = make_map(&sd.mb, sg.B, g.N, sg.K, sg.ldb, 64, TC_BK);
-                if (rc) return rc;
-                nkbs[i] += sd.nkb;
-                kflops[i] += (double)sg.K;
-            }
+            if ((rc = fill_segs(p.s, g, bn, &ksums[i]))) return rc;
+            nkbs[i] = p.s[0].nkb + p.s[1].nkb;
             tiles[i] = tiles_m * p.tiles_n;
             p.n_tiles = tiles[i];
             p.splits = 1;
@@ -1117,14 +1117,17 @@ int gemm_bf16_group(cudaStream_t st, const TcGemm* ops, int n, void* ws, size_t 
             p.kb_per_split = (nkbs[i] + p.splits - 1) / p.splits;
             p.cta_begin = cta;
             cta += (tiles[i] * p.splits + cluster - 1) / cluster * cluster;        // whole clusters per problem
-            flops += 2.0 * p.M * p.N * kflops[i];
-            bytes += 2.0 * ((double)p.M + (double)p.N) * kflops[i] + (p.C ? 4.0 : 0.0) * p.M * p.N + (p.Cb ? 2.0 : 0.0) * p.M * p.N;
+            add_cost(flops, bytes, *sel[i], ksums[i]);
         }
         grp.n = np;
         grp.cluster = cluster;
         grp.stages = cta <= NUM_SMS ? TC_MAX_STAGES : TC_STAGES;
-        grp.dbg = g_dbg != nullptr ? g_dbg + (size_t)(g_dbg_launch++ % 32) * 1024 * 16 : nullptr;
-        if ((rc = tc_launch(st, grp, cta, flops, bytes))) return rc;
+        grp.dbg = next_dbg();
+        if ((rc = set_smem_once(smem_set, (const void*)gemm_bf16_tcgen05_kernel, tc_smem_bytes(TC_MAX_STAGES)))) return rc;
+        ProfScope prof(st, flops, bytes);
+        if ((rc = tc_launch(st, gemm_bf16_tcgen05_kernel, grp, "gemm_bf16_tcgen05_kernel", cta, TC_THREADS, tc_smem_bytes(grp.stages),
+                            grp.cluster)))
+            return rc;
     }
     return TEAM_OK;
 }
@@ -1135,6 +1138,44 @@ int to_bf16(cudaStream_t st, const float* src, int64_t lds, int64_t rows, int co
     if (n == 0) return TEAM_OK;
     f32_to_bf16_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(src, lds, rows, cols, reinterpret_cast<__nv_bfloat16*>(hi), reinterpret_cast<__nv_bfloat16*>(lo), ldd);
     TEAM_LAUNCH_CHECK("f32_to_bf16_kernel");
+    return TEAM_OK;
+}
+
+int run_wave(cudaStream_t st, int mode, Wave& wv, void* ws, size_t ws_bytes) {
+    if (wv.n == 0) return TEAM_OK;
+    int rc;
+    if (mode == TEAM_MODE_BF16) {
+        TcGemm t[TC_MAXP];
+        int nt = 0;
+        for (int i = 0; i < wv.n; ++i) {
+            const GOp& o = wv.op[i];
+            if (o.M <= 0 || o.N <= 0) continue;
+            TcGemm& g = t[nt++];
+            memset(&g, 0, sizeof(g));
+            g.M = o.M; g.N = o.N; g.nseg = o.nseg; g.alpha = o.alpha; g.beta = o.beta;
+            for (int q = 0; q < o.nseg; ++q) {
+                TEAM_REQUIRE(o.s[q].A.h != nullptr && o.s[q].B.h != nullptr, "gemm: operand without bf16 shadow (wave op %d)", i);
+                g.s[q].a_mn = o.s[q].a_mn; g.s[q].b_mn = o.s[q].b_mn; g.s[q].K = o.s[q].K;
+                g.s[q].A = o.s[q].A.h; g.s[q].lda = o.s[q].A.ld; g.s[q].B = o.s[q].B.h; g.s[q].ldb = o.s[q].B.ld;
+            }
+            g.C = o.C.f; g.ldc = o.C.ld; g.Cb = o.C.h; g.ldcb = o.C.ld; g.bias = o.bias;
+        }
+        rc = gemm_bf16_group(st, t, nt, ws, ws_bytes);
+        wv.n = 0;
+        return rc;
+    }
+    // F32 mode: segment 0 applies beta and bias, later segments accumulate
+    for (int i = 0; i < wv.n; ++i) {
+        const GOp& o = wv.op[i];
+        if (o.M <= 0 || o.N <= 0) continue;
+        for (int q = 0; q < o.nseg; ++q) {
+            const GSeg& g = o.s[q];
+            rc = gemm_f32(st, g.a_mn, !g.b_mn, o.M, o.N, g.K, o.alpha, g.A.f, g.A.ld, g.B.f, g.B.ld, q == 0 ? o.beta : 1.f,
+                          o.C.f, o.C.ld, q == 0 ? o.bias : nullptr, ws, ws_bytes);
+            if (rc) return rc;
+        }
+    }
+    wv.n = 0;
     return TEAM_OK;
 }
 

@@ -7,7 +7,6 @@
 #include "head_proof_kernels.cuh"
 #include "head_table_kernels.cuh"
 #include "head_table_gram.cuh"
-#include "gemm_tc.cuh"
 
 namespace team {
 
@@ -87,85 +86,15 @@ struct HeadCtx {
 };
 
 // ---------------------------------------------------------------------------------------------------------
-// GEMM waves.  The head is a short chain of WAVES; every wave is a set of independent products
-//   C[M,N] = alpha * sum_{s<nseg} op(A_s) op(B_s) (+ bias) (+ beta C)
-// BF16 mode: the whole wave is ONE launch of the grouped tcgen05 kernel (bf16 shadows of the operands,
-// fp32 accumulation in tensor memory, fp32 output + optional bf16 shadow written by the epilogue).
-// F32 mode: one fp32 FFMA GEMM per segment (parity mode, not the fast path).
-struct GSeg {
-    bool a_mn, b_mn;          // false: operand stored [rows,K] (K-major); true: stored [K,rows]
-    int64_t K;
-    Mat A, B;
-};
-struct GOp {
-    int64_t M, N;
-    int nseg;
-    GSeg s[2];
-    float alpha, beta;
-    Mat C;                    // C.h (if any) receives the bf16 shadow of the result
-    const float* bias;
-};
-
-struct Wave {
-    GOp op[8];
-    int n = 0;
-    GOp& add(int64_t M, int64_t N, float beta, const Mat& C, const float* bias = nullptr) {
-        GOp& o = op[n++];
-        o.M = M; o.N = N; o.nseg = 0; o.alpha = 1.f; o.beta = beta; o.C = C; o.bias = bias;
-        return o;
-    }
-};
-// A [M,K] K-major / A stored [K,M] (a_mn) times B stored [N,K] (K-major) / B stored [K,N] (b_mn)
-static GOp& seg(GOp& o, bool a_mn, const Mat& A, bool b_mn, const Mat& B, int64_t K) {
-    GSeg& g = o.s[o.nseg++];
-    g.a_mn = a_mn; g.b_mn = b_mn; g.K = K; g.A = A; g.B = B;
-    return o;
-}
+// GEMM waves (gemm.cuh): BF16 mode runs a wave as one grouped tcgen05 launch, F32 mode as fp32 FFMA GEMMs.
 static Mat fonly(float* p, int64_t ld) { return Mat{p, nullptr, ld}; }
 // outputs that are only ever GEMM operands: in BF16 mode the fp32 copy is not written at all
 static Mat honly(const Mat& m, int mode) { return mode == TEAM_MODE_BF16 ? Mat{nullptr, m.h, m.ld} : m; }
 
-static int run_wave(HeadCtx& cx, Wave& wv) {
-    if (wv.n == 0) return TEAM_OK;
-    int rc;
-    if (cx.mode == TEAM_MODE_BF16) {
-        TcGemm t[8];
-        int nt = 0;
-        for (int i = 0; i < wv.n; ++i) {
-            const GOp& o = wv.op[i];
-            if (o.M <= 0 || o.N <= 0) continue;
-            TcGemm& g = t[nt++];
-            memset(&g, 0, sizeof(g));
-            g.M = o.M; g.N = o.N; g.nseg = o.nseg; g.alpha = o.alpha; g.beta = o.beta;
-            for (int q = 0; q < o.nseg; ++q) {
-                TEAM_REQUIRE(o.s[q].A.h != nullptr && o.s[q].B.h != nullptr, "head: GEMM operand without bf16 shadow (wave op %d)", i);
-                g.s[q].a_mn = o.s[q].a_mn; g.s[q].b_mn = o.s[q].b_mn; g.s[q].K = o.s[q].K;
-                g.s[q].A = o.s[q].A.h; g.s[q].lda = o.s[q].A.ld; g.s[q].B = o.s[q].B.h; g.s[q].ldb = o.s[q].B.ld;
-            }
-            g.C = o.C.f; g.ldc = o.C.ld; g.Cb = o.C.h; g.ldcb = o.C.ld; g.bias = o.bias;
-        }
-        rc = gemm_bf16_group(cx.st, t, nt, cx.w.gemm_ws, cx.w.gemm_ws_bytes);
-        wv.n = 0;
-        return rc;
-    }
-    for (int i = 0; i < wv.n; ++i) {
-        const GOp& o = wv.op[i];
-        if (o.M <= 0 || o.N <= 0) continue;
-        for (int q = 0; q < o.nseg; ++q) {
-            const GSeg& g = o.s[q];
-            rc = gemm_f32(cx.st, g.a_mn, !g.b_mn, o.M, o.N, g.K, o.alpha, g.A.f, g.A.ld, g.B.f, g.B.ld, q == 0 ? o.beta : 1.f,
-                          o.C.f, o.C.ld, q == 0 ? o.bias : nullptr, cx.w.gemm_ws, cx.w.gemm_ws_bytes);
-            if (rc) return rc;
-        }
-    }
-    wv.n = 0;
-    return TEAM_OK;
-}
-
-#define RUN(wave)                                     \
-    do {                                              \
-        int _rc = run_wave(cx, wave);                 \
-        if (_rc != TEAM_OK) return _rc;               \
+#define RUN(wave)                                                                  \
+    do {                                                                           \
+        int _rc = run_wave(cx.st, cx.mode, wave, cx.w.gemm_ws, cx.w.gemm_ws_bytes); \
+        if (_rc != TEAM_OK) return _rc;                                            \
     } while (0)
 
 static int validate(const team_head_weights* hw, int mode, int64_t batch) {

@@ -22,23 +22,7 @@ struct HeadDims {
 constexpr int OWN_PARTIAL_LEN = 3 * D;   // dgamma, dbeta, dbfc of the own rows
 constexpr int NRM_MAX_PARTIALS = 64;     // per-segment column-sum partials of nrm_bwd (bias gradients)
 
-// fp32 matrix + (mode BF16) its bf16 shadow with the same leading dimension.  Every GEMM operand of the
-// head is a Mat: the fp32 side feeds the CUDA-core kernels and the F32 mode, the bf16 side feeds tcgen05.
-// The shadow is written by whoever produces the fp32 values (GEMM epilogue or row kernel) - there is no
-// separate conversion pass except for the caller's inputs and weights (prep_kernel).
-struct Mat {
-    float* f;
-    __nv_bfloat16* h;
-    int64_t ld;
-};
-inline Mat sub(const Mat& m, int64_t r0, int64_t c0) {
-    Mat o;
-    o.f = m.f ? m.f + r0 * m.ld + c0 : nullptr;
-    o.h = m.h ? m.h + r0 * m.ld + c0 : nullptr;
-    o.ld = m.ld;
-    return o;
-}
-
+// Every GEMM operand of the head is a Mat (gemm.cuh).
 struct HeadWS {
     // ---- step level
     Mat Wsum[3];                      // [D][D] summed projections img/text/state

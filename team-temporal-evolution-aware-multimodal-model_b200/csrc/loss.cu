@@ -6,7 +6,6 @@
 // (fp32 FFMA GEMMs in TEAM_MODE_F32); the softmax statistics, the per-sample 3 x 3 instance term and the
 // normalise-backward are warp-per-row kernels; every batch reduction is a fixed-order fold (deterministic).
 #include "head_kernels.cuh"
-#include "gemm_tc.cuh"
 
 namespace team {
 
@@ -55,27 +54,6 @@ static void loss_plan(int64_t B, void* base, LossWS* w) {
     w->gemm_ws_bytes = 64u << 20;
     w->gemm_ws = take(w->gemm_ws_bytes);
     w->total = off;
-}
-
-// one product C[M,N] = op(A) op(B) (+ second K-segment) through the mode's GEMM engine
-struct LSeg { bool a_mn, b_mn; int64_t K; Mat A, B; };
-static int loss_gemm(cudaStream_t st, int mode, LossWS& w, int64_t M, int64_t N, float* C, int64_t ldc, const LSeg* s, int nseg) {
-    if (mode == TEAM_MODE_BF16) {
-        TcGemm g;
-        memset(&g, 0, sizeof(g));
-        g.M = M; g.N = N; g.nseg = nseg; g.alpha = 1.f; g.beta = 0.f; g.C = C; g.ldc = ldc;
-        for (int q = 0; q < nseg; ++q) {
-            g.s[q].a_mn = s[q].a_mn; g.s[q].b_mn = s[q].b_mn; g.s[q].K = s[q].K;
-            g.s[q].A = s[q].A.h; g.s[q].lda = s[q].A.ld; g.s[q].B = s[q].B.h; g.s[q].ldb = s[q].B.ld;
-        }
-        return gemm_bf16_group(st, &g, 1, w.gemm_ws, w.gemm_ws_bytes);
-    }
-    for (int q = 0; q < nseg; ++q) {
-        const int rc = gemm_f32(st, s[q].a_mn, !s[q].b_mn, M, N, s[q].K, 1.f, s[q].A.f, s[q].A.ld, s[q].B.f, s[q].B.ld,
-                                q == 0 ? 0.f : 1.f, C, ldc, nullptr, w.gemm_ws, w.gemm_ws_bytes);
-        if (rc) return rc;
-    }
-    return TEAM_OK;
 }
 
 // ------------------------------------------------------------------ kernels
@@ -660,15 +638,17 @@ static int unicl_impl(int mode, const float* image, const float* text, const flo
         TEAM_LAUNCH(evo_fwd_kernel, (B + 7) / 8, 256, 0, st, B, w.X[2].f, labels, ev->state_ids, ev->num_evo, ev->evo, ev->evo_mask, SS, cnt, Xe, Mh, sc, rowmask);
     }
     {   // sim = Xi Xi^T
-        LSeg s{false, false, D, w.X[0], w.X[0]};
-        if ((rc = loss_gemm(st, mode, w, B, B, w.sim, ld, &s, 1))) return rc;
+        Wave wv;
+        seg(wv.add(B, B, 0.f, Mat{w.sim, nullptr, ld}), false, w.X[0], false, w.X[0], D);
+        if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     }
     TEAM_LAUNCH(unicl_cat_stats_kernel, (B + 7) / 8, 256, 0, st, B, ld, w.sim, labels, inv_tau, w.rmax, w.rpos, w.rall, w.rloss);
     TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, B, w.rmax + B, w.rloss, w.scal, 0, 0.f, (const float*)nullptr, (float*)nullptr);   // valid count, category sum
     TEAM_LAUNCH(unicl_cat_grad_kernel, (B + 7) / 8, 256, 0, st, B, ld, w.sim, labels, inv_tau, 0.5f * grad_scale, w.rmax, w.rpos, w.rall, w.scal, w.G.f, bf ? w.G.h : nullptr);
     {   // dcat = G Xi + G^T Xi
-        LSeg s[2] = {{false, true, B, w.G, w.X[0]}, {true, true, B, w.G, w.X[0]}};
-        if ((rc = loss_gemm(st, mode, w, B, D, w.dcat, D, s, 2))) return rc;
+        Wave wv;
+        seg(seg(wv.add(B, D, 0.f, Mat{w.dcat, nullptr, D}), false, w.G, true, w.X[0], B), true, w.G, true, w.X[0], B);
+        if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     }
     TEAM_LAUNCH(unicl_instance_kernel, (B + 7) / 8, 256, 0, st, B, w.X[0].f, w.X[1].f, ev != nullptr ? Xe : w.X[2].f, w.inv[0], w.inv[1], w.inv[2], w.dcat, inv_tau, grad_scale / (3.0f * (float)B), g_image, g_text, g_state, w.rloss + B, dXe);
     if (ev != nullptr) {
@@ -760,20 +740,17 @@ extern "C" int team_clip_loss(int mode, const float* image, const float* text, i
     // staged copies (bf16 shadows for the tensor-core path); ClipLoss does not normalise (the caller did)
     TEAM_LAUNCH(loss_normalize_kernel, (2 * B + 7) / 8, 256, 0, st, batch, image, text, (const float*)nullptr, w.X[0].f, w.X[1].f, (float*)nullptr,
                 bf ? w.X[0].h : nullptr, bf ? w.X[1].h : nullptr, (__nv_bfloat16*)nullptr, (float*)nullptr, (float*)nullptr, (float*)nullptr, 2, 0);
-    {
-        LSeg s{false, false, D, w.X[0], w.X[1]};
-        if ((rc = loss_gemm(st, mode, w, B, B, w.sim, ld, &s, 1))) return rc;                    // L = I T^T
-        LSeg t{false, false, D, w.X[1], w.X[0]};
-        if ((rc = loss_gemm(st, mode, w, B, B, w.simT, ld, &t, 1))) return rc;                   // L^T = T I^T
-    }
+    Wave wv;       // one product per wave: a wave of two would plan its split-K, and so its summation order, as a group
+    seg(wv.add(B, B, 0.f, Mat{w.sim, nullptr, ld}), false, w.X[0], false, w.X[1], D);               // L = I T^T
+    if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
+    seg(wv.add(B, B, 0.f, Mat{w.simT, nullptr, ld}), false, w.X[1], false, w.X[0], D);              // L^T = T I^T
+    if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     TEAM_LAUNCH(clip_stats_kernel, (2 * B + 7) / 8, 256, 0, st, B, ld, w.sim, w.simT, logit_scale, w.rmax, w.rloss);
     TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, 2 * B, w.rloss, (const float*)nullptr, w.scal, 1, 1.0f / (2.0f * (float)B), (const float*)nullptr, loss);
     TEAM_LAUNCH(clip_grad_kernel, (B + 7) / 8, 256, 0, st, B, ld, w.sim, logit_scale, logit_scale * grad_scale / (2.0f * (float)B), w.rmax, w.G.f, bf ? w.G.h : nullptr);
-    {
-        LSeg s{false, true, B, w.G, w.X[1]};
-        if ((rc = loss_gemm(st, mode, w, B, D, g_image, D, &s, 1))) return rc;                   // dI = G T
-        LSeg t{true, true, B, w.G, w.X[0]};
-        if ((rc = loss_gemm(st, mode, w, B, D, g_text, D, &t, 1))) return rc;                    // dT = G^T I
-    }
+    seg(wv.add(B, D, 0.f, Mat{g_image, nullptr, D}), false, w.G, true, w.X[1], B);                  // dI = G T
+    if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
+    seg(wv.add(B, D, 0.f, Mat{g_text, nullptr, D}), true, w.G, true, w.X[0], B);                    // dT = G^T I
+    if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     return TEAM_OK;
 }

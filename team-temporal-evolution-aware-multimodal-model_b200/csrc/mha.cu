@@ -13,7 +13,6 @@
 // gradients through per-CTA partials folded in CTA order) has a fixed order, so results are run-to-run reproducible.
 #include "common.cuh"
 #include "gemm.cuh"
-#include "gemm_tc.cuh"
 
 namespace team {
 
@@ -354,6 +353,7 @@ __global__ void __launch_bounds__(256) mean_mid_bwd_kernel(const float* __restri
 
 // ------------------------------------------------------------------------------------------------ dense products
 // C[M,N] = op(A) op(B) (+ bias) (+ beta C) on the mode's GEMM engine.  ta: A stored [K,M]; tb: B stored [N,K].
+// BF16 mode stages both operands to bf16 first; shapes the tcgen05 engine cannot take run on the fp32 engine.
 struct Dense {
     cudaStream_t st;
     int mode;
@@ -363,19 +363,16 @@ struct Dense {
 static int dense(const Dense& e, bool ta, bool tb, int64_t M, int64_t N, int64_t K, const float* A, int64_t lda, const float* B, int64_t ldb,
                  float beta, float* C, int64_t ldc, const float* bias) {
     if (M <= 0 || N <= 0) return TEAM_OK;
-    if (e.mode != TEAM_MODE_BF16 || K % 8 != 0 || lda % 8 != 0 || ldb % 8 != 0 || K < 64)
-        return gemm_f32(e.st, ta, tb, M, N, K, 1.f, A, lda, B, ldb, beta, C, ldc, bias, e.gws, e.gws_bytes);
+    const bool tc = e.mode == TEAM_MODE_BF16 && K % 8 == 0 && lda % 8 == 0 && ldb % 8 == 0 && K >= 64;
     int rc;
-    const int64_t ar = ta ? K : M, ac = ta ? M : K, br = tb ? N : K, bc = tb ? K : N;
-    if ((rc = to_bf16(e.st, A, lda, ar, (int)ac, e.ha, nullptr, lda))) return rc;
-    if ((rc = to_bf16(e.st, B, ldb, br, (int)bc, e.hb, nullptr, ldb))) return rc;
-    TcGemm g;
-    memset(&g, 0, sizeof(g));
-    g.M = M; g.N = N; g.nseg = 1;
-    g.s[0].a_mn = ta; g.s[0].b_mn = !tb; g.s[0].K = K;
-    g.s[0].A = e.ha; g.s[0].lda = lda; g.s[0].B = e.hb; g.s[0].ldb = ldb;
-    g.alpha = 1.f; g.beta = beta; g.C = C; g.ldc = ldc; g.bias = bias;
-    return gemm_bf16_group(e.st, &g, 1, e.gws, e.gws_bytes);
+    if (tc) {
+        const int64_t ar = ta ? K : M, ac = ta ? M : K, br = tb ? N : K, bc = tb ? K : N;
+        if ((rc = to_bf16(e.st, A, lda, ar, (int)ac, e.ha, nullptr, lda))) return rc;
+        if ((rc = to_bf16(e.st, B, ldb, br, (int)bc, e.hb, nullptr, ldb))) return rc;
+    }
+    Wave wv;
+    seg(wv.add(M, N, beta, Mat{C, nullptr, ldc}, bias), ta, Mat{const_cast<float*>(A), e.ha, lda}, !tb, Mat{const_cast<float*>(B), e.hb, ldb}, K);
+    return run_wave(e.st, tc ? e.mode : TEAM_MODE_F32, wv, e.gws, e.gws_bytes);
 }
 
 struct MhaPlan {
