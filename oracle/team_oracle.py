@@ -249,12 +249,12 @@ def unicl_loss(image_features, text_features, state_features, labels, temperatur
         tau = temperature
     tri = torch.stack([im, tx, st], dim=1)                       # [B,3,D]
     sim = torch.matmul(tri, tri.transpose(1, 2)) / tau           # [B,3,3]
-    eye = torch.eye(3, dtype=sim.dtype)
+    eye = torch.eye(3, dtype=sim.dtype, device=sim.device)
     pos = torch.exp(sim * (1 - eye)).sum(-1)                     # self entry -> exp(0)
     allv = torch.exp(sim).sum(-1)
     instance = -(torch.log(pos / (allv + 1e-8))).sum() / (3 * B)
     lm = (labels.unsqueeze(1) == labels.unsqueeze(0)).to(sim.dtype)
-    sm = 1 - torch.eye(B, dtype=sim.dtype)
+    sm = 1 - torch.eye(B, dtype=sim.dtype, device=sim.device)
     lm = lm * sm
     ii = im @ im.t() / tau
     ex = torch.exp(ii - ii.max(dim=1, keepdim=True).values)
@@ -310,7 +310,7 @@ def clip_loss(image_features, text_features, logit_scale):
     """ClipLoss.forward, world_size 1: utils/toolkit.py:110-141."""
     li = logit_scale * image_features @ text_features.t()
     lt = logit_scale * text_features @ image_features.t()
-    y = torch.arange(li.shape[0])
+    y = torch.arange(li.shape[0], device=li.device)
     return (F.cross_entropy(li, y) + F.cross_entropy(lt, y)) / 2
 
 

@@ -112,7 +112,8 @@ static int adamw_launch(int32_t n_tensors, float* const* params, const float* co
     memset(&L, 0, sizeof(L));
     long long blocks = 0;
     for (int i = 0; i < n_tensors; ++i) {
-        TEAM_REQUIRE(params[i] && grads[i] && exp_avg[i] && exp_avg_sq[i] && numel[i] >= 0, "adamw: bad tensor %d", i);
+        // a tensor without elements may have null pointers (torch gives an empty tensor none): no block maps to it
+        TEAM_REQUIRE(numel[i] >= 0 && (numel[i] == 0 || (params[i] && grads[i] && exp_avg[i] && exp_avg_sq[i])), "adamw: bad tensor %d", i);
         L.p[i] = params[i]; L.g[i] = grads[i]; L.m[i] = exp_avg[i]; L.v[i] = exp_avg_sq[i]; L.n[i] = numel[i];
         L.blk0[i] = blocks;
         blocks += (numel[i] + 1023) / 1024;

@@ -264,6 +264,9 @@ class FusedAdamW:
         self.exp_avg = [torch.zeros_like(p) for p in self.params]
         self.exp_avg_sq = [torch.zeros_like(p) for p in self.params]
         self.steps = [0] * len(self.params)      # per tensor, like torch: a tensor without gradient does not advance
+        # step count of step_graph, created here rather than on first use: a first use inside a CUDA graph capture would
+        # allocate it from the graph's pool and capture its zero fill, so every replay would restart the count at 1
+        self.step_dev = torch.zeros((1,), dtype=torch.int64, device=self.params[0].device) if self.params else None
 
     @torch.no_grad()
     def step(self, grads=None):
@@ -298,8 +301,6 @@ class FusedAdamW:
         import ctypes as C
         if any(g is None for g in grads) or len(grads) != len(self.params):
             raise ValueError("step_graph needs one gradient per parameter")
-        if not hasattr(self, "step_dev"):
-            self.step_dev = torch.zeros((1,), dtype=torch.int64, device=self.params[0].device)
         L = capi.lib()
         idx = list(range(len(self.params)))
         for lo in range(0, len(idx), 48):

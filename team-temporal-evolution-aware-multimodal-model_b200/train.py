@@ -101,16 +101,13 @@ class TrainStep:
         with torch.cuda.stream(st):
             # warm-up outside the capture (lazy initialisation, autograd buffers) on a snapshot of the trainable state
             snap = [(p.detach().clone(), m.clone(), v.clone()) for p, m, v in zip(self.opt.params, self.opt.exp_avg, self.opt.exp_avg_sq)]
-            step0 = self.opt.step_dev.clone() if hasattr(self.opt, "step_dev") else None
+            step0 = self.opt.step_dev.clone()
             self._body(epoch)
             st.synchronize()
             with torch.no_grad():
                 for p, m, v, (p0, m0, v0) in zip(self.opt.params, self.opt.exp_avg, self.opt.exp_avg_sq, snap):
                     p.copy_(p0); m.copy_(m0); v.copy_(v0)
-                if step0 is not None:
-                    self.opt.step_dev.copy_(step0)
-                else:
-                    self.opt.step_dev.zero_()
+                self.opt.step_dev.copy_(step0)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, stream=st):
                 self._body(epoch)
