@@ -196,8 +196,8 @@ int team_head_tri_fwd(const team_head_weights* w, int mode, int64_t batch,
                       void* workspace, size_t workspace_bytes, void* stream);
 
 /* g_proto may be NULL = a zero cotangent for the prototype output (what the learner's losses produce: neither
- * unicl_loss nor ClipLoss reads proto_feats, models/proof.py:434-442); the C prototype query rows of every sample
- * are then skipped in the backward. */
+ * unicl_loss nor ClipLoss reads proto_feats, models/proof.py:434-442); heads of up to 22 classes then skip the C
+ * prototype query rows of every sample in the backward, larger heads run them with a zero cotangent. */
 int team_head_tri_bwd(const team_head_weights* w, int mode, int64_t batch,
                       const float* image_feat, const float* text_feat, const int64_t* state_ids,
                       const float* g_image, const float* g_text, const float* g_state,

@@ -548,7 +548,6 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
         TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_bwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
         TEAM_LAUNCH(table_rows_bwd2_kernel, tgrid, TW * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, state_ids, g_proto, g_state, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials, w.VFs.f + (size_t)d.Nsp * D);
     } else {
-        TEAM_REQUIRE(g_proto != nullptr, "head bwd: g_proto = NULL needs the warp-per-sample table-row kernel (C <= 22)");
         tgrid = d.B < d.nctas ? d.B : d.nctas;
         const size_t tsm = table_bwd_smem_floats(d) * sizeof(float);
         TEAM_REQUIRE(tsm <= 200 * 1024, "head bwd: too many classes for the table-row kernel (%d)", d.C);

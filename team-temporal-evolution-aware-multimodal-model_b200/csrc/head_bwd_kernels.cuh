@@ -41,6 +41,8 @@ __host__ __device__ inline size_t table_bwd_smem_floats(const HeadDims& d) {
 // a_t VT_b + a_s VS_b,  so  R = A1^T GG + A23^T VFo  (one two-segment tensor-core GEMM, K = 2B each) plus
 // rank-1 / table-row corrections assembled from the scalar sums in `scal` (expand_table_kernel).
 // A1 / A23 are [2B, ldA]: column tr holds the R coefficient, column ldA/2 + tr the G coefficient.
+// g_proto = NULL is a zero prototype cotangent: the prototype rows are still visited, with dY = 0 (a branch that skips
+// them makes ptxas spill more of this register-bound kernel).
 // dynamic smem: vec[5][D] (VI, VT, VS, gamma.*g_proto/C, gamma.*g_state) | lnp[2][D] (gamma, bfc) | slots[TQ_WARPS][4][D] | xst[D] |
 //               dvfst[10][D] | scal[Rt][TQ_NSC] | red[16]
 __global__ void __launch_bounds__(TQ_WARPS * 32, 3)
@@ -81,7 +83,7 @@ table_rows_bwd_kernel(HeadDims d, const float* __restrict__ SK, const float* __r
         __syncthreads();                                      // previous sample's slots / vec fully consumed
         {   // stage the sample's vectors; GG rows (cotangent .* gamma) for the coefficient GEMM; zero the sparse rows
             const float4 g4 = reinterpret_cast<const float4*>(lnp)[tid];
-            float4 gp = reinterpret_cast<const float4*>(g_proto + (size_t)b * D)[tid];
+            float4 gp = g_proto != nullptr ? reinterpret_cast<const float4*>(g_proto + (size_t)b * D)[tid] : make_float4(0.f, 0.f, 0.f, 0.f);
             const float4 gs = reinterpret_cast<const float4*>(g_state + (size_t)b * D)[tid];
             gp.x *= invC; gp.y *= invC; gp.z *= invC; gp.w *= invC;
             reinterpret_cast<float4*>(vec)[tid] = reinterpret_cast<const float4*>(VFo + (size_t)b * D)[tid];

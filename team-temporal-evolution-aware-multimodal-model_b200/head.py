@@ -610,7 +610,7 @@ class HeadStepRunner:
         return self.ws[off:off + 2 * self.B * capi.D * 4].view(torch.float32).view(2 * self.B, capi.D)
 
     def backward(self, image, text, sid, cots, g_own_rows: Optional[torch.Tensor] = None):
-        """``cots[3]`` (cotangent of the prototype output) may be None: the prototype rows are then skipped.
+        """``cots[3]`` (cotangent of the prototype output) may be None, a zero cotangent (team_head_tri_bwd).
         ``g_own_rows``: optional extra cotangent [2B,512] (or [2,B,512]) on ``own_rows()`` (``team_head_grads.g_own_rows``)."""
         if g_own_rows is not None and (g_own_rows.numel() != 2 * self.B * capi.D or g_own_rows.dtype != torch.float32
                                        or not g_own_rows.is_contiguous()):

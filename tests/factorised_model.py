@@ -1,5 +1,5 @@
 """Executable specification of the factorised head algorithm the CUDA kernels implement
-(DESIGN.md section 3).  Pure torch on CPU, fp64-capable, hand-written backward - no
+(DESIGN.md section 3).  Pure torch on the inputs' device, fp64-capable, hand-written backward - no
 autograd - so that the algebra (shared-row dedup, fc folded into V, table-query
 factorisation, batch-reduced shared gradients) is verified against the oracle before and
 independently of any CUDA code.  Lives in tests/: it is a test helper, not the product.
@@ -84,13 +84,14 @@ def head_fwd_bwd(p, image, text, sid, protos, cots):
     VFo = Vo @ Wfc.t()
     SQ = Qo @ Ks.t()                                   # own queries vs step keys   [2B, Ns]
     SK = Ko @ Qs.t()                                   # own keys vs step queries   [2B, Ns]
-    bidx = torch.arange(B)
+    dev = image.device
+    bidx = torch.arange(B, device=dev)
     rows_b = torch.cat([bidx, bidx])                   # sample of each own row
     scol = M + sid                                     # state column per sample
     # own query rows
-    mask = torch.zeros(2 * B, Ns, dtype=torch.bool)
+    mask = torch.zeros(2 * B, Ns, dtype=torch.bool, device=dev)
     mask[:, :M] = True
-    mask[torch.arange(2 * B), scol[rows_b]] = True
+    mask[torch.arange(2 * B, device=dev), scol[rows_b]] = True
     s_ext = torch.where(mask, SQ / tau, torch.full_like(SQ, -float("inf")))
     s_own = torch.stack([(Qo * Ko[rows_b]).sum(-1), (Qo * Ko[rows_b + B]).sum(-1)], 1) / tau   # vs img key, text key
     mx = torch.maximum(s_ext.max(1).values, s_own.max(1).values).unsqueeze(1)
@@ -101,7 +102,7 @@ def head_fwd_bwd(p, image, text, sid, protos, cots):
     out_o, xh_o, rstd_o = _ln(Ybar_o + bfc + Xo, gam, bet)
     out_img, out_txt = out_o[:B], out_o[B:]
     # table query rows, per sample: rows r in [0,C) and the state row
-    rt = torch.cat([torch.arange(C).unsqueeze(0).expand(B, C), scol.unsqueeze(1)], 1)      # [B, C+1] step-row ids
+    rt = torch.cat([torch.arange(C, device=dev).unsqueeze(0).expand(B, C), scol.unsqueeze(1)], 1)      # [B, C+1] step-row ids
     s_i = SK[:B].gather(1, rt) / tau                   # vs own image key
     s_t = SK[B:].gather(1, rt) / tau                   # vs own text key
     s_s = TT[rt, scol.unsqueeze(1).expand(B, C + 1)] / tau   # vs own state key
@@ -127,18 +128,18 @@ def head_fwd_bwd(p, image, text, sid, protos, cots):
     dgam += (go_t * xh_t).sum((0, 1)); dbet += go_t.sum((0, 1))
     du_t = _ln_bwd(go_t, xh_t, rstd_t, gam)            # [B, C+1, D] = dY = residual grad
     dbfc += du_t.sum((0, 1))
-    R = torch.zeros(Ns, D, dtype=S.dtype).index_add_(0, rt.reshape(-1), du_t.reshape(-1, D))
+    R = torch.zeros(Ns, D, dtype=S.dtype, device=dev).index_add_(0, rt.reshape(-1), du_t.reshape(-1, D))
     w = 1.0 / den_t
     dot_yy = (du_t * Ybar_t).sum(-1)                   # dY . Ybar
-    G = torch.zeros(Ns, D, dtype=S.dtype).index_add_(0, rt.reshape(-1), ((c * w).unsqueeze(-1) * du_t).reshape(-1, D))
-    h = torch.zeros(Ns, dtype=S.dtype).index_add_(0, rt.reshape(-1), (c * w * dot_yy).reshape(-1))
+    G = torch.zeros(Ns, D, dtype=S.dtype, device=dev).index_add_(0, rt.reshape(-1), ((c * w).unsqueeze(-1) * du_t).reshape(-1, D))
+    h = torch.zeros(Ns, dtype=S.dtype, device=dev).index_add_(0, rt.reshape(-1), (c * w * dot_yy).reshape(-1))
     a_i, a_t, a_s = p_i * w, p_t * w, p_s * w
     ds_i = a_i * ((du_t * VFo[:B].unsqueeze(1)).sum(-1) - dot_yy) / tau
     ds_t = a_t * ((du_t * VFo[B:].unsqueeze(1)).sum(-1) - dot_yy) / tau
     ds_s = a_s * ((du_t * VFst.unsqueeze(1)).sum(-1) - dot_yy) / tau
-    dSK = torch.zeros(2 * B, Ns, dtype=S.dtype)
+    dSK = torch.zeros(2 * B, Ns, dtype=S.dtype, device=dev)
     dSK[:B].scatter_(1, rt, ds_i); dSK[B:].scatter_(1, rt, ds_t)
-    dTT = torch.zeros(Ns, Ns, dtype=S.dtype)
+    dTT = torch.zeros(Ns, Ns, dtype=S.dtype, device=dev)
     dTT.index_put_((rt.reshape(-1), scol.unsqueeze(1).expand(B, C + 1).reshape(-1)), ds_s.reshape(-1), accumulate=True)
     dVFo = torch.zeros_like(VFo)
     dVFo[:B] += (a_i.unsqueeze(-1) * du_t).sum(1); dVFo[B:] += (a_t.unsqueeze(-1) * du_t).sum(1)

@@ -406,8 +406,8 @@ def _reference_step(p64, params, protos, text_cls, evo, batch, epoch, ts, names)
         return [float(v.detach()) for v in (total, ce, cl, un, inst)], grads, _clip_conditioning(ei, et, ls)
     # T = 10, B = 1024: the factorised head (pinned to the oracle by tests/test_quantised_model.py) with cotangents
     # from autograd through the oracle's unicl_loss, plus the ClipLoss gradient through the projections
-    zeros = [torch.zeros(B, 512, dtype=torch.float64), torch.zeros(B, 1, 512, dtype=torch.float64),
-             torch.zeros(B, 512, dtype=torch.float64), torch.zeros(B, 512, dtype=torch.float64)]
+    z = dict(dtype=torch.float64, device=img.device)
+    zeros = [torch.zeros(B, 512, **z), torch.zeros(B, 1, 512, **z), torch.zeros(B, 512, **z), torch.zeros(B, 512, **z)]
     outs, _ = head_fwd_bwd(p64, img, txt, sid, pr, zeros)
     o = [t.detach().clone().requires_grad_(True) for t in outs[:3]]
     un, inst, _ = O.unicl_loss(o[0], o[1], o[2], y, epoch=epoch, max_epoch=ts.tuned_epoch, state_ids=sid,
@@ -433,7 +433,7 @@ def _clip_conditioning(ei, et, ls):
     their relative error is about this factor times the bf16 rounding."""
     with torch.no_grad():
         L = ls * ei @ et.t()
-        G = torch.softmax(L, 1) + torch.softmax(L.t(), 1).t() - 2 * torch.eye(L.shape[0], dtype=L.dtype)
+        G = torch.softmax(L, 1) + torch.softmax(L.t(), 1).t() - 2 * torch.eye(L.shape[0], dtype=L.dtype, device=L.device)
         return max(float((G.abs() @ et.abs()).norm() / (G @ et).norm()),
                    float((G.abs().t() @ ei.abs()).norm() / (G.t() @ ei).norm()))
 
