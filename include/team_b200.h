@@ -174,6 +174,29 @@ typedef struct team_head_grads {            /* all OVERWRITTEN by team_head_tri_
 
 size_t team_head_workspace_bytes(int64_t batch, int32_t num_classes, int32_t num_prompts,
                                  int32_t num_text_cls, int mode);
+
+/* Train-mode dropout of sel_attn inside team_head_tri_fwd / team_head_tri_bwd (convs/projections.py:28, :62, :84): the
+ * attention probabilities and the fc output are masked exactly as team_mha_fwd masks the token tensor
+ * [image | text | state | C prototypes | P prompts] (L = 3 + C + P) of every sample: probability (b L + i) L + j with the
+ * Philox stream (seed, offset), fc element (b L + i) 512 + c with (seed, offset + 1); kept iff the output is >= p 2^32,
+ * kept values scaled by 1 / (1 - p).  Only the query tokens i < 3 + C are computed (the prompt outputs are discarded).
+ * offset_dev, if not NULL, is read on the device and overrides offset (a replayed CUDA graph then draws the masks of
+ * whatever offset the device holds).  workspace: team_head_dropout_workspace_bytes, untouched between the forward and
+ * the backward of one step, 256-byte aligned.  p = 0 (or a NULL team_dropout*) runs the undropped head. */
+typedef struct team_dropout {
+    float p;
+    uint64_t seed;
+    uint64_t offset;
+    const uint64_t* offset_dev;
+    void* workspace;
+    size_t workspace_bytes;
+} team_dropout;
+/* Bytes of the dropout workspace, linear in the batch: about (C + 1) B (10 Nsp + 7 200) + 12 B Nsp in BF16 mode and
+ * (C + 1) B (8 Nsp + 6 176) + 8 B Nsp in F32 mode (Nsp = C + P + 10 rounded up to 16): 188 MB at B = 1024, C = 20, P = 100. */
+size_t team_head_dropout_workspace_bytes(int64_t batch, int32_t num_classes, int32_t num_prompts, int mode);
+/* *p += v on the device, on `stream` (one thread, no host sync; capturable): advances team_dropout.offset_dev by 2 per
+ * step, so the replays of a captured step draw fresh masks. */
+int team_u64_add(uint64_t* p, uint64_t v, void* stream);
 /* Byte offset, inside the workspace of team_head_tri_fwd (same arguments as team_head_workspace_bytes), of the
  * [2B,512] fp32 rows normalize(encode_image(x)) | normalize(encode_text(t)) the forward leaves there (valid until the
  * matching team_head_tri_bwd): the inputs of the ClipLoss branch, models/proof.py:428-430. */
@@ -193,16 +216,17 @@ int team_head_tri_fwd(const team_head_weights* w, int mode, int64_t batch,
                       const float* text_cls, int64_t num_text_cls,
                       float* out_image, float* out_text, float* out_state, float* out_proto,
                       float* cls_logits, int64_t* cls_argmax,
-                      void* workspace, size_t workspace_bytes, void* stream);
+                      void* workspace, size_t workspace_bytes, void* stream, const team_dropout* dropout);
 
 /* g_proto may be NULL = a zero cotangent for the prototype output (what the learner's losses produce: neither
  * unicl_loss nor ClipLoss reads proto_feats, models/proof.py:434-442); heads of up to 22 classes then skip the C
- * prototype query rows of every sample in the backward, larger heads run them with a zero cotangent. */
+ * prototype query rows of every sample in the backward, larger heads run them with a zero cotangent.
+ * dropout: the team_dropout of the matching forward (same p, seed, offset and workspace). */
 int team_head_tri_bwd(const team_head_weights* w, int mode, int64_t batch,
                       const float* image_feat, const float* text_feat, const int64_t* state_ids,
                       const float* g_image, const float* g_text, const float* g_state,
                       const float* g_proto, const team_head_grads* grads,
-                      void* workspace, size_t workspace_bytes, void* stream);
+                      void* workspace, size_t workspace_bytes, void* stream, const team_dropout* dropout);
 
 /* encode_* alone (utils/inc_net.py:401-422, :518-526): out = [normalize](sum_t x W_t^T + b_t).
  * which: 0 image, 1 text, 2 state (x = state_ids int64, embedding gather fused), 3 prototypes

@@ -53,6 +53,11 @@ class HeadGrads(C.Structure):
                                                                                                   ("g_own_rows", C.c_void_p)]
 
 
+class Dropout(C.Structure):
+    _fields_ = [("p", C.c_float), ("seed", C.c_uint64), ("offset", C.c_uint64), ("offset_dev", C.c_void_p),
+                ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+
+
 class TgcnBlock(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in
                 ("msg_w", "msg_b", "msg_ln_g", "msg_ln_b", "upd_w", "upd_b", "upd_ln_g", "upd_ln_b", "gate_w", "gate_b")]
@@ -125,10 +130,14 @@ def _declare(lib):
         lib.team_head_own_rows_offset.argtypes = [i64, C.c_int32, C.c_int32, C.c_int32, i32]
         lib.team_head_tri_fwd.restype = i32
         lib.team_head_tri_fwd.argtypes = [C.POINTER(HeadWeights), i32, i64, vp, vp, vp, vp, i64,
-                                          vp, vp, vp, vp, vp, vp, vp, sz, vp]
+                                          vp, vp, vp, vp, vp, vp, vp, sz, vp, C.POINTER(Dropout)]
         lib.team_head_tri_bwd.restype = i32
         lib.team_head_tri_bwd.argtypes = [C.POINTER(HeadWeights), i32, i64, vp, vp, vp, vp, vp, vp, vp,
-                                          C.POINTER(HeadGrads), vp, sz, vp]
+                                          C.POINTER(HeadGrads), vp, sz, vp, C.POINTER(Dropout)]
+        lib.team_head_dropout_workspace_bytes.restype = sz
+        lib.team_head_dropout_workspace_bytes.argtypes = [i64, C.c_int32, C.c_int32, i32]
+        lib.team_u64_add.restype = i32
+        lib.team_u64_add.argtypes = [vp, C.c_uint64, vp]
         lib.team_head_encode.restype = i32
         lib.team_head_encode.argtypes = [C.POINTER(HeadWeights), i32, i32, vp, i64, i32, vp, vp, sz, vp]
         lib.team_peer_allreduce_flag_bytes.restype = sz

@@ -99,6 +99,38 @@ __device__ __forceinline__ uint2 pack_bf16x4(float4 v) {
     return o;
 }
 
+// ------------------------------------------------------------------------------------------------ dropout masks
+// Train-mode dropout of the block (attention probabilities and fc output, p = 0.1 in the reference: convs/projections.py:28,
+// :62, :84) as COUNTER-BASED masks: element i of a tensor is kept iff philox4x32-10(key = seed, counter = (i / 4, offset))
+// [i % 4] * 2^-32 >= p.  Nothing is stored: the backward regenerates the mask from the same (seed, offset).  The stream is
+// this library's own (torch's Philox offsets depend on its launch geometry and cannot be reproduced), so parity in train
+// mode is checked against the reference math with the SAME masks (oracle/team_oracle.py:philox_keep_mask) and statistically.
+struct Philox {
+    uint32_t k0, k1;
+    uint64_t offset;
+};
+__host__ __device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1, n3 = (uint32_t)p0;
+    c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
+}
+// the four 32-bit outputs of counter block `blk`
+__host__ __device__ __forceinline__ void philox4(const Philox& g, uint64_t blk, uint32_t (&c)[4]) {
+    c[0] = (uint32_t)blk; c[1] = (uint32_t)(blk >> 32); c[2] = (uint32_t)g.offset; c[3] = (uint32_t)(g.offset >> 32);
+    uint32_t k0 = g.k0, k1 = g.k1;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        philox_round(c, k0, k1);
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+}
+// keep-scale of element idx: 0 (dropped) or 1 / (1 - p); thr = p * 2^32
+__device__ __forceinline__ float drop_scale(const Philox& g, uint64_t idx, uint32_t thr, float inv_keep) {
+    uint32_t c[4];
+    philox4(g, idx >> 2, c);
+    return c[idx & 3] >= thr ? inv_keep : 0.f;
+}
+
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 }  // namespace team

@@ -7,6 +7,7 @@
 #include "head_proof_kernels.cuh"
 #include "head_table_kernels.cuh"
 #include "head_table_gram.cuh"
+#include "head_dropout_kernels.cuh"
 
 namespace team {
 
@@ -76,6 +77,69 @@ void head_plan(const HeadDims& d, int mode, void* base, HeadWS* w) {
     w->tcls = mat((size_t)(d.Tc > 0 ? d.Tc : 1), D, false);
     w->Zc = take((size_t)(d.Tc > 0 ? d.Tc : 1) * D);
     w->total_bytes = off;
+}
+
+// Workspace of the dropout route (team_head_dropout_workspace_bytes), NT = B (C + 1) table-query rows.
+struct DropWS {
+    Mat Ad;              // [B2][Nsp]  masked own-row probabilities
+    float* aownd;        // [B2][2]    masked own-key probabilities
+    Mat Wd;              // [NT][Nsp]  masked table-row probabilities
+    float* tsc;          // [NT][DROP_NSC] row scalars
+    float* Yt;           // [NT][D]    Wd VFs, then Ybar of the table rows
+    Mat dYt;             // [NT][D]    gradient of the fc output of the table rows
+    float* dU;           // [NT][D]    residual gradient of the table rows
+    float* dWd;          // [NT][Nsp]  dYt VFs^T
+    float* tpart;        // [NUM_SMS][OWN_PARTIAL_LEN] per-CTA partials of drop_table_bwd_kernel
+    size_t total_bytes;
+};
+static void drop_plan(const HeadDims& d, int mode, void* base, DropWS* w) {
+    size_t off = 0;
+    const bool bf = mode == TEAM_MODE_BF16;
+    auto take_bytes = [&](size_t bytes) -> char* {
+        char* p = base ? reinterpret_cast<char*>(base) + off : nullptr;
+        off += align_up(bytes, 256);
+        return p;
+    };
+    auto take = [&](size_t n) -> float* { return reinterpret_cast<float*>(take_bytes(n * sizeof(float))); };
+    auto mat = [&](size_t rows, size_t cols) -> Mat {
+        Mat m;
+        m.f = take(rows * cols);
+        m.h = bf ? reinterpret_cast<__nv_bfloat16*>(take_bytes(rows * cols * 2)) : nullptr;
+        m.ld = (int64_t)cols;
+        return m;
+    };
+    const size_t NT = (size_t)d.B * (d.C + 1);
+    w->Ad = mat(d.B2, d.Nsp); w->aownd = take((size_t)d.B2 * 2);
+    w->Wd = mat(NT, d.Nsp); w->tsc = take(NT * DROP_NSC);
+    w->Yt = take(NT * D); w->dYt = mat(NT, D); w->dU = take(NT * D); w->dWd = take(NT * d.Nsp);
+    w->tpart = take((size_t)NUM_SMS * OWN_PARTIAL_LEN);
+    w->total_bytes = off;
+}
+
+// A team_dropout with p > 0, checked, and its workspace laid out; on = false: the undropped head.
+struct DropCfg {
+    bool on = false;
+    DropArgs a;
+    DropWS w;
+};
+static int drop_setup(const HeadDims& d, int mode, const team_dropout* dr, DropCfg* c) {
+    c->on = false;
+    if (dr == nullptr || dr->p == 0.f) return TEAM_OK;
+    TEAM_REQUIRE(dr->p > 0.f && dr->p < 1.f, "head dropout: p = %g out of [0, 1)", (double)dr->p);
+    drop_plan(d, mode, dr->workspace, &c->w);
+    if (dr->workspace == nullptr || dr->workspace_bytes < c->w.total_bytes) {
+        set_error("head dropout: workspace %zu < %zu bytes", dr->workspace_bytes, c->w.total_bytes);
+        return TEAM_EWORKSPACE;
+    }
+    TEAM_REQUIRE((reinterpret_cast<uintptr_t>(dr->workspace) & 255) == 0, "head dropout: workspace must be 256-byte aligned");
+    c->on = true;
+    c->a.attn = Philox{(uint32_t)dr->seed, (uint32_t)(dr->seed >> 32), dr->offset};
+    const double t = (double)dr->p * 4294967296.0;
+    c->a.thr = t >= 4294967295.0 ? 4294967295u : (uint32_t)t;
+    c->a.inv_keep = 1.f / (1.f - dr->p);
+    c->a.offset_dev = dr->offset_dev;
+    c->a.L = 3 + d.M;
+    return TEAM_OK;
 }
 
 struct HeadCtx {
@@ -362,237 +426,49 @@ static int shared_rows_fwd(HeadCtx& cx, const team_head_weights* hw, const float
     return TEAM_OK;
 }
 
-}  // namespace team
-
-using namespace team;
-
-extern "C" size_t team_head_workspace_bytes(int64_t batch, int32_t num_classes, int32_t num_prompts,
-                                            int32_t num_text_cls, int mode) {
-    HeadDims d = head_dims(batch, num_classes, num_prompts, num_text_cls);
-    HeadWS w;
-    head_plan(d, mode, nullptr, &w);
-    return w.total_bytes;
-}
-
-extern "C" int team_head_frozen_sums(const team_head_weights* hw, int32_t num_frozen, float* w_sums, float* b_sums, void* stream) {
-    TEAM_REQUIRE(hw != nullptr && w_sums != nullptr && b_sums != nullptr, "head frozen sums: null pointer");
-    TEAM_REQUIRE(num_frozen >= 1 && num_frozen <= hw->num_tasks && hw->num_tasks <= TEAM_MAX_TASKS, "head frozen sums: num_frozen %d out of [1, %d]", num_frozen, hw->num_tasks);
-    PrepSum ps;
-    memset(&ps, 0, sizeof(ps));
-    const float* const* Ws[3] = {hw->w_img, hw->w_text, hw->w_state};
-    const float* const* Bs[3] = {hw->b_img, hw->b_text, hw->b_state};
-    for (int k = 0; k < 3; ++k) {
-        for (int t = 0; t < num_frozen; ++t) TEAM_REQUIRE(Ws[k][t] != nullptr && Bs[k][t] != nullptr, "head frozen sums: null projection %d of task %d", k, t);
-        ps.W[k] = plist(Ws[k], num_frozen); ps.Bv[k] = plist(Bs[k], num_frozen);
-        ps.Wout[k] = w_sums + (size_t)k * D * D; ps.Wh[k] = nullptr; ps.bout[k] = b_sums + (size_t)k * D;
-    }
-    ps.n = 3;
-    ConvList cl;
-    memset(&cl, 0, sizeof(cl));
-    cl.sum_blocks = 3 * PREP_SUM_BLOCKS_PER_W;
-    TEAM_LAUNCH(prep_kernel, cl.sum_blocks, 256, 0, (cudaStream_t)stream, ps, cl);
-    return TEAM_OK;
-}
-
-// byte offset of the normalised projected own rows Xo ([2B,512] fp32: image rows, then text rows) inside the workspace
-extern "C" size_t team_head_own_rows_offset(int64_t batch, int32_t num_classes, int32_t num_prompts, int32_t num_text_cls, int mode) {
-    HeadDims d = head_dims(batch, num_classes, num_prompts, num_text_cls);
-    HeadWS w;
-    head_plan(d, mode, reinterpret_cast<void*>(uintptr_t(256)), &w);          // a non-null fake base: only the offsets are used
-    return (size_t)(reinterpret_cast<uintptr_t>(w.Xo.f) - 256);
-}
-
-// Forward: 13 launches (prologue, prompt rows, 4 GEMM waves, 7 row kernels; three short side-lane branches) - see
-// DESIGN.md section 4.
-extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t batch, const float* image_feat,
-                                 const float* text_feat, const int64_t* state_ids, const float* text_cls,
-                                 int64_t num_text_cls, float* out_image, float* out_text, float* out_state,
-                                 float* out_proto, float* cls_logits, int64_t* cls_argmax, void* workspace,
-                                 size_t workspace_bytes, void* stream) {
-    HeadCtx cx;
-    int rc = setup(cx, "head", hw, mode, batch, 0, (int)(text_cls ? num_text_cls : 0), workspace, workspace_bytes, stream);
-    if (rc) return rc;
-    TEAM_REQUIRE(image_feat && text_feat && state_ids && out_image && out_text && out_state && out_proto, "head fwd: null pointer");
-    TEAM_REQUIRE(hw->w_q && hw->w_k && hw->w_v && hw->w_fc && hw->b_fc && hw->ln_g && hw->ln_b && hw->state_emb && hw->prototypes, "head fwd: null weight");
+// Forward of the dropout route from the score matrices on (after GEMM wave 3): the two softmax kernels as in the undropped
+// forward, the masked probability rows, GEMM wave 4 with one product per probability set, and the fc / LayerNorm rows.
+static int drop_fwd(HeadCtx& cx, const team_head_weights* hw, const DropCfg& dc, const int64_t* state_ids, bool want_cls,
+                    float* cls_logits, int64_t* cls_argmax, float* out_image, float* out_text, float* out_state, float* out_proto) {
     const HeadDims& d = cx.d;
     HeadWS& w = cx.w;
-    const bool want_cls = d.Tc > 0 && (cls_logits != nullptr || cls_argmax != nullptr);
-    bind_inputs(cx, hw, image_feat, text_feat, text_cls);
+    const DropWS& dw = dc.w;
+    int rc;
     SideStream* side = nullptr;
-    const int fill_rows = d.P + (d.Nsp - d.Ns);
-    if (fill_rows > 0) {          // prompt rows of S: independent of the prologue -> side lane
-        const cudaStream_t fst = fork_side(cx.st, &side);
-        TEAM_LAUNCH(fill_prompt_rows_kernel, fill_rows, 128, 0, fst, plist(hw->prompts, hw->num_tasks), hw->prompts_per_task > 0 ? hw->prompts_per_task : 1, d.C, d.Ns, d.Nsp, w.S.f, w.S.h);
-    }
-    if ((rc = prologue(cx, hw, 3, image_feat, text_feat, want_cls ? text_cls : nullptr, batch))) return rc;
-    SideStream* fill_side = side;        // joined before wave 2 (the first reader of the prompt rows): wave 1 chains straight behind the prologue
-    Wave wv;
-    // ---- wave 1: every projection of the step (prototype rows, state table, image rows, text rows, class text)
-    seg(wv.add(d.C, D, 0.f, fonly(w.Ztab, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
-    seg(wv.add(10, D, 0.f, fonly(w.Ztab + (size_t)d.C * D, D), w.bsum[2]), false, w.E, false, w.Wsum[2], D);
-    seg(wv.add(d.B, D, 0.f, fonly(w.Xo.f, D), w.bsum[0]), false, w.img, false, w.Wsum[0], D);
-    seg(wv.add(d.B, D, 0.f, fonly(w.Xo.f + (size_t)d.B * D, D), w.bsum[1]), false, w.txt, false, w.Wsum[1], D);
-    if (want_cls) seg(wv.add(d.Tc, D, 0.f, fonly(w.Zc, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
-    RUN(wv);
-    {   // L2-normalise: prototype rows -> S[0,C), state table -> S[M,M+10), own rows in place
-        NormList nl;
-        memset(&nl, 0, sizeof(nl));
-        nl.do_normalize = 1;
-        int blocks = 0;
-        norm_add(nl, blocks, w.Ztab, w.S.f, w.S.h, w.invS, d.C);
-        norm_add(nl, blocks, w.Ztab + (size_t)d.C * D, w.S.f + (size_t)d.M * D, w.S.h ? w.S.h + (size_t)d.M * D : nullptr, w.invS + d.M, 10);
-        norm_add(nl, blocks, w.Xo.f, w.Xo.f, w.Xo.h, w.invo, d.B2);
-        TEAM_LAUNCH(rows_normalize_kernel, blocks, 256, 0, cx.st, nl);
-    }
-    if ((rc = join_side(cx.st, fill_side))) return rc;
-    // waves 2 and 3; VFo keeps its bf16 shadow (GEMM operand of the backward and of the Gram table rows)
-    if ((rc = qkv_score_waves(cx, d.B2, w.VFo))) return rc;
-    SideStream* gram_side = nullptr;
-    {   // the two softmax kernels (step-row table, own rows) are independent
+    {
         const cudaStream_t tst = fork_side(cx.st, &side);
-        const bool gram = use_table_gram(d);
-        const int xwarps = TG_RP;                            // + the s rows S_r + b_fc (bulk-copy source of the table-row kernels; Gram operand)
-        TEAM_LAUNCH(table_prep_kernel, (d.Nsp + xwarps + 7) / 8, 256, 0, tst, w.TT, d.M, d.Nsp, w.mt, w.Zt, w.Pt.f, w.Pt.h, w.S.f, hw->b_fc,
-                    w.VFs.f, (const __nv_bfloat16*)w.VFs.h, d.C, TG_RP,
-                    w.VFs.f + (size_t)d.Nsp * D, w.VFs.h ? w.VFs.h + (size_t)d.Nsp * D : (__nv_bfloat16*)nullptr);
-        if (gram)             // ... and its n rows
-            TEAM_LAUNCH(table_nf_kernel, d.Rt, 256, ((d.M + 3) / 4 * 4 + 512) * sizeof(float), tst, w.TT, d.M, d.Nsp, d.C, w.VFs.f, (const __nv_bfloat16*)w.VFs.h,
-                        w.VFs.f + (size_t)(d.Nsp + TG_RP) * D, w.VFs.h ? w.VFs.h + (size_t)(d.Nsp + TG_RP) * D : (__nv_bfloat16*)nullptr);
-        TEAM_LAUNCH(attn_own_kernel, (d.B2 + 7) / 8, 256, 0, cx.st, d, w.SQ.f, w.QKVo.f, cx.mode == TEAM_MODE_BF16 ? w.QKVo.h : nullptr, state_ids, w.Aext.f, w.Aext.h, w.aown);
+        TEAM_LAUNCH(table_prep_kernel, (d.Nsp + 7) / 8, 256, 0, tst, w.TT, d.M, d.Nsp, w.mt, w.Zt, w.Pt.f, (__nv_bfloat16*)nullptr, (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, (const __nv_bfloat16*)nullptr, 0, 0, (float*)nullptr, (__nv_bfloat16*)nullptr);
+        TEAM_LAUNCH(attn_own_kernel, (d.B2 + 7) / 8, 256, 0, cx.st, d, w.SQ.f, w.QKVo.f, cx.mode == TEAM_MODE_BF16 ? w.QKVo.h : nullptr, state_ids, w.Aext.f, (__nv_bfloat16*)nullptr, w.aown);
         if ((rc = join_side(cx.st, side))) return rc;
-        // step-level dot products of the table rows: beside GEMM wave 4 (joined before the table-row kernel)
-        if (gram) TEAM_LAUNCH(table_gram_prep_kernel, (d.Rt + 10 + 7) / 8, 256, 0, side != nullptr ? side->st : cx.st, d.Rt, w.VFs.f + (size_t)d.Nsp * D, w.VFs.f + (size_t)d.M * D, w.GT);
-        gram_side = gram ? side : nullptr;
     }
-    // ---- wave 4: probabilities x (fc-space) values
-    seg(wv.add(d.Nsp, D, 0.f, fonly(w.NFt, D)), false, w.Pt, true, w.VFs, d.Nsp);
-    seg(wv.add(d.B2, D, 0.f, fonly(w.Ybo, D)), false, w.Aext, true, w.VFs, d.Nsp);
-    // sample x table dot products of the table-query rows (head_table_gram.cuh): W0 = VFo x [VFs ; S_table + b_fc]^T
-    if (use_table_gram(d)) seg(wv.add(d.B2, tg_ldw(d), 0.f, fonly(w.W0, tg_ldw(d))), false, w.VFo, false, w.VFs, D);
+    const int64_t NT = (int64_t)d.B * (d.C + 1);
+    const int own_blocks = (d.B2 + 7) / 8;
+    TEAM_LAUNCH(drop_probs_kernel, own_blocks + (NT + 7) / 8, 256, 0, cx.st, d, dc.a, own_blocks, (const float*)w.Aext.f, (const float*)w.aown, state_ids, (const float*)w.SK, (const float*)w.TT, (const float*)w.mt, (const float*)w.Zt, (const float*)w.Pt.f, dw.Ad.f, dw.Ad.h, dw.aownd, dw.Wd.f, dw.Wd.h, dw.tsc);
+    // ---- wave 4: masked probabilities x (fc-space) values
+    Wave wv;
+    seg(wv.add(d.B2, D, 0.f, fonly(w.Ybo, D)), false, dw.Ad, true, w.VFs, d.Nsp);
+    seg(wv.add(NT, D, 0.f, fonly(dw.Yt, D)), false, dw.Wd, true, w.VFs, d.Nsp);
     RUN(wv);
-    // the own-row outputs and the classification logits do not depend on the table-query rows: side stream
-    const cudaStream_t sst = fork_side(cx.st, &side);
-    TEAM_LAUNCH(ln_own_fwd_kernel, (d.B2 + 7) / 8, 256, 0, sst, d, w.Ybo, w.aown, w.VFo.f, w.Xo.f, hw->b_fc, hw->ln_g, hw->ln_b, out_image, out_text);
-    // forward_for_classification (models/proof.py:519-536; image rows are already normalised in Xo): a third lane beside the
-    // own-row LayerNorm and the table rows.  Measured alternatives (tools/timeline.py, profiles/r2z_timeline_*): behind
-    // ln_own_fwd on the same lane the pair outlasts the table rows by 5 us; forked right after the normalisation (its inputs
-    // are ready there, 45 us of slack) it slows GEMM waves 2 and 3 by more than it saves (0.194 vs 0.189 ms per step), at the
-    // lowest stream priority as well - the kernels of one step compete for the same SMs and L2 bandwidth.
     SideStream* cls_side = nullptr;
     if (want_cls) {
         const cudaStream_t cst = fork_side(cx.st, &cls_side, 2);
         if ((rc = cosine_logits_launch(cst, w.Xo.f, d.B, w.Zc, d.Tc, nullptr, cls_logits, cls_argmax))) return rc;
     }
-    if (use_table_gram(d)) {      // Gram formulation: scalar LayerNorm algebra per (sample, row), vector outputs as coefficient sums
-        if ((rc = join_side(cx.st, gram_side))) return rc;          // table_gram_prep_kernel
-        const int nw = tg_warps(d), groups = (d.B + nw - 1) / nw;
-        const size_t tsm = tg_fwd_smem_floats(d) * sizeof(float);
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_gram_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
-        TEAM_LAUNCH(table_gram_fwd_kernel, groups < NUM_SMS ? groups : NUM_SMS, nw * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.VFs.f + (size_t)d.Nsp * D, w.GT, w.W0, w.VFo.f, w.VFs.f, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state, w.xs, w.xst, w.RS);
-    } else if (use_table2(d)) {   // warp per sample, table rows resident in shared memory (head_table_kernels.cuh)
-        const int groups = (d.B + TW - 1) / TW;
-        const size_t tsm = table2_fwd_smem_floats(d) * sizeof(float);
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
-        TEAM_LAUNCH(table_rows_fwd2_kernel, groups < NUM_SMS ? groups : NUM_SMS, TW * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state, w.VFs.f + (size_t)d.Nsp * D);
-    } else {
-        const int tgrid = d.B < 6 * NUM_SMS ? d.B : 6 * NUM_SMS;
-        TEAM_LAUNCH(table_rows_fwd_kernel, tgrid, TQ_WARPS * 32, 0, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state);
-    }
-    if ((rc = join_side(cx.st, side))) return rc;
-    if ((rc = join_side(cx.st, cls_side))) return rc;
-    return TEAM_OK;
+    TEAM_LAUNCH(drop_ln_fwd_kernel, own_blocks + (d.B + 7) / 8, 256, 0, cx.st, d, dc.a, own_blocks, w.Ybo, (const float*)dw.aownd, dw.Yt, (const float*)dw.tsc, (const float*)w.VFo.f, (const float*)w.Xo.f, (const float*)w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_image, out_text, out_state, out_proto);
+    return join_side(cx.st, cls_side);
 }
 
-// Backward: 13 launches at the headline size (5 GEMM waves, 8 row kernels; more when split-K runs through the fix-up
-// kernel or the gradient exchange is folded in); needs the workspace of the matching forward call.
-extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t batch, const float* image_feat,
-                                 const float* text_feat, const int64_t* state_ids, const float* g_image,
-                                 const float* g_text, const float* g_state, const float* g_proto,
-                                 const team_head_grads* gr, void* workspace, size_t workspace_bytes, void* stream) {
-    HeadCtx cx;
-    int rc = setup(cx, "head", hw, mode, batch, 0, 0, workspace, workspace_bytes, stream);
-    if (rc) return rc;
-    TEAM_REQUIRE(gr && g_image && g_text && g_state && image_feat && text_feat && state_ids, "head bwd: null pointer");
-    TEAM_REQUIRE(gr->w_img && gr->b_img && gr->w_text && gr->b_text && gr->w_state && gr->b_state && gr->state_emb &&
-                 gr->w_q && gr->w_k && gr->w_v && gr->w_fc && gr->b_fc && gr->ln_g && gr->ln_b, "head bwd: null gradient buffer");
+// The backward from GEMM wave 7 on (score gradients dS / dSK / dTT, dVFo, dVFs, Rfull and the LayerNorm / bias partials are
+// complete): shared by the undropped head and the dropout route.
+static int bwd_tail(HeadCtx& cx, const team_head_grads* gr) {
     const HeadDims& d = cx.d;
     HeadWS& w = cx.w;
-    bind_inputs(cx, hw, image_feat, text_feat, nullptr);
-    const TabOff to = tab_offsets(d);
-    const bool bf = cx.mode == TEAM_MODE_BF16;
-    // ---- own query rows: independent of the table-query rows -> side lane, beside them (its dVF part goes to dVFo_own)
-    int ogrid = (d.B + 7) / 8;
-    if (ogrid > NUM_SMS) ogrid = NUM_SMS;
-    SideStream* own_side = nullptr;
-    // (Enqueueing the table-row kernel first - it needs a whole register file per CTA and cannot share an SM with these two -
-    // was measured: it then runs alone in 26 us, but the own-row kernels are squeezed onto the 20 remaining SMs and finish
-    // later than before: 0.1948 vs 0.1885 ms per step, tools/timeline.py.)
-    const cudaStream_t ost = fork_side(cx.st, &own_side);
-    TEAM_LAUNCH(ln_own_bwd_kernel, ogrid, 256, 0, ost, d, w.Ybo, w.Xo.f, w.VFo.f, w.aown, hw->b_fc, hw->ln_g, hw->ln_b, g_image, g_text, w.dYo.f, w.dYo.h, w.dXo.f, w.rowdot, w.dsown, w.dVFo_own, (__nv_bfloat16*)nullptr, w.own_partials, gr->g_own_rows);
-    // own x own score gradients: initial values of the dQ / dK rows (the GEMMs of waves 5 and 7 accumulate on top)
-    TEAM_LAUNCH(own_own_bwd_kernel, (d.B + 7) / 8, 256, 0, ost, d, w.QKVo.f, bf ? w.QKVo.h : nullptr, w.dsown, w.dQKVo.f, (__nv_bfloat16*)nullptr);
-    // ---- table-query rows (prototype / state outputs)
-    int tgrid;
-    if (use_table_gram(d)) {      // Gram formulation (head_table_gram.cuh); needs W0 / GT / xs / xst / RS of the matching forward
-        const int nw = 8, groups = (d.B + nw - 1) / nw;
-        tgrid = groups < NUM_SMS ? groups : NUM_SMS;
-        // LayerNorm gamma / beta gradients of the table rows: own kernel on the side lane (fields dgam / dbet of the records)
-        TEAM_LAUNCH(table_dgamma_kernel, tgrid, 256, 0, own_side != nullptr ? own_side->st : cx.st, d, g_proto, g_state, w.xs, w.xst, w.tab_partials);
-        const size_t tsm = tg_bwd_smem_floats(d, nw) * sizeof(float);
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_gram_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
-        TEAM_LAUNCH(table_gram_bwd_kernel, tgrid, nw * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.VFs.f + (size_t)d.Nsp * D, w.GT, w.VFo.f, w.VFs.f, hw->ln_g, state_ids, g_proto, g_state, w.RS, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials);
-    } else if (use_table2(d)) {   // warp per sample, table rows resident in shared memory (head_table_kernels.cuh)
-        const int groups = (d.B + TW - 1) / TW;
-        tgrid = groups < NUM_SMS ? groups : NUM_SMS;
-        const size_t tsm = table2_bwd_smem_floats(d) * sizeof(float);
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_bwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
-        TEAM_LAUNCH(table_rows_bwd2_kernel, tgrid, TW * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, state_ids, g_proto, g_state, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials, w.VFs.f + (size_t)d.Nsp * D);
-    } else {
-        tgrid = d.B < d.nctas ? d.B : d.nctas;
-        const size_t tsm = table_bwd_smem_floats(d) * sizeof(float);
-        TEAM_REQUIRE(tsm <= 200 * 1024, "head bwd: too many classes for the table-row kernel (%d)", d.C);
-        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
-        TEAM_LAUNCH(table_rows_bwd_kernel, tgrid, TQ_WARPS * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, state_ids, g_proto, g_state, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials);
-    }
-    if ((rc = join_side(cx.st, own_side))) return rc;
-    // the fixed-order fold of the per-CTA partials and dVFo += dVFo_own are not needed before expand_table / wave 7:
-    // side lane, beside GEMM wave 5
-    SideStream* red_side = nullptr;
-    {
-        const cudaStream_t rst = fork_side(cx.st, &red_side);
-        ReduceJobs rj;
-        rj.j[0] = ReduceJob{w.tab_partials, w.tab_reduced, to.len / 4, tgrid};
-        rj.j[1] = ReduceJob{w.own_partials, w.own_reduced, OWN_PARTIAL_LEN / 4, ogrid};
-        rj.blocks0 = (int)((to.len / 4 + RP_COLS - 1) / RP_COLS);
-        TEAM_LAUNCH(reduce_partials_kernel, rj.blocks0 + (OWN_PARTIAL_LEN / 4 + RP_COLS - 1) / RP_COLS, RP_COLS * RP_GROUPS, 0, rst, rj);
-        const int64_t n4 = (int64_t)d.B2 * D / 4;
-        TEAM_LAUNCH(add_rows_kernel, (unsigned)((n4 + 255) / 256), 256, 0, rst, n4, w.dVFo.f, w.dVFo_own, w.dVFo.h);
-    }
+    int rc;
     const Mat Qs = sub(w.QKVs, 0, 0), Ks = sub(w.QKVs, 0, D), Vs = sub(w.QKVs, 0, 2 * D);
     const Mat Qo = sub(w.QKVo, 0, 0), Ko = sub(w.QKVo, 0, D), Vo = sub(w.QKVo, 0, 2 * D);
-    const Mat dQo = sub(w.dQKVo, 0, 0), dKo = sub(w.dQKVo, 0, D), dVo = sub(w.dQKVo, 0, 2 * D);
+    const Mat dQo = sub(w.dQKVo, 0, 0), dVo = sub(w.dQKVo, 0, 2 * D);
     const Mat dQs = sub(w.dQKVs, 0, 0), dKs = sub(w.dQKVs, 0, D), dVs = sub(w.dQKVs, 0, 2 * D);
     Wave wv;
-    // ---- wave 5: R/G coefficient GEMM (A1^T GG + A23^T VFo), dA = dYo VFs^T (into SQ), dKo = dSK Qs
-    seg(seg(wv.add(w.ldA, D, 0.f, fonly(w.RG, D)), true, w.A1, true, w.GG, d.B2), true, w.A23, true, w.VFo, d.B2);
-    seg(wv.add(d.B2, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, w.dYo, false, w.VFs, D);
-    seg(wv.add(d.B2, D, 1.f, dKo), false, w.dSK, true, Qs, d.Nsp);                       // += the own x own part (own_own_bwd_kernel)
-    seg(wv.add(d.Nsp, D, 0.f, fonly(w.dVFs_a, D)), true, w.Aext, true, w.dYo, d.B2);
-    RUN(wv);
-    if ((rc = join_side(cx.st, red_side))) return rc;
-    TEAM_LAUNCH(expand_table_kernel, d.Nsp + EXP_SUM_BLOCKS, 128, 0, cx.st, d, w.tab_reduced, w.own_reduced, w.RG, w.ldA / 2, w.NFt, w.S.f, w.VFs.f, hw->b_fc, w.Rfull, w.Gfull.f, w.Gfull.h, w.hfull, w.dTT.f, w.dVFs.f, w.dVFs_a, gr->ln_g, gr->ln_b, w.dbfc_parts);
-    // ---- wave 6: G VFs^T, dVFs += Pt^T G
-    seg(wv.add(d.Nsp, d.Nsp, 0.f, fonly(w.tmpNN, d.Nsp)), false, w.Gfull, false, w.VFs, D);
-    seg(wv.add(d.Nsp, D, 1.f, w.dVFs), true, w.Pt, true, w.Gfull, d.Nsp);
-    RUN(wv);
-    {   // dS = Aext .* (dA - rowdot) / tau (in place);  dTT += Pt .* (G VFs^T - h) / tau
-        const int64_t n4 = (int64_t)d.B2 * d.Nsp / 4;
-        SideStream* sd = nullptr;
-        const cudaStream_t dst = fork_side(cx.st, &sd);
-        TEAM_LAUNCH(dtt_kernel, (d.Nsp * d.Nsp + 255) / 256, 256, 0, dst, d.Nsp, d.M, w.Pt.f, w.tmpNN, w.hfull, w.dTT.f, w.dTT.h);
-        TEAM_LAUNCH(ds_kernel, (unsigned)((n4 + 255) / 256), 256, 0, cx.st, n4, d.Nsp / 4, w.Aext.f, w.rowdot, w.SQ.f, w.SQ.h, bf ? 0 : 1);
-        if ((rc = join_side(cx.st, sd))) return rc;
-    }
     const Mat& dS = w.SQ;
     // ---- wave 7: score gradients -> dQ/dK, fc folded into V, dWfc
     seg(wv.add(d.B2, D, 1.f, dQo), false, dS, true, Ks, d.Nsp);                                                                     // dQo = dS Ks + the own x own part
@@ -696,6 +572,301 @@ extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t 
         if (overlap_late && (rc = join_side(cx.st, comm_side))) return rc;
     }
     return TEAM_OK;
+}
+
+// Backward of the dropout route up to GEMM wave 7: own rows (side lane) beside the table-query rows, then one wave with
+// dA = dYo VFs^T, dKo += dSK Qs, dVFs = Ad^T dYo + Wd^T dYt and dWd = dYt VFs^T, the own-query softmax backward and the
+// fixed-order batch folds of the table rows (dTT, Rfull, LayerNorm and fc-bias gradients).
+static int drop_bwd(HeadCtx& cx, const team_head_weights* hw, const DropCfg& dc, const int64_t* state_ids, const float* g_image,
+                    const float* g_text, const float* g_state, const float* g_proto, const team_head_grads* gr) {
+    const HeadDims& d = cx.d;
+    HeadWS& w = cx.w;
+    const DropWS& dw = dc.w;
+    const bool bf = cx.mode == TEAM_MODE_BF16;
+    int rc;
+    int ogrid = (d.B + 7) / 8;
+    if (ogrid > NUM_SMS) ogrid = NUM_SMS;
+    SideStream* own_side = nullptr;
+    const cudaStream_t ost = fork_side(cx.st, &own_side);
+    TEAM_LAUNCH(drop_ln_own_bwd_kernel, ogrid, 256, 0, ost, d, dc.a, (const float*)w.Ybo, (const float*)w.Xo.f, (const float*)w.VFo.f, (const float*)w.aown, (const float*)dw.aownd, hw->b_fc, hw->ln_g, hw->ln_b, g_image, g_text, w.dYo.f, w.dYo.h, w.dXo.f, w.rowdot, w.dsown, w.dVFo_own, w.own_partials, gr->g_own_rows);
+    TEAM_LAUNCH(own_own_bwd_kernel, (d.B + 7) / 8, 256, 0, ost, d, w.QKVo.f, bf ? w.QKVo.h : nullptr, w.dsown, w.dQKVo.f, (__nv_bfloat16*)nullptr);
+    TEAM_LAUNCH(drop_table_bwd_kernel, ogrid, 256, 0, cx.st, d, dc.a, (const float*)dw.Yt, dw.tsc, (const float*)w.VFo.f, (const float*)w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, g_proto, g_state, dw.dYt.f, dw.dYt.h, dw.dU, w.dSK.f, w.dSK.h, w.dVFo.f, dw.tpart);
+    if ((rc = join_side(cx.st, own_side))) return rc;
+    {
+        const int64_t n4 = (int64_t)d.B2 * D / 4;
+        TEAM_LAUNCH(add_rows_kernel, (unsigned)((n4 + 255) / 256), 256, 0, cx.st, n4, w.dVFo.f, (const float*)w.dVFo_own, w.dVFo.h);
+    }
+    const int64_t NT = (int64_t)d.B * (d.C + 1);
+    const Mat Qs = sub(w.QKVs, 0, 0), dKo = sub(w.dQKVo, 0, D);
+    Wave wv;
+    seg(wv.add(d.B2, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, w.dYo, false, w.VFs, D);                            // dA = dYo VFs^T
+    seg(wv.add(d.B2, D, 1.f, dKo), false, w.dSK, true, Qs, d.Nsp);                                                 // dKo += dSK Qs
+    seg(seg(wv.add(d.Nsp, D, 0.f, w.dVFs), true, dw.Ad, true, w.dYo, d.B2), true, dw.Wd, true, dw.dYt, NT);       // dVFs
+    seg(wv.add(NT, d.Nsp, 0.f, fonly(dw.dWd, d.Nsp)), false, dw.dYt, false, w.VFs, D);                            // dWd = dYt VFs^T
+    RUN(wv);
+    {
+        const int64_t n4 = (int64_t)d.B2 * d.Nsp / 4;
+        TEAM_LAUNCH(drop_ds_kernel, (unsigned)((n4 + 255) / 256), 256, 0, cx.st, n4, d.Nsp / 4, (const float*)w.Aext.f, (const float*)dw.Ad.f, (const float*)w.rowdot, w.SQ.f, w.SQ.h, bf ? 0 : 1);
+        const int tt_blocks = (d.Nsp * d.Nsp + 255) / 256;
+        TEAM_LAUNCH(drop_fold_kernel, tt_blocks + d.Nsp + 1, 256, 0, cx.st, d, tt_blocks, (const float*)dw.Wd.f, (const float*)dw.dWd, (const float*)w.Pt.f, (const float*)dw.tsc, state_ids, (const float*)dw.dU, (const float*)dw.tpart, ogrid, (const float*)w.own_partials, ogrid, w.dTT.f, w.dTT.h, w.Rfull, gr->ln_g, gr->ln_b, w.dbfc_parts);
+    }
+    return bwd_tail(cx, gr);
+}
+
+}  // namespace team
+
+using namespace team;
+
+extern "C" size_t team_head_workspace_bytes(int64_t batch, int32_t num_classes, int32_t num_prompts,
+                                            int32_t num_text_cls, int mode) {
+    HeadDims d = head_dims(batch, num_classes, num_prompts, num_text_cls);
+    HeadWS w;
+    head_plan(d, mode, nullptr, &w);
+    return w.total_bytes;
+}
+
+// *p += v on the device (one thread): the per-step advance of team_dropout.offset_dev, capturable, no host sync
+static __global__ void u64_add_kernel(uint64_t* p, uint64_t v) {
+    pdl_trigger();
+    pdl_wait();
+    *p += v;
+}
+extern "C" int team_u64_add(uint64_t* p, uint64_t v, void* stream) {
+    TEAM_REQUIRE(p != nullptr, "u64 add: null pointer");
+    TEAM_LAUNCH(u64_add_kernel, 1, 1, 0, (cudaStream_t)stream, p, v);
+    return TEAM_OK;
+}
+
+extern "C" size_t team_head_dropout_workspace_bytes(int64_t batch, int32_t num_classes, int32_t num_prompts, int mode) {
+    DropWS w;
+    drop_plan(head_dims(batch, num_classes, num_prompts, 0), mode, nullptr, &w);
+    return w.total_bytes;
+}
+
+extern "C" int team_head_frozen_sums(const team_head_weights* hw, int32_t num_frozen, float* w_sums, float* b_sums, void* stream) {
+    TEAM_REQUIRE(hw != nullptr && w_sums != nullptr && b_sums != nullptr, "head frozen sums: null pointer");
+    TEAM_REQUIRE(num_frozen >= 1 && num_frozen <= hw->num_tasks && hw->num_tasks <= TEAM_MAX_TASKS, "head frozen sums: num_frozen %d out of [1, %d]", num_frozen, hw->num_tasks);
+    PrepSum ps;
+    memset(&ps, 0, sizeof(ps));
+    const float* const* Ws[3] = {hw->w_img, hw->w_text, hw->w_state};
+    const float* const* Bs[3] = {hw->b_img, hw->b_text, hw->b_state};
+    for (int k = 0; k < 3; ++k) {
+        for (int t = 0; t < num_frozen; ++t) TEAM_REQUIRE(Ws[k][t] != nullptr && Bs[k][t] != nullptr, "head frozen sums: null projection %d of task %d", k, t);
+        ps.W[k] = plist(Ws[k], num_frozen); ps.Bv[k] = plist(Bs[k], num_frozen);
+        ps.Wout[k] = w_sums + (size_t)k * D * D; ps.Wh[k] = nullptr; ps.bout[k] = b_sums + (size_t)k * D;
+    }
+    ps.n = 3;
+    ConvList cl;
+    memset(&cl, 0, sizeof(cl));
+    cl.sum_blocks = 3 * PREP_SUM_BLOCKS_PER_W;
+    TEAM_LAUNCH(prep_kernel, cl.sum_blocks, 256, 0, (cudaStream_t)stream, ps, cl);
+    return TEAM_OK;
+}
+
+// byte offset of the normalised projected own rows Xo ([2B,512] fp32: image rows, then text rows) inside the workspace
+extern "C" size_t team_head_own_rows_offset(int64_t batch, int32_t num_classes, int32_t num_prompts, int32_t num_text_cls, int mode) {
+    HeadDims d = head_dims(batch, num_classes, num_prompts, num_text_cls);
+    HeadWS w;
+    head_plan(d, mode, reinterpret_cast<void*>(uintptr_t(256)), &w);          // a non-null fake base: only the offsets are used
+    return (size_t)(reinterpret_cast<uintptr_t>(w.Xo.f) - 256);
+}
+
+// Forward: 13 launches (prologue, prompt rows, 4 GEMM waves, 7 row kernels; three short side-lane branches) - see
+// DESIGN.md section 4.
+extern "C" int team_head_tri_fwd(const team_head_weights* hw, int mode, int64_t batch, const float* image_feat,
+                                 const float* text_feat, const int64_t* state_ids, const float* text_cls,
+                                 int64_t num_text_cls, float* out_image, float* out_text, float* out_state,
+                                 float* out_proto, float* cls_logits, int64_t* cls_argmax, void* workspace,
+                                 size_t workspace_bytes, void* stream, const team_dropout* dropout) {
+    HeadCtx cx;
+    int rc = setup(cx, "head", hw, mode, batch, 0, (int)(text_cls ? num_text_cls : 0), workspace, workspace_bytes, stream);
+    if (rc) return rc;
+    DropCfg dc;
+    if ((rc = drop_setup(cx.d, mode, dropout, &dc))) return rc;
+    TEAM_REQUIRE(image_feat && text_feat && state_ids && out_image && out_text && out_state && out_proto, "head fwd: null pointer");
+    TEAM_REQUIRE(hw->w_q && hw->w_k && hw->w_v && hw->w_fc && hw->b_fc && hw->ln_g && hw->ln_b && hw->state_emb && hw->prototypes, "head fwd: null weight");
+    const HeadDims& d = cx.d;
+    HeadWS& w = cx.w;
+    const bool want_cls = d.Tc > 0 && (cls_logits != nullptr || cls_argmax != nullptr);
+    bind_inputs(cx, hw, image_feat, text_feat, text_cls);
+    SideStream* side = nullptr;
+    const int fill_rows = d.P + (d.Nsp - d.Ns);
+    if (fill_rows > 0) {          // prompt rows of S: independent of the prologue -> side lane
+        const cudaStream_t fst = fork_side(cx.st, &side);
+        TEAM_LAUNCH(fill_prompt_rows_kernel, fill_rows, 128, 0, fst, plist(hw->prompts, hw->num_tasks), hw->prompts_per_task > 0 ? hw->prompts_per_task : 1, d.C, d.Ns, d.Nsp, w.S.f, w.S.h);
+    }
+    if ((rc = prologue(cx, hw, 3, image_feat, text_feat, want_cls ? text_cls : nullptr, batch))) return rc;
+    SideStream* fill_side = side;        // joined before wave 2 (the first reader of the prompt rows): wave 1 chains straight behind the prologue
+    Wave wv;
+    // ---- wave 1: every projection of the step (prototype rows, state table, image rows, text rows, class text)
+    seg(wv.add(d.C, D, 0.f, fonly(w.Ztab, D), w.bsum[0]), false, w.protos, false, w.Wsum[0], D);
+    seg(wv.add(10, D, 0.f, fonly(w.Ztab + (size_t)d.C * D, D), w.bsum[2]), false, w.E, false, w.Wsum[2], D);
+    seg(wv.add(d.B, D, 0.f, fonly(w.Xo.f, D), w.bsum[0]), false, w.img, false, w.Wsum[0], D);
+    seg(wv.add(d.B, D, 0.f, fonly(w.Xo.f + (size_t)d.B * D, D), w.bsum[1]), false, w.txt, false, w.Wsum[1], D);
+    if (want_cls) seg(wv.add(d.Tc, D, 0.f, fonly(w.Zc, D), w.bsum[1]), false, w.tcls, false, w.Wsum[1], D);
+    RUN(wv);
+    {   // L2-normalise: prototype rows -> S[0,C), state table -> S[M,M+10), own rows in place
+        NormList nl;
+        memset(&nl, 0, sizeof(nl));
+        nl.do_normalize = 1;
+        int blocks = 0;
+        norm_add(nl, blocks, w.Ztab, w.S.f, w.S.h, w.invS, d.C);
+        norm_add(nl, blocks, w.Ztab + (size_t)d.C * D, w.S.f + (size_t)d.M * D, w.S.h ? w.S.h + (size_t)d.M * D : nullptr, w.invS + d.M, 10);
+        norm_add(nl, blocks, w.Xo.f, w.Xo.f, w.Xo.h, w.invo, d.B2);
+        TEAM_LAUNCH(rows_normalize_kernel, blocks, 256, 0, cx.st, nl);
+    }
+    if ((rc = join_side(cx.st, fill_side))) return rc;
+    // waves 2 and 3; VFo keeps its bf16 shadow (GEMM operand of the backward and of the Gram table rows)
+    if ((rc = qkv_score_waves(cx, d.B2, w.VFo))) return rc;
+    if (dc.on) return drop_fwd(cx, hw, dc, state_ids, want_cls, cls_logits, cls_argmax, out_image, out_text, out_state, out_proto);
+    SideStream* gram_side = nullptr;
+    {   // the two softmax kernels (step-row table, own rows) are independent
+        const cudaStream_t tst = fork_side(cx.st, &side);
+        const bool gram = use_table_gram(d);
+        const int xwarps = TG_RP;                            // + the s rows S_r + b_fc (bulk-copy source of the table-row kernels; Gram operand)
+        TEAM_LAUNCH(table_prep_kernel, (d.Nsp + xwarps + 7) / 8, 256, 0, tst, w.TT, d.M, d.Nsp, w.mt, w.Zt, w.Pt.f, w.Pt.h, w.S.f, hw->b_fc,
+                    w.VFs.f, (const __nv_bfloat16*)w.VFs.h, d.C, TG_RP,
+                    w.VFs.f + (size_t)d.Nsp * D, w.VFs.h ? w.VFs.h + (size_t)d.Nsp * D : (__nv_bfloat16*)nullptr);
+        if (gram)             // ... and its n rows
+            TEAM_LAUNCH(table_nf_kernel, d.Rt, 256, ((d.M + 3) / 4 * 4 + 512) * sizeof(float), tst, w.TT, d.M, d.Nsp, d.C, w.VFs.f, (const __nv_bfloat16*)w.VFs.h,
+                        w.VFs.f + (size_t)(d.Nsp + TG_RP) * D, w.VFs.h ? w.VFs.h + (size_t)(d.Nsp + TG_RP) * D : (__nv_bfloat16*)nullptr);
+        TEAM_LAUNCH(attn_own_kernel, (d.B2 + 7) / 8, 256, 0, cx.st, d, w.SQ.f, w.QKVo.f, cx.mode == TEAM_MODE_BF16 ? w.QKVo.h : nullptr, state_ids, w.Aext.f, w.Aext.h, w.aown);
+        if ((rc = join_side(cx.st, side))) return rc;
+        // step-level dot products of the table rows: beside GEMM wave 4 (joined before the table-row kernel)
+        if (gram) TEAM_LAUNCH(table_gram_prep_kernel, (d.Rt + 10 + 7) / 8, 256, 0, side != nullptr ? side->st : cx.st, d.Rt, w.VFs.f + (size_t)d.Nsp * D, w.VFs.f + (size_t)d.M * D, w.GT);
+        gram_side = gram ? side : nullptr;
+    }
+    // ---- wave 4: probabilities x (fc-space) values
+    seg(wv.add(d.Nsp, D, 0.f, fonly(w.NFt, D)), false, w.Pt, true, w.VFs, d.Nsp);
+    seg(wv.add(d.B2, D, 0.f, fonly(w.Ybo, D)), false, w.Aext, true, w.VFs, d.Nsp);
+    // sample x table dot products of the table-query rows (head_table_gram.cuh): W0 = VFo x [VFs ; S_table + b_fc]^T
+    if (use_table_gram(d)) seg(wv.add(d.B2, tg_ldw(d), 0.f, fonly(w.W0, tg_ldw(d))), false, w.VFo, false, w.VFs, D);
+    RUN(wv);
+    // the own-row outputs and the classification logits do not depend on the table-query rows: side stream
+    const cudaStream_t sst = fork_side(cx.st, &side);
+    TEAM_LAUNCH(ln_own_fwd_kernel, (d.B2 + 7) / 8, 256, 0, sst, d, w.Ybo, w.aown, w.VFo.f, w.Xo.f, hw->b_fc, hw->ln_g, hw->ln_b, out_image, out_text);
+    // forward_for_classification (models/proof.py:519-536; image rows are already normalised in Xo): a third lane beside the
+    // own-row LayerNorm and the table rows.  Measured alternatives (tools/timeline.py, profiles/r2z_timeline_*): behind
+    // ln_own_fwd on the same lane the pair outlasts the table rows by 5 us; forked right after the normalisation (its inputs
+    // are ready there, 45 us of slack) it slows GEMM waves 2 and 3 by more than it saves (0.194 vs 0.189 ms per step), at the
+    // lowest stream priority as well - the kernels of one step compete for the same SMs and L2 bandwidth.
+    SideStream* cls_side = nullptr;
+    if (want_cls) {
+        const cudaStream_t cst = fork_side(cx.st, &cls_side, 2);
+        if ((rc = cosine_logits_launch(cst, w.Xo.f, d.B, w.Zc, d.Tc, nullptr, cls_logits, cls_argmax))) return rc;
+    }
+    if (use_table_gram(d)) {      // Gram formulation: scalar LayerNorm algebra per (sample, row), vector outputs as coefficient sums
+        if ((rc = join_side(cx.st, gram_side))) return rc;          // table_gram_prep_kernel
+        const int nw = tg_warps(d), groups = (d.B + nw - 1) / nw;
+        const size_t tsm = tg_fwd_smem_floats(d) * sizeof(float);
+        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_gram_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
+        TEAM_LAUNCH(table_gram_fwd_kernel, groups < NUM_SMS ? groups : NUM_SMS, nw * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.VFs.f + (size_t)d.Nsp * D, w.GT, w.W0, w.VFo.f, w.VFs.f, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state, w.xs, w.xst, w.RS);
+    } else if (use_table2(d)) {   // warp per sample, table rows resident in shared memory (head_table_kernels.cuh)
+        const int groups = (d.B + TW - 1) / TW;
+        const size_t tsm = table2_fwd_smem_floats(d) * sizeof(float);
+        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
+        TEAM_LAUNCH(table_rows_fwd2_kernel, groups < NUM_SMS ? groups : NUM_SMS, TW * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state, w.VFs.f + (size_t)d.Nsp * D);
+    } else {
+        const int tgrid = d.B < 6 * NUM_SMS ? d.B : 6 * NUM_SMS;
+        TEAM_LAUNCH(table_rows_fwd_kernel, tgrid, TQ_WARPS * 32, 0, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, hw->ln_b, state_ids, out_proto, out_state);
+    }
+    if ((rc = join_side(cx.st, side))) return rc;
+    if ((rc = join_side(cx.st, cls_side))) return rc;
+    return TEAM_OK;
+}
+
+// Backward: 13 launches at the headline size (5 GEMM waves, 8 row kernels; more when split-K runs through the fix-up
+// kernel or the gradient exchange is folded in); needs the workspace of the matching forward call.
+extern "C" int team_head_tri_bwd(const team_head_weights* hw, int mode, int64_t batch, const float* image_feat,
+                                 const float* text_feat, const int64_t* state_ids, const float* g_image,
+                                 const float* g_text, const float* g_state, const float* g_proto,
+                                 const team_head_grads* gr, void* workspace, size_t workspace_bytes, void* stream,
+                                 const team_dropout* dropout) {
+    HeadCtx cx;
+    int rc = setup(cx, "head", hw, mode, batch, 0, 0, workspace, workspace_bytes, stream);
+    if (rc) return rc;
+    DropCfg dc;
+    if ((rc = drop_setup(cx.d, mode, dropout, &dc))) return rc;
+    TEAM_REQUIRE(gr && g_image && g_text && g_state && image_feat && text_feat && state_ids, "head bwd: null pointer");
+    TEAM_REQUIRE(gr->w_img && gr->b_img && gr->w_text && gr->b_text && gr->w_state && gr->b_state && gr->state_emb &&
+                 gr->w_q && gr->w_k && gr->w_v && gr->w_fc && gr->b_fc && gr->ln_g && gr->ln_b, "head bwd: null gradient buffer");
+    const HeadDims& d = cx.d;
+    HeadWS& w = cx.w;
+    bind_inputs(cx, hw, image_feat, text_feat, nullptr);
+    if (dc.on) return drop_bwd(cx, hw, dc, state_ids, g_image, g_text, g_state, g_proto, gr);
+    const TabOff to = tab_offsets(d);
+    const bool bf = cx.mode == TEAM_MODE_BF16;
+    // ---- own query rows: independent of the table-query rows -> side lane, beside them (its dVF part goes to dVFo_own)
+    int ogrid = (d.B + 7) / 8;
+    if (ogrid > NUM_SMS) ogrid = NUM_SMS;
+    SideStream* own_side = nullptr;
+    // (Enqueueing the table-row kernel first - it needs a whole register file per CTA and cannot share an SM with these two -
+    // was measured: it then runs alone in 26 us, but the own-row kernels are squeezed onto the 20 remaining SMs and finish
+    // later than before: 0.1948 vs 0.1885 ms per step, tools/timeline.py.)
+    const cudaStream_t ost = fork_side(cx.st, &own_side);
+    TEAM_LAUNCH(ln_own_bwd_kernel, ogrid, 256, 0, ost, d, w.Ybo, w.Xo.f, w.VFo.f, w.aown, hw->b_fc, hw->ln_g, hw->ln_b, g_image, g_text, w.dYo.f, w.dYo.h, w.dXo.f, w.rowdot, w.dsown, w.dVFo_own, (__nv_bfloat16*)nullptr, w.own_partials, gr->g_own_rows);
+    // own x own score gradients: initial values of the dQ / dK rows (the GEMMs of waves 5 and 7 accumulate on top)
+    TEAM_LAUNCH(own_own_bwd_kernel, (d.B + 7) / 8, 256, 0, ost, d, w.QKVo.f, bf ? w.QKVo.h : nullptr, w.dsown, w.dQKVo.f, (__nv_bfloat16*)nullptr);
+    // ---- table-query rows (prototype / state outputs)
+    int tgrid;
+    if (use_table_gram(d)) {      // Gram formulation (head_table_gram.cuh); needs W0 / GT / xs / xst / RS of the matching forward
+        const int nw = 8, groups = (d.B + nw - 1) / nw;
+        tgrid = groups < NUM_SMS ? groups : NUM_SMS;
+        // LayerNorm gamma / beta gradients of the table rows: own kernel on the side lane (fields dgam / dbet of the records)
+        TEAM_LAUNCH(table_dgamma_kernel, tgrid, 256, 0, own_side != nullptr ? own_side->st : cx.st, d, g_proto, g_state, w.xs, w.xst, w.tab_partials);
+        const size_t tsm = tg_bwd_smem_floats(d, nw) * sizeof(float);
+        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_gram_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
+        TEAM_LAUNCH(table_gram_bwd_kernel, tgrid, nw * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.VFs.f + (size_t)d.Nsp * D, w.GT, w.VFo.f, w.VFs.f, hw->ln_g, state_ids, g_proto, g_state, w.RS, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials);
+    } else if (use_table2(d)) {   // warp per sample, table rows resident in shared memory (head_table_kernels.cuh)
+        const int groups = (d.B + TW - 1) / TW;
+        tgrid = groups < NUM_SMS ? groups : NUM_SMS;
+        const size_t tsm = table2_bwd_smem_floats(d) * sizeof(float);
+        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_bwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
+        TEAM_LAUNCH(table_rows_bwd2_kernel, tgrid, TW * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, state_ids, g_proto, g_state, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials, w.VFs.f + (size_t)d.Nsp * D);
+    } else {
+        tgrid = d.B < d.nctas ? d.B : d.nctas;
+        const size_t tsm = table_bwd_smem_floats(d) * sizeof(float);
+        TEAM_REQUIRE(tsm <= 200 * 1024, "head bwd: too many classes for the table-row kernel (%d)", d.C);
+        TEAM_CUDA_CHECK(cudaFuncSetAttribute(table_rows_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm));
+        TEAM_LAUNCH(table_rows_bwd_kernel, tgrid, TQ_WARPS * 32, tsm, cx.st, d, w.SK, w.TT, w.mt, w.Zt, w.NFt, w.VFo.f, w.VFs.f, w.S.f, hw->b_fc, hw->ln_g, state_ids, g_proto, g_state, w.dSK.f, w.dSK.h, w.dVFo.f, w.GG.f, w.GG.h, w.A1.f, w.A1.h, w.A23.f, w.A23.h, w.ldA, w.tab_partials);
+    }
+    if ((rc = join_side(cx.st, own_side))) return rc;
+    // the fixed-order fold of the per-CTA partials and dVFo += dVFo_own are not needed before expand_table / wave 7:
+    // side lane, beside GEMM wave 5
+    SideStream* red_side = nullptr;
+    {
+        const cudaStream_t rst = fork_side(cx.st, &red_side);
+        ReduceJobs rj;
+        rj.j[0] = ReduceJob{w.tab_partials, w.tab_reduced, to.len / 4, tgrid};
+        rj.j[1] = ReduceJob{w.own_partials, w.own_reduced, OWN_PARTIAL_LEN / 4, ogrid};
+        rj.blocks0 = (int)((to.len / 4 + RP_COLS - 1) / RP_COLS);
+        TEAM_LAUNCH(reduce_partials_kernel, rj.blocks0 + (OWN_PARTIAL_LEN / 4 + RP_COLS - 1) / RP_COLS, RP_COLS * RP_GROUPS, 0, rst, rj);
+        const int64_t n4 = (int64_t)d.B2 * D / 4;
+        TEAM_LAUNCH(add_rows_kernel, (unsigned)((n4 + 255) / 256), 256, 0, rst, n4, w.dVFo.f, w.dVFo_own, w.dVFo.h);
+    }
+    const Mat Qs = sub(w.QKVs, 0, 0), dKo = sub(w.dQKVo, 0, D);
+    Wave wv;
+    // ---- wave 5: R/G coefficient GEMM (A1^T GG + A23^T VFo), dA = dYo VFs^T (into SQ), dKo = dSK Qs
+    seg(seg(wv.add(w.ldA, D, 0.f, fonly(w.RG, D)), true, w.A1, true, w.GG, d.B2), true, w.A23, true, w.VFo, d.B2);
+    seg(wv.add(d.B2, d.Nsp, 0.f, fonly(w.SQ.f, d.Nsp)), false, w.dYo, false, w.VFs, D);
+    seg(wv.add(d.B2, D, 1.f, dKo), false, w.dSK, true, Qs, d.Nsp);                       // += the own x own part (own_own_bwd_kernel)
+    seg(wv.add(d.Nsp, D, 0.f, fonly(w.dVFs_a, D)), true, w.Aext, true, w.dYo, d.B2);
+    RUN(wv);
+    if ((rc = join_side(cx.st, red_side))) return rc;
+    TEAM_LAUNCH(expand_table_kernel, d.Nsp + EXP_SUM_BLOCKS, 128, 0, cx.st, d, w.tab_reduced, w.own_reduced, w.RG, w.ldA / 2, w.NFt, w.S.f, w.VFs.f, hw->b_fc, w.Rfull, w.Gfull.f, w.Gfull.h, w.hfull, w.dTT.f, w.dVFs.f, w.dVFs_a, gr->ln_g, gr->ln_b, w.dbfc_parts);
+    // ---- wave 6: G VFs^T, dVFs += Pt^T G
+    seg(wv.add(d.Nsp, d.Nsp, 0.f, fonly(w.tmpNN, d.Nsp)), false, w.Gfull, false, w.VFs, D);
+    seg(wv.add(d.Nsp, D, 1.f, w.dVFs), true, w.Pt, true, w.Gfull, d.Nsp);
+    RUN(wv);
+    {   // dS = Aext .* (dA - rowdot) / tau (in place);  dTT += Pt .* (G VFs^T - h) / tau
+        const int64_t n4 = (int64_t)d.B2 * d.Nsp / 4;
+        SideStream* sd = nullptr;
+        const cudaStream_t dst = fork_side(cx.st, &sd);
+        TEAM_LAUNCH(dtt_kernel, (d.Nsp * d.Nsp + 255) / 256, 256, 0, dst, d.Nsp, d.M, w.Pt.f, w.tmpNN, w.hfull, w.dTT.f, w.dTT.h);
+        TEAM_LAUNCH(ds_kernel, (unsigned)((n4 + 255) / 256), 256, 0, cx.st, n4, d.Nsp / 4, w.Aext.f, w.rowdot, w.SQ.f, w.SQ.h, bf ? 0 : 1);
+        if ((rc = join_side(cx.st, sd))) return rc;
+    }
+    return bwd_tail(cx, gr);
 }
 
 // PROOF fusion forward (Proof_Net.forward, utils/inc_net.py:436-463; forward_transformer with transformer=True,

@@ -85,7 +85,7 @@ def _fill_weights(T: int, ppt: int, flat: Sequence[torch.Tensor], protos: torch.
 
 class _TriModalFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, image, text, state_ids, protos, text_cls, mode, T, ppt, *params):
+    def forward(ctx, image, text, state_ids, protos, text_cls, mode, T, ppt, dropout, *params):
         capi.require_device()
         dev = image.device
         if not image.is_cuda:
@@ -103,6 +103,7 @@ class _TriModalFn(torch.autograd.Function):
         L = capi.lib()
         nbytes = L.team_head_workspace_bytes(B, hw.num_classes, T * ppt, n_cls, mode)
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+        dr, dws = _dropout_arg(dropout, B, hw.num_classes, T * ppt, mode, dev)
         outs = torch.empty((4, B, capi.D), dtype=torch.float32, device=dev)
         logits = torch.empty((B, n_cls), dtype=torch.float32, device=dev) if n_cls else None
         amax = torch.empty((B,), dtype=torch.int64, device=dev) if n_cls else None
@@ -111,8 +112,8 @@ class _TriModalFn(torch.autograd.Function):
             text_cls.data_ptr() if n_cls else None, n_cls,
             outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr(), outs[3].data_ptr(),
             logits.data_ptr() if n_cls else None, amax.data_ptr() if n_cls else None,
-            ws.data_ptr(), nbytes, _stream_ptr()), "team_head_tri_fwd")
-        ctx.hold = (image, text, sid, protos, flat, ws)
+            ws.data_ptr(), nbytes, _stream_ptr(), dr), "team_head_tri_fwd")
+        ctx.hold = (image, text, sid, protos, flat, ws, dr, dws)
         ctx.meta = (mode, T, ppt, B, nbytes)
         ctx.set_materialize_grads(False)        # an unused output arrives as None: a None g_proto skips the prototype rows
         res = (outs[0], outs[1].view(B, 1, capi.D), outs[2], outs[3])
@@ -123,7 +124,7 @@ class _TriModalFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g_img, g_txt, g_st, g_pr, *unused):
-        image, text, sid, protos, flat, ws = ctx.hold
+        image, text, sid, protos, flat, ws, dr, dws = ctx.hold
         mode, T, ppt, B, nbytes = ctx.meta
         dev = image.device
         hw = _fill_weights(T, ppt, flat, protos)
@@ -150,8 +151,8 @@ class _TriModalFn(torch.autograd.Function):
         capi.check(capi.lib().team_head_tri_bwd(
             C.byref(hw), mode, B, image.data_ptr(), text.data_ptr(), sid.data_ptr(),
             cots[0].data_ptr(), cots[1].data_ptr(), cots[2].data_ptr(), cots[3].data_ptr() if cots[3] is not None else None,
-            C.byref(hg), ws.data_ptr(), nbytes, _stream_ptr()), "team_head_tri_bwd")
-        need = ctx.needs_input_grad[8:]
+            C.byref(hg), ws.data_ptr(), nbytes, _stream_ptr(), dr), "team_head_tri_bwd")
+        need = ctx.needs_input_grad[9:]
         out: List[Optional[torch.Tensor]] = []
         names = ("w_img", "b_img", "w_text", "b_text", "w_state", "b_state")
         for k, n in enumerate(names):           # W = sum_t W_t  =>  dW_t = dW for every unfrozen t
@@ -161,15 +162,30 @@ class _TriModalFn(torch.autograd.Function):
             out.append(g["prompts"][t * ppt:(t + 1) * ppt] if need[6 * T + t] else None)
         for i, n in enumerate(("state_emb", "w_q", "w_k", "w_v", "w_fc", "b_fc", "ln_g", "ln_b")):
             out.append(g[n] if need[7 * T + i] else None)
-        return (None,) * 8 + tuple(out)
+        return (None,) * 9 + tuple(out)
+
+
+def _dropout_arg(dropout, B: int, C_: int, P: int, mode: int, dev):
+    """(team_dropout or None, its workspace) for ``dropout`` = None or (p, seed, offset)."""
+    if dropout is None or float(dropout[0]) == 0.0:
+        return None, None
+    p, seed, offset = float(dropout[0]), int(dropout[1]), int(dropout[2])
+    if not 0.0 < p < 1.0:
+        raise ValueError(f"dropout p = {p} out of [0, 1)")
+    n = capi.lib().team_head_dropout_workspace_bytes(B, C_, P, mode)
+    dws = torch.empty((n,), dtype=torch.uint8, device=dev)
+    dr = capi.Dropout(p, seed & 0xFFFFFFFFFFFFFFFF, offset & 0xFFFFFFFFFFFFFFFF, None, dws.data_ptr(), n)
+    return C.pointer(dr), dws
 
 
 def forward_tri_modal(pack: HeadParamPack, image: torch.Tensor, text: torch.Tensor,
                       state_ids: torch.Tensor, img_prototypes: torch.Tensor, *,
-                      text_cls: Optional[torch.Tensor] = None, mode: int = MODE_F32):
+                      text_cls: Optional[torch.Tensor] = None, mode: int = MODE_F32, dropout=None):
     """(image[B,512], text[B,1,512], state[B,512], proto[B,512]) [+ (cls_logits[B,Tc], argmax[B])].
-    ``image``/``text`` are post-CLIP 512-d features (per-sample text)."""
-    return _TriModalFn.apply(image, text, state_ids, img_prototypes, text_cls, mode, pack.T, pack.ppt,
+    ``image``/``text`` are post-CLIP 512-d features (per-sample text).  ``dropout`` = (p, seed, offset): sel_attn in train
+    mode, with the masks ``mha(..., dropout_p=p, seed=seed, offset=offset)`` draws on the token tensor
+    [image | text | state | C prototypes | P prompts]; the backward reuses the same masks.  None or p = 0: eval mode."""
+    return _TriModalFn.apply(image, text, state_ids, img_prototypes, text_cls, mode, pack.T, pack.ppt, dropout,
                              *pack.flat)
 
 
@@ -483,9 +499,14 @@ class HeadStepRunner:
 
     def __init__(self, pack: HeadParamPack, img_prototypes: torch.Tensor, batch: int, num_text_cls: int,
                  mode: int = MODE_F32, grad_events: bool = False, grad_buffer: Optional[torch.Tensor] = None,
-                 peer=None):
+                 peer=None, dropout_p: float = 0.0, seed: Optional[int] = None):
         """``peer``: a ``parallel.PeerAllReduce`` whose ``buffer`` becomes the gradient buffer; the backward then
-        sums the gradients over the ranks itself (early bucket under its last kernels, late bucket at its end)."""
+        sums the gradients over the ranks itself (early bucket under its last kernels, late bucket at its end).
+        ``dropout_p`` > 0: sel_attn in train mode (the masks of ``forward_tri_modal(dropout=(p, seed, offset))``).  The
+        runner owns the dropout workspace and a device-resident offset (``offset_dev``, initially 2 randint(0, 2^62) from
+        torch's CPU generator, as MultiHeadAttention.forward draws it; ``seed`` defaults to ``torch.initial_seed()``);
+        ``advance_offset`` moves it to the next step's masks on the device, so a captured step draws fresh masks on
+        every replay."""
         capi.require_device()
         dev = pack.flat[0].device
         self.dev, self.B, self.mode, self.n_cls = dev, batch, mode, num_text_cls
@@ -501,6 +522,17 @@ class HeadStepRunner:
         self.nbytes = L.team_head_workspace_bytes(batch, self.hw.num_classes, pack.T * pack.ppt, num_text_cls, mode)
         self.ws = torch.empty((self.nbytes,), dtype=torch.uint8, device=dev)
         self.outs = torch.empty((4, batch, capi.D), dtype=torch.float32, device=dev)
+        self.dropout_p = float(dropout_p)
+        self._drop = None
+        if self.dropout_p != 0.0:
+            if not 0.0 < self.dropout_p < 1.0:
+                raise ValueError(f"dropout_p = {dropout_p} out of [0, 1)")
+            self.seed = int(torch.initial_seed() if seed is None else seed) & 0xFFFFFFFFFFFFFFFF
+            base = int(torch.randint(0, 2 ** 62, (1,)).item()) * 2
+            self.offset_dev = torch.tensor([base], dtype=torch.int64, device=dev)      # read as uint64 by the kernels
+            n = L.team_head_dropout_workspace_bytes(batch, self.hw.num_classes, pack.T * pack.ppt, mode)
+            self.drop_ws = torch.empty((n,), dtype=torch.uint8, device=dev)
+            self._drop = C.pointer(capi.Dropout(self.dropout_p, self.seed, base, self.offset_dev.data_ptr(), self.drop_ws.data_ptr(), n))
         self.logits = torch.empty((batch, max(num_text_cls, 1)), dtype=torch.float32, device=dev)
         self.argmax = torch.empty((batch,), dtype=torch.int64, device=dev)
         P = pack.T * pack.ppt
@@ -601,7 +633,7 @@ class HeadStepRunner:
             text_cls.data_ptr() if n_cls else None, n_cls,
             self.outs[0].data_ptr(), self.outs[1].data_ptr(), self.outs[2].data_ptr(), self.outs[3].data_ptr(),
             self.logits.data_ptr() if n_cls else None, self.argmax.data_ptr() if n_cls else None,
-            self.ws.data_ptr(), self.nbytes, _stream_ptr()), "team_head_tri_fwd")
+            self.ws.data_ptr(), self.nbytes, _stream_ptr(), self._drop), "team_head_tri_fwd")
 
     def own_rows(self) -> torch.Tensor:
         """[2B,512] view of normalize(encode_image(x)) | normalize(encode_text(t)) as the last ``forward`` left them in the
@@ -619,7 +651,18 @@ class HeadStepRunner:
         capi.check(capi.lib().team_head_tri_bwd(
             C.byref(self.hw), self.mode, self.B, image.data_ptr(), text.data_ptr(), sid.data_ptr(),
             cots[0].data_ptr(), cots[1].data_ptr(), cots[2].data_ptr(), cots[3].data_ptr() if cots[3] is not None else None,
-            C.byref(self.hg), self.ws.data_ptr(), self.nbytes, _stream_ptr()), "team_head_tri_bwd")
+            C.byref(self.hg), self.ws.data_ptr(), self.nbytes, _stream_ptr(), self._drop), "team_head_tri_bwd")
+
+    def advance_offset(self):
+        """Next step's dropout masks: offset_dev += 2 (the attention and fc streams of one step use offset and offset + 1),
+        on the device and on the current stream - no host sync, so it can be captured with the step.  No-op at p = 0."""
+        if self._drop is not None:
+            capi.check(capi.lib().team_u64_add(self.offset_dev.data_ptr(), 2, _stream_ptr()), "team_u64_add")
+
+    @property
+    def offset(self) -> int:
+        """The dropout offset the next forward uses (host read: synchronises)."""
+        return int(self.offset_dev.item()) if self._drop is not None else 0
 
     def step(self, image, text, sid, text_cls, cots):
         self.forward(image, text, sid, text_cls)

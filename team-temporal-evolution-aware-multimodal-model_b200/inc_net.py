@@ -293,11 +293,11 @@ class Proof_Net(nn.Module):
 
     def _dropout_active(self) -> bool:
         """The reference applies Dropout(0.1) to the attention probabilities and to the fc output in train mode
-        (convs/projections.py:28,62,84; `.train()` at models/proof.py:398).  The factorised kernels share the softmax of the
-        step rows between all samples, which a per-(sample, query, key) mask would break, so they implement p = 0 only;
-        with dropout active the head runs the token-tensor route instead (encode_* with autograd -> the [B, L, 512] tokens
-        the reference builds -> the stand-alone attention block with its dropout masks, team_mha_fwd / team_mha_bwd): the
-        reference's semantics at the reference's cost model (every token of every sample through q / k / v / fc)."""
+        (convs/projections.py:28,62,84; `.train()` at models/proof.py:398).  With dropout active, ``forward_tri_modal`` with
+        per-sample text (the learner's form) runs the fused head with masks (``head.forward_tri_modal(dropout=...)``: one
+        masked probability row per sample and table query, the same mask bits the token route draws); the class-text
+        form and the PROOF fusion run the token-tensor route (encode_* with autograd -> the [B, L, 512] tokens the
+        reference builds -> the stand-alone attention block with its dropout masks, team_mha_fwd / team_mha_bwd)."""
         return self.training and self.sel_attn.dropout.p > 0
 
     def encode_image(self, x, normalize: bool = False):
@@ -325,7 +325,14 @@ class Proof_Net(nn.Module):
             text = self.tokenizer(text)
         txt = self._txt_feats(text)
         if self._dropout_active():
-            return self._tri_modal_tokens(img, txt, state_ids.to(self._device))
+            if txt.shape[0] != img.shape[0]:
+                return self._tri_modal_tokens(img, txt, state_ids.to(self._device))
+            # seed and offset drawn exactly as MultiHeadAttention.forward draws them: the same torch.manual_seed gives
+            # the same masks (and the same consumption of torch's generator) on either route
+            drop = (float(self.sel_attn.dropout.p), torch.initial_seed(), int(torch.randint(0, 2 ** 62, (1,)).item()) * 2)
+            o = head.forward_tri_modal(self._pack(), img, txt, state_ids.to(self._device), self._protos(),
+                                       mode=self.team_mode, dropout=drop)
+            return o[0], o[1], o[2], o[3], self.convnet.logit_scale.exp()
         if txt.shape[0] != img.shape[0]:          # class texts shared by all samples: text output = mean over them
             if self._wants_grad():
                 return self._tri_modal_tokens(img, txt, state_ids.to(self._device))

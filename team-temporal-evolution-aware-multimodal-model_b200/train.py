@@ -25,8 +25,11 @@ class TrainStep:
     def __init__(self, params: Dict[str, torch.Tensor], img_prototypes: torch.Tensor, batch: int, text_cls: torch.Tensor,
                  mode: int = head.MODE_BF16, init_lr: float = 0.004, min_lr: float = 1e-8, weight_decay: float = 0.05,
                  tuned_epoch: int = 20, logit_scale: float = math.exp(2.6592600369327783),
-                 evolution_features=None):
-        """``params``: the network's parameters under their state_dict names (updated IN PLACE by ``step``)."""
+                 evolution_features=None, dropout_p: float = 0.0, seed: Optional[int] = None):
+        """``params``: the network's parameters under their state_dict names (updated IN PLACE by ``step``).
+        ``dropout_p`` > 0: sel_attn in train mode, as the learner trains it (models/proof.py:398).  Every replay draws
+        fresh masks: step k (counted over all epochs) uses offset ``dropout_offset(k)`` = base + 2 k, advanced on the
+        device inside the graph."""
         capi.require_device()
         self.params, self.mode, self.B = params, mode, batch
         self.pack = head.HeadParamPack.from_state_dict(params)
@@ -35,7 +38,9 @@ class TrainStep:
         dev = pack.flat[0].device
         self.dev = dev
         self.text_cls = text_cls.to(device=dev, dtype=torch.float32).contiguous()
-        self.runner = head.HeadStepRunner(pack, img_prototypes, batch, int(self.text_cls.shape[0]), mode)
+        self.runner = head.HeadStepRunner(pack, img_prototypes, batch, int(self.text_cls.shape[0]), mode,
+                                          dropout_p=dropout_p, seed=seed)
+        self.dropout_base = self.runner.offset
         gv = self.runner.grad_views
         P = pack.T * pack.ppt
         D = capi.D
@@ -91,6 +96,7 @@ class TrainStep:
         with torch.cuda.stream(self._side):
             ops.ce_total(r.logits, y, self.losses6, w_clip=1.0, w_unicl=0.3)
         r.backward(img, txt, sid, [cots[0], cots[1], cots[2], None], g_own_rows=self.g_own)   # the losses never touch the prototype output
+        r.advance_offset()                                                        # next step's dropout masks (no-op at p = 0)
         self.opt.lr = self.lr_at(epoch)
         self.opt.step_graph([g for _, g in self.pairs])
         cur.wait_stream(self._side)
@@ -102,17 +108,24 @@ class TrainStep:
             # warm-up outside the capture (lazy initialisation, autograd buffers) on a snapshot of the trainable state
             snap = [(p.detach().clone(), m.clone(), v.clone()) for p, m, v in zip(self.opt.params, self.opt.exp_avg, self.opt.exp_avg_sq)]
             step0 = self.opt.step_dev.clone()
+            off0 = self.runner.offset_dev.clone() if self.runner.dropout_p else None
             self._body(epoch)
             st.synchronize()
             with torch.no_grad():
                 for p, m, v, (p0, m0, v0) in zip(self.opt.params, self.opt.exp_avg, self.opt.exp_avg_sq, snap):
                     p.copy_(p0); m.copy_(m0); v.copy_(v0)
                 self.opt.step_dev.copy_(step0)
+                if off0 is not None:
+                    self.runner.offset_dev.copy_(off0)
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, stream=st):
                 self._body(epoch)
         torch.cuda.current_stream().wait_stream(st)
         self._graphs[epoch] = g
+
+    def dropout_offset(self, k: int) -> int:
+        """The dropout offset of optimisation step k (0-based, counted over all epochs): base + 2 k."""
+        return self.dropout_base + 2 * k
 
     def load(self, image, text, state_ids, labels):
         """Copy one batch (host or device tensors) into the step's static input buffers on the current stream."""
