@@ -360,6 +360,60 @@ int team_clip_loss(int mode, const float* image, const float* text, int64_t batc
                    float* loss, float* g_image, float* g_text,
                    void* workspace, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------ the same losses under data parallelism
+ * `world` ranks hold `batch` samples each; the global batch is their concatenation in rank order (Bg = world * batch).
+ * Every rank computes the rows of its own samples against the columns of the whole global batch, so together the
+ * ranks compute what team_clip_loss + team_unicl_loss(_evo) + team_ce_total compute on one GPU at batch Bg:
+ *   - losses6 = [total, ce, clip, unicl, unicl_instance, unicl_category], the same values on every rank,
+ *     total = ce + w_clip * clip + w_unicl * unicl;
+ *   - the gradient of that total w.r.t. this rank's rows: g_image / g_text / g_state (the cotangents of the head's three
+ *     feature outputs, unicl) and g_own_rows [2B,512] (image rows, then text rows: ClipLoss on the normalised own rows,
+ *     team_head_grads.g_own_rows).  The head's parameter gradient is then the SUM over ranks of each rank's backward.
+ * The call is split into phases with an exchange between consecutive ones: phase p writes this rank's slice of exchange
+ * p into send[p] (team_loss_shard_xchg_bytes(.., p) bytes), the caller all-gathers the slices of all ranks in rank order
+ * into gathered[p] (world * that many bytes), and phase p + 1 reads it.  Nothing is reduced by the exchange: every sum
+ * over ranks is folded in rank order by the next phase, so the results are deterministic and identical on all ranks.
+ *   exchange 0: per sample [normalised image row | own image row | own text row | label]: the GEMM operands of the B x Bg
+ *               blocks, bf16 in TEAM_MODE_BF16 and fp32 in TEAM_MODE_F32
+ *   exchange 1: per-row statistics (ClipLoss logsumexps, unicl category max / positive / all / valid), the loss partial
+ *               sums and, with evolution features, the (class, state) keyed sums and counts of the state rows
+ *   exchange 2: (evolution features only) the keyed sums of the mixture gradients and the unicl instance loss partial
+ * Phases: team_loss_shard_phases(num_evo) = 3 without evolution features, 4 with them.  All gathered buffers must stay
+ * intact until the last phase; the workspace carries state from phase to phase (same struct, same workspace).
+ * Limits: 1 <= batch <= 16384, 2 <= Bg <= 65536 (the B x Bg similarity and coefficient blocks live in the workspace),
+ * world <= 64.  Equal shards only.  world = 1 is the single-GPU computation.  Pointers: see the fields. */
+typedef struct team_loss_shard {
+    int32_t mode;                  /* TEAM_MODE_F32 / TEAM_MODE_BF16 */
+    int32_t rank, world;
+    int32_t num_evo;               /* rows of evo; 0 = no evolution features */
+    int64_t batch;                 /* samples per rank */
+    int64_t num_classes;           /* columns of logits */
+    const float* image;            /* [B,512] head outputs (un-normalised), as team_unicl_loss */
+    const float* text;
+    const float* state;
+    const float* own_rows;         /* [2B,512] normalised own rows (image, then text), as team_clip_loss's inputs */
+    const float* logits;           /* [B,num_classes] classification logits (value only) */
+    const int64_t* labels;         /* [B] */
+    const int64_t* state_ids;      /* [B] in [0,10); read only with evolution features */
+    const float* evo;              /* [num_evo,512] */
+    const unsigned char* evo_mask; /* [num_evo] */
+    float temperature, logit_scale, w_clip, w_unicl;
+    void* send[3];                 /* this rank's slice of exchange p (written by phase p) */
+    const void* gathered[3];       /* all ranks' slices of exchange p in rank order (read by phases > p) */
+    float* g_image;                /* [B,512] outputs, OVERWRITTEN */
+    float* g_text;
+    float* g_state;
+    float* g_own_rows;             /* [2B,512] */
+    float* losses6;                /* [6], written by the last phase */
+    void* workspace;               /* 256-byte aligned */
+    size_t workspace_bytes;
+} team_loss_shard;
+int team_loss_shard_phases(int32_t num_evo);
+size_t team_loss_shard_workspace_bytes(int32_t mode, int64_t batch, int32_t world, int32_t num_evo);
+/* bytes of ONE rank's slice of exchange `exchange` (0 = no such exchange) */
+size_t team_loss_shard_xchg_bytes(int32_t mode, int64_t batch, int32_t num_evo, int32_t exchange);
+int team_loss_shard_run(int32_t phase, const team_loss_shard* s, void* stream);
+
 /* Fused multi-tensor AdamW step (SURVEY 8f "next").
  * Replaces: torch.optim.AdamW(...).step()    models/proof.py:361, :445  (decoupled weight decay, bias correction,
  * amsgrad off).  params / grads / exp_avg / exp_avg_sq: HOST arrays of n_tensors device pointers (fp32, numel[i]

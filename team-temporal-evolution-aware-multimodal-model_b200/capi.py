@@ -84,6 +84,17 @@ class GemmDesc(C.Structure):
                 ("A2", C.c_void_p), ("lda2", C.c_int64), ("B2", C.c_void_p), ("ldb2", C.c_int64)]
 
 
+class LossShard(C.Structure):
+    _fields_ = ([("mode", C.c_int32), ("rank", C.c_int32), ("world", C.c_int32), ("num_evo", C.c_int32),
+                 ("batch", C.c_int64), ("num_classes", C.c_int64)] +
+                [(n, C.c_void_p) for n in ("image", "text", "state", "own_rows", "logits", "labels", "state_ids", "evo",
+                                           "evo_mask")] +
+                [(n, C.c_float) for n in ("temperature", "logit_scale", "w_clip", "w_unicl")] +
+                [("send", C.c_void_p * 3), ("gathered", C.c_void_p * 3)] +
+                [(n, C.c_void_p) for n in ("g_image", "g_text", "g_state", "g_own_rows", "losses6", "workspace")] +
+                [("workspace_bytes", C.c_size_t)])
+
+
 _lib = None
 _lock = threading.Lock()
 
@@ -166,6 +177,14 @@ def _declare(lib):
         lib.team_unicl_loss_evo.argtypes = [i32, vp, vp, vp, vp, vp, vp, vp, i32, i64, C.c_float, C.c_float, vp, vp, vp, vp, vp, sz, vp]
         lib.team_clip_loss.restype = i32
         lib.team_clip_loss.argtypes = [i32, vp, vp, i64, C.c_float, C.c_float, vp, vp, vp, vp, sz, vp]
+        lib.team_loss_shard_phases.restype = i32
+        lib.team_loss_shard_phases.argtypes = [C.c_int32]
+        lib.team_loss_shard_workspace_bytes.restype = sz
+        lib.team_loss_shard_workspace_bytes.argtypes = [C.c_int32, i64, C.c_int32, C.c_int32]
+        lib.team_loss_shard_xchg_bytes.restype = sz
+        lib.team_loss_shard_xchg_bytes.argtypes = [C.c_int32, i64, C.c_int32, C.c_int32]
+        lib.team_loss_shard_run.restype = i32
+        lib.team_loss_shard_run.argtypes = [C.c_int32, C.POINTER(LossShard), vp]
         lib.team_head_tri_classtext_fwd.restype = i32
         lib.team_head_tri_classtext_fwd.argtypes = [C.POINTER(HeadWeights), i32, i64, vp, vp, i64, vp, vp, vp, vp, vp, vp, sz, vp]
         lib.team_head_proof_fwd.restype = i32

@@ -85,10 +85,13 @@ loss_normalize_kernel(int64_t B, const float* __restrict__ x0, const float* __re
     if (lane == 0 && iv != nullptr) iv[b] = s;
 }
 
-// category term, per row i of sim / tau: max over ALL j, pos = sum_{j != i, y_j == y_i} e_j, all = sum_{j != i} e_j
+// category term, per row i of sim / tau: max over ALL j, pos = sum_{j != i, y_j == y_i} e_j, all = sum_{j != i} e_j.
+// Rows are the B samples starting at global row r0, columns the ncols samples of the (global) batch: the diagonal is
+// column r0 + i.  Single GPU: r0 = 0, ncols = B.
 __global__ void __launch_bounds__(256)
-unicl_cat_stats_kernel(int B, int ld, const float* __restrict__ sim, const int64_t* __restrict__ labels, float inv_tau,
-                       float* __restrict__ rmax, float* __restrict__ rpos, float* __restrict__ rall, float* __restrict__ rloss) {
+unicl_cat_stats_kernel(int B, int ncols, int r0, int ld, const float* __restrict__ sim, const int64_t* __restrict__ labels,
+                       float inv_tau, float* __restrict__ rmax, float* __restrict__ rpos, float* __restrict__ rall,
+                       float* __restrict__ rloss, float* __restrict__ rvalid) {
     pdl_trigger();
     pdl_wait();
     const int lane = threadIdx.x & 31;
@@ -98,17 +101,17 @@ unicl_cat_stats_kernel(int B, int ld, const float* __restrict__ sim, const int64
     // the compiler's own unrolling the two passes were chains of L2 round trips (16 us at B = 1 024, tools/timeline_train.py)
     const float4* row4 = reinterpret_cast<const float4*>(sim + (size_t)i * ld);
     const longlong2* lab2 = reinterpret_cast<const longlong2*>(labels);
-    const int64_t yi = labels[i];
-    const int n4 = (B + 3) >> 2;
+    const int64_t yi = labels[r0 + i];
+    const int n4 = (ncols + 3) >> 2;
     float mx = -INFINITY;
 #pragma unroll 4
     for (int q = lane; q < n4; q += 32) {
         const float4 v = row4[q];
         const int j = 4 * q;
         mx = fmaxf(mx, v.x * inv_tau);
-        if (j + 1 < B) mx = fmaxf(mx, v.y * inv_tau);
-        if (j + 2 < B) mx = fmaxf(mx, v.z * inv_tau);
-        if (j + 3 < B) mx = fmaxf(mx, v.w * inv_tau);
+        if (j + 1 < ncols) mx = fmaxf(mx, v.y * inv_tau);
+        if (j + 2 < ncols) mx = fmaxf(mx, v.z * inv_tau);
+        if (j + 3 < ncols) mx = fmaxf(mx, v.w * inv_tau);
     }
     mx = warp_max(mx);
     float pos = 0.f, all = 0.f;
@@ -117,17 +120,17 @@ unicl_cat_stats_kernel(int B, int ld, const float* __restrict__ sim, const int64
         const float4 v = row4[q];
         const int j = 4 * q;
         long long y[4];
-        if (j + 3 < B) {
+        if (j + 3 < ncols) {
             const longlong2 la = lab2[2 * q], lb = lab2[2 * q + 1];
             y[0] = la.x; y[1] = la.y; y[2] = lb.x; y[3] = lb.y;
         } else {
 #pragma unroll
-            for (int u = 0; u < 4; ++u) y[u] = j + u < B ? labels[j + u] : -1;
+            for (int u = 0; u < 4; ++u) y[u] = j + u < ncols ? labels[j + u] : -1;
         }
         const float x[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            if (j + u >= B || j + u == i) continue;
+            if (j + u >= ncols || j + u == r0 + i) continue;
             const float e = expf(x[u] * inv_tau - mx);
             all += e;
             if (y[u] == yi) pos += e;
@@ -138,7 +141,7 @@ unicl_cat_stats_kernel(int B, int ld, const float* __restrict__ sim, const int64
         const bool valid = pos > 0.f && all > 0.f;
         rmax[i] = mx; rpos[i] = pos; rall[i] = all;
         rloss[i] = valid ? -logf(pos / (all + 1e-8f)) : 0.f;
-        rmax[B + i] = valid ? 1.f : 0.f;                      // valid flag
+        rvalid[i] = valid ? 1.f : 0.f;
     }
 }
 
@@ -170,55 +173,70 @@ loss_fold2_kernel(int n, const float* __restrict__ a, const float* __restrict__ 
     }
 }
 
-// G[i][j] = d(0.5 * grad_scale * category_loss) / d(sim_ij)   (scal[0] = valid count)
+// G[i][j] = d(0.5 * grad_scale * category_loss) / d(sim_ij)   (scal[0] = valid count); rows r0 + [0, B), ncols columns.
+// With column statistics (cmax != null, indexed by column) the kernel also writes the transposed half
+// H[i][j] = G[j][r0 + i] (sim is symmetric) into H: dcat of the rows is then G X + H X over all columns, one GEMM of two
+// K-segments, and H is rounded to bf16 entry by entry like the single-GPU G^T.
 __global__ void __launch_bounds__(256)
-unicl_cat_grad_kernel(int B, int ld, const float* __restrict__ sim, const int64_t* __restrict__ labels, float inv_tau,
-                      float weight, const float* __restrict__ rmax, const float* __restrict__ rpos,
-                      const float* __restrict__ rall, const float* __restrict__ scal, float* __restrict__ G,
-                      __nv_bfloat16* __restrict__ Gh) {
+unicl_cat_grad_kernel(int B, int ncols, int r0, int ld, const float* __restrict__ sim, const int64_t* __restrict__ labels,
+                      float inv_tau, float weight, const float* __restrict__ rmax, const float* __restrict__ rpos,
+                      const float* __restrict__ rall, const float* __restrict__ rvalid, const float* __restrict__ cmax,
+                      const float* __restrict__ cpos, const float* __restrict__ call, const float* __restrict__ cvalid,
+                      const float* __restrict__ scal, float* __restrict__ G, __nv_bfloat16* __restrict__ Gh,
+                      float* __restrict__ H, __nv_bfloat16* __restrict__ Hh) {
     pdl_trigger();
     pdl_wait();
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * 8 + (threadIdx.x >> 5);
     if (i >= B) return;
     const float nvalid = scal[0];
-    const bool valid = rmax[B + i] != 0.f && nvalid > 0.f;
-    const float k = valid ? weight * inv_tau / nvalid : 0.f;
+    const bool valid = rvalid[i] != 0.f && nvalid > 0.f;
+    const float kk = nvalid > 0.f ? weight * inv_tau / nvalid : 0.f;
+    const float k = valid ? kk : 0.f;
     const float mx = rmax[i], ip = valid ? 1.0f / rpos[i] : 0.f, ia = valid ? 1.0f / (rall[i] + 1e-8f) : 0.f;
-    const int64_t yi = labels[i];
+    const int64_t yi = labels[r0 + i];
     const float4* row4 = reinterpret_cast<const float4*>(sim + (size_t)i * ld);
     const longlong2* lab2 = reinterpret_cast<const longlong2*>(labels);
     float4* g4 = reinterpret_cast<float4*>(G + (size_t)i * ld);
     uint2* h4 = Gh != nullptr ? reinterpret_cast<uint2*>(Gh + (size_t)i * ld) : nullptr;
+    float4* t4 = H != nullptr ? reinterpret_cast<float4*>(H + (size_t)i * ld) : nullptr;
+    uint2* th4 = Hh != nullptr ? reinterpret_cast<uint2*>(Hh + (size_t)i * ld) : nullptr;
 #pragma unroll 4
     for (int q = lane; q < ld / 4; q += 32) {
         const int j = 4 * q;
-        float g[4] = {0.f, 0.f, 0.f, 0.f};
-        if (valid && j < B) {
+        float g[4] = {0.f, 0.f, 0.f, 0.f}, t[4] = {0.f, 0.f, 0.f, 0.f};
+        if ((valid || cmax != nullptr) && j < ncols) {
             const float4 v = row4[q];
             long long y[4];
-            if (j + 3 < B) {
+            if (j + 3 < ncols) {
                 const longlong2 la = lab2[2 * q], lb = lab2[2 * q + 1];
                 y[0] = la.x; y[1] = la.y; y[2] = lb.x; y[3] = lb.y;
             } else {
 #pragma unroll
-                for (int u = 0; u < 4; ++u) y[u] = j + u < B ? labels[j + u] : -1;
+                for (int u = 0; u < 4; ++u) y[u] = j + u < ncols ? labels[j + u] : -1;
             }
             const float x[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
-                if (j + u >= B || j + u == i) continue;
-                const float e = expf(x[u] * inv_tau - mx);
-                g[u] = k * e * (ia - (y[u] == yi ? ip : 0.f));
+                const int c = j + u;
+                if (c >= ncols || c == r0 + i) continue;
+                if (valid) g[u] = k * expf(x[u] * inv_tau - mx) * (ia - (y[u] == yi ? ip : 0.f));
+                if (cmax != nullptr && cvalid[c] != 0.f)
+                    t[u] = kk * expf(x[u] * inv_tau - cmax[c]) * (1.0f / (call[c] + 1e-8f) - (y[u] == yi ? 1.0f / cpos[c] : 0.f));
             }
         }
         const float4 o = make_float4(g[0], g[1], g[2], g[3]);
         g4[q] = o;
         if (h4 != nullptr) h4[q] = pack_bf16x4(o);
+        if (t4 != nullptr) {
+            const float4 ot = make_float4(t[0], t[1], t[2], t[3]);
+            t4[q] = ot;
+            if (th4 != nullptr) th4[q] = pack_bf16x4(ot);
+        }
     }
 }
 
-// instance term + assembly of the three cotangents (warp per sample):
+// instance term + assembly of the three cotangents (warp per sample; rloss may be null, g_image null = loss only):
 //   3 x 3 similarities of (image, text, state) / tau; row r: pos = 1 + sum_{c != r} e_rc, all = sum_c e_rc,
 //   loss -= log(pos / (all + 1e-8));  then d total / d xhat = instance part + dcat (image only), normalise-backward.
 __global__ void __launch_bounds__(256)
@@ -255,7 +273,8 @@ unicl_instance_kernel(int B, const float* __restrict__ Xi, const float* __restri
 #pragma unroll
         for (int c = 0; c < 3; ++c) wgt[r][c] = c == r ? e[c] * ia : e[c] * (ia - ip);
     }
-    if (lane == 0) rloss[b] = loss;
+    if (lane == 0 && rloss != nullptr) rloss[b] = loss;
+    if (g_image == nullptr) return;                      // loss only (data-parallel form: the value is exchanged first)
     const float k = inst_weight * inv_tau;
     const float* invs[3] = {inv_i, inv_t, inv_s};
     float* outs[3] = {g_image, g_text, g_state};
@@ -312,8 +331,12 @@ evo_keysum_kernel(int B, const float* __restrict__ rows, const unsigned char* __
     pdl_trigger();
     pdl_wait();
     const int key = blockIdx.x, c = key / EVO_NS, st = key - c * EVO_NS;
-    if (!evo_mask[c]) return;
     const int t = threadIdx.x, lane = t & 31;
+    if (!evo_mask[c]) {                  // defined zeros (the data-parallel form exchanges every key)
+        reinterpret_cast<float4*>(out + (size_t)key * D)[t] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (cnt != nullptr && t == 0) cnt[key] = 0;
+        return;
+    }
     const int nwords = (B + 31) / 32;
 #pragma unroll 4
     for (int base = 0; base < nwords * 32; base += 128) {
@@ -495,9 +518,10 @@ evo_bwd2_kernel(int B, const float* __restrict__ Xs, const float* __restrict__ i
     st_row(g_state + (size_t)b * D, lane, d);
 }
 
-// ---- ClipLoss: per row of s * L (rows [0,B): image->text from L, rows [B,2B): text->image from L^T): lse and loss
+// ---- ClipLoss: per row of s * L (rows [0,B): image->text from L, rows [B,2B): text->image from L^T): lse and loss.
+// The rows are the samples r0 + [0, B) against ncols columns (single GPU: r0 = 0, ncols = B).
 __global__ void __launch_bounds__(256)
-clip_stats_kernel(int B, int ld, const float* __restrict__ L, const float* __restrict__ LT, float scale,
+clip_stats_kernel(int B, int ncols, int r0, int ld, const float* __restrict__ L, const float* __restrict__ LT, float scale,
                   float* __restrict__ lse, float* __restrict__ rloss) {
     pdl_trigger();
     pdl_wait();
@@ -507,16 +531,16 @@ clip_stats_kernel(int B, int ld, const float* __restrict__ L, const float* __res
     const int i = r < B ? r : r - B;
     const float* row = (r < B ? L : LT) + (size_t)i * ld;
     const float4* row4 = reinterpret_cast<const float4*>(row);
-    const int n4 = (B + 3) >> 2;
+    const int n4 = (ncols + 3) >> 2;
     float mx = -INFINITY;
 #pragma unroll 4
     for (int q = lane; q < n4; q += 32) {
         const float4 v = row4[q];
         const int j = 4 * q;
         mx = fmaxf(mx, v.x * scale);
-        if (j + 1 < B) mx = fmaxf(mx, v.y * scale);
-        if (j + 2 < B) mx = fmaxf(mx, v.z * scale);
-        if (j + 3 < B) mx = fmaxf(mx, v.w * scale);
+        if (j + 1 < ncols) mx = fmaxf(mx, v.y * scale);
+        if (j + 2 < ncols) mx = fmaxf(mx, v.z * scale);
+        if (j + 3 < ncols) mx = fmaxf(mx, v.w * scale);
     }
     mx = warp_max(mx);
     float z = 0.f;
@@ -525,27 +549,30 @@ clip_stats_kernel(int B, int ld, const float* __restrict__ L, const float* __res
         const float4 v = row4[q];
         const int j = 4 * q;
         z += expf(v.x * scale - mx);
-        if (j + 1 < B) z += expf(v.y * scale - mx);
-        if (j + 2 < B) z += expf(v.z * scale - mx);
-        if (j + 3 < B) z += expf(v.w * scale - mx);
+        if (j + 1 < ncols) z += expf(v.y * scale - mx);
+        if (j + 2 < ncols) z += expf(v.z * scale - mx);
+        if (j + 3 < ncols) z += expf(v.w * scale - mx);
     }
     z = warp_sum(z);
     if (lane == 0) {
         const float l = logf(z) + mx;
         lse[r] = l;
-        rloss[r] = l - row[i] * scale;
+        rloss[r] = l - row[r0 + i] * scale;
     }
 }
 // G[i][j] = d(grad_scale * loss) / d(L_ij) = k * (softmax_i2t[i][j] + softmax_t2i[j][i] - 2 delta_ij),  k = scale*grad_scale/(2B)
+// lse_row: the logsumexps of the B rows (row r0 + i of the global L), lse_col: those of the ncols columns' other direction.
+// Fed L^T's rows with the two vectors swapped it gives the rows of G^T (data-parallel form).
 __global__ void __launch_bounds__(256)
-clip_grad_kernel(int B, int ld, const float* __restrict__ L, float scale, float k, const float* __restrict__ lse,
-                 float* __restrict__ G, __nv_bfloat16* __restrict__ Gh) {
+clip_grad_kernel(int B, int ncols, int r0, int ld, const float* __restrict__ L, float scale, float k,
+                 const float* __restrict__ lse_row, const float* __restrict__ lse_col, float* __restrict__ G,
+                 __nv_bfloat16* __restrict__ Gh) {
     pdl_trigger();
     pdl_wait();
     const int lane = threadIdx.x & 31;
     const int i = blockIdx.x * 8 + (threadIdx.x >> 5);
     if (i >= B) return;
-    const float li = lse[i];
+    const float li = lse_row[i];
     const float4* row4 = reinterpret_cast<const float4*>(L + (size_t)i * ld);
     float4* g4 = reinterpret_cast<float4*>(G + (size_t)i * ld);
     uint2* h4 = Gh != nullptr ? reinterpret_cast<uint2*>(Gh + (size_t)i * ld) : nullptr;
@@ -553,12 +580,12 @@ clip_grad_kernel(int B, int ld, const float* __restrict__ L, float scale, float 
     for (int q = lane; q < ld / 4; q += 32) {
         const int j = 4 * q;
         float g[4] = {0.f, 0.f, 0.f, 0.f};
-        if (j < B) {
+        if (j < ncols) {
             const float4 v = row4[q];
             const float x[4] = {v.x * scale, v.y * scale, v.z * scale, v.w * scale};
 #pragma unroll
             for (int u = 0; u < 4; ++u)
-                if (j + u < B) g[u] = k * (expf(x[u] - li) + expf(x[u] - lse[B + j + u]) - (j + u == i ? 2.f : 0.f));
+                if (j + u < ncols) g[u] = k * (expf(x[u] - li) + expf(x[u] - lse_col[j + u]) - (j + u == r0 + i ? 2.f : 0.f));
         }
         const float4 o = make_float4(g[0], g[1], g[2], g[3]);
         g4[q] = o;
@@ -642,9 +669,11 @@ static int unicl_impl(int mode, const float* image, const float* text, const flo
         seg(wv.add(B, B, 0.f, Mat{w.sim, nullptr, ld}), false, w.X[0], false, w.X[0], D);
         if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     }
-    TEAM_LAUNCH(unicl_cat_stats_kernel, (B + 7) / 8, 256, 0, st, B, ld, w.sim, labels, inv_tau, w.rmax, w.rpos, w.rall, w.rloss);
+    TEAM_LAUNCH(unicl_cat_stats_kernel, (B + 7) / 8, 256, 0, st, B, B, 0, ld, w.sim, labels, inv_tau, w.rmax, w.rpos, w.rall, w.rloss, w.rmax + B);
     TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, B, w.rmax + B, w.rloss, w.scal, 0, 0.f, (const float*)nullptr, (float*)nullptr);   // valid count, category sum
-    TEAM_LAUNCH(unicl_cat_grad_kernel, (B + 7) / 8, 256, 0, st, B, ld, w.sim, labels, inv_tau, 0.5f * grad_scale, w.rmax, w.rpos, w.rall, w.scal, w.G.f, bf ? w.G.h : nullptr);
+    TEAM_LAUNCH(unicl_cat_grad_kernel, (B + 7) / 8, 256, 0, st, B, B, 0, ld, w.sim, labels, inv_tau, 0.5f * grad_scale, w.rmax, w.rpos, w.rall, w.rmax + B,
+                (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, w.scal, w.G.f, bf ? w.G.h : nullptr,
+                (float*)nullptr, (__nv_bfloat16*)nullptr);
     {   // dcat = G Xi + G^T Xi
         Wave wv;
         seg(seg(wv.add(B, D, 0.f, Mat{w.dcat, nullptr, D}), false, w.G, true, w.X[0], B), true, w.G, true, w.X[0], B);
@@ -674,7 +703,7 @@ extern "C" int team_unicl_loss(int mode, const float* image, const float* text, 
 // One CTA, rows strided over the threads, block fold in a fixed order (deterministic).
 __global__ void __launch_bounds__(1024)
 ce_total_kernel(int B, int C, const float* __restrict__ logits, const int64_t* __restrict__ labels, float w_clip, float w_unicl,
-                float* __restrict__ losses6) {
+                float* __restrict__ losses6, float* __restrict__ partial) {
     __shared__ float part[1024];
     pdl_trigger();
     pdl_wait();
@@ -694,7 +723,9 @@ ce_total_kernel(int B, int C, const float* __restrict__ logits, const int64_t* _
         if ((int)threadIdx.x < o) part[threadIdx.x] += part[threadIdx.x + o];
         __syncthreads();
     }
-    if (threadIdx.x == 0) {
+    if (threadIdx.x == 0 && partial != nullptr) {      // data-parallel form: the shard's sum; mean and total after the exchange
+        partial[0] = part[0];
+    } else if (threadIdx.x == 0) {
         const float ce = part[0] / (float)B;
         losses6[1] = ce;
         losses6[0] = ce + w_clip * losses6[2] + w_unicl * losses6[3];
@@ -705,7 +736,7 @@ extern "C" int team_ce_total(const float* logits, const int64_t* labels, int64_t
                              float w_unicl, float* losses6, void* stream) {
     TEAM_REQUIRE(logits && labels && losses6 && batch >= 1 && batch < (1ll << 31) && num_classes >= 1 && num_classes < (1 << 20),
                  "ce_total: bad arguments");
-    TEAM_LAUNCH(ce_total_kernel, 1, 1024, 0, (cudaStream_t)stream, (int)batch, (int)num_classes, logits, labels, w_clip, w_unicl, losses6);
+    TEAM_LAUNCH(ce_total_kernel, 1, 1024, 0, (cudaStream_t)stream, (int)batch, (int)num_classes, logits, labels, w_clip, w_unicl, losses6, (float*)nullptr);
     return TEAM_OK;
 }
 
@@ -745,12 +776,319 @@ extern "C" int team_clip_loss(int mode, const float* image, const float* text, i
     if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     seg(wv.add(B, B, 0.f, Mat{w.simT, nullptr, ld}), false, w.X[1], false, w.X[0], D);              // L^T = T I^T
     if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
-    TEAM_LAUNCH(clip_stats_kernel, (2 * B + 7) / 8, 256, 0, st, B, ld, w.sim, w.simT, logit_scale, w.rmax, w.rloss);
+    TEAM_LAUNCH(clip_stats_kernel, (2 * B + 7) / 8, 256, 0, st, B, B, 0, ld, w.sim, w.simT, logit_scale, w.rmax, w.rloss);
     TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, 2 * B, w.rloss, (const float*)nullptr, w.scal, 1, 1.0f / (2.0f * (float)B), (const float*)nullptr, loss);
-    TEAM_LAUNCH(clip_grad_kernel, (B + 7) / 8, 256, 0, st, B, ld, w.sim, logit_scale, logit_scale * grad_scale / (2.0f * (float)B), w.rmax, w.G.f, bf ? w.G.h : nullptr);
+    TEAM_LAUNCH(clip_grad_kernel, (B + 7) / 8, 256, 0, st, B, B, 0, ld, w.sim, logit_scale, logit_scale * grad_scale / (2.0f * (float)B), w.rmax, w.rmax + B, w.G.f, bf ? w.G.h : nullptr);
     seg(wv.add(B, D, 0.f, Mat{g_image, nullptr, D}), false, w.G, true, w.X[1], B);                  // dI = G T
     if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
     seg(wv.add(B, D, 0.f, Mat{g_text, nullptr, D}), true, w.G, true, w.X[0], B);                    // dT = G^T I
     if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
+    return TEAM_OK;
+}
+
+// ------------------------------------------------------------------ data-parallel form (team_loss_shard_*)
+// Rank r owns the global rows r0 + [0, B), r0 = r B.  The similarity blocks are B x Bg (own rows against every column)
+// and the kernels above run on them with (r0, ncols = Bg); the exchanges only move slices, every sum over ranks is a
+// rank-order fold in the next phase.  See include/team_b200.h for the phases and the exchanges.
+namespace team {
+
+constexpr int64_t SHARD_MAX_GLOBAL = 65536;
+constexpr int SHARD_MAX_WORLD = 64;
+
+// exchange 0 row: [normalised image | own image | own text | label (int64), 0 (int64)] in the GEMM operand format
+static int64_t shard_row_ld(int mode) { return 3 * D + (mode == TEAM_MODE_BF16 ? 8 : 4); }
+static int shard_elem(int mode) { return mode == TEAM_MODE_BF16 ? 2 : 4; }
+
+// float offsets inside one rank's slice of exchanges 1 and 2
+struct ShardX {
+    int64_t keys;
+    int64_t x1_scal, x1_ss, x1_cnt;       // exchange 1: columns [6][B] at 0 (lse i2t, lse t2i, max, pos, all, valid)
+    int64_t x2_scal;                      // exchange 2: DM [keys][D] at 0
+    size_t bytes[3];
+};
+// scalar slots of an exchange: 0 valid count, 1 category sum, 2 clip sum, 4 ce sum, 5 instance sum (3, 6, 7: zero)
+static void shard_xplan(int mode, int64_t B, int num_evo, ShardX* x) {
+    const int64_t a = 64;                             // 256 bytes in floats
+    auto up = [&](int64_t n) { return (n + a - 1) / a * a; };
+    x->keys = (int64_t)num_evo * EVO_NS;
+    x->bytes[0] = (size_t)(B * shard_row_ld(mode) * shard_elem(mode));     // no padding: the gathered rows are one matrix
+    x->x1_scal = up(6 * B);
+    int64_t n1 = x->x1_scal + a;
+    x->x1_ss = n1;
+    x->x1_cnt = num_evo ? x->x1_ss + up(x->keys * D) : n1;
+    if (num_evo) n1 = x->x1_cnt + up(x->keys);
+    x->bytes[1] = (size_t)n1 * 4;
+    x->x2_scal = up(x->keys * D);
+    x->bytes[2] = num_evo ? (size_t)(x->x2_scal + a) * 4 : 0;
+}
+
+struct ShardWS {
+    float* X[3]; float* inv[3];
+    int64_t* labels_g;        // [Bg]
+    Mat S[3];                 // [B][Bgp] fp32: 0 unicl X_loc X_g^T, 1 ClipLoss I_loc T_g^T, 2 T_loc I_g^T
+    Mat G[4];                 // [B][Bgp] coefficients (+ bf16 shadow in BF16 mode): 0 unicl G, 1 ClipLoss G, 2 G^T, 3 unicl H
+    float* rloss;             // [3B]: ClipLoss rows [2B], unicl category rows [B]
+    float* rinst;             // [B]
+    float* cols;              // [6][Bg] gathered per-row statistics, column-contiguous
+    float* scal;              // [8] global sums (slots as in the exchange)
+    float* dcat;              // [B][D]
+    void* gemm_ws; size_t gemm_ws_bytes;
+    float *Xe, *Mh, *dXe, *dMix, *SS, *DM, *sc; int* cnt; unsigned char* rowmask;
+    size_t total;
+};
+static void shard_plan(int mode, int64_t B, int world, int num_evo, void* base, ShardWS* w) {
+    size_t off = 0;
+    auto take = [&](size_t bytes) -> char* {
+        char* p = base ? reinterpret_cast<char*>(base) + off : nullptr;
+        off += align_up(bytes, 256);
+        return p;
+    };
+    const int64_t Bg = B * world, Bgp = (Bg + 7) / 8 * 8;
+    for (int i = 0; i < 3; ++i) {
+        w->X[i] = reinterpret_cast<float*>(take((size_t)B * D * 4));
+        w->inv[i] = reinterpret_cast<float*>(take((size_t)B * 4));
+    }
+    w->labels_g = reinterpret_cast<int64_t*>(take((size_t)Bg * 8));
+    for (int i = 0; i < 3; ++i) w->S[i] = Mat{reinterpret_cast<float*>(take((size_t)B * Bgp * 4)), nullptr, Bgp};
+    for (int i = 0; i < 4; ++i) {
+        w->G[i].f = reinterpret_cast<float*>(take((size_t)B * Bgp * 4));
+        w->G[i].h = mode == TEAM_MODE_BF16 ? reinterpret_cast<__nv_bfloat16*>(take((size_t)B * Bgp * 2)) : nullptr;
+        w->G[i].ld = Bgp;
+    }
+    w->rloss = reinterpret_cast<float*>(take((size_t)3 * B * 4));
+    w->rinst = reinterpret_cast<float*>(take((size_t)B * 4));
+    w->cols = reinterpret_cast<float*>(take((size_t)6 * Bg * 4));
+    w->scal = reinterpret_cast<float*>(take(8 * 4));
+    w->dcat = reinterpret_cast<float*>(take((size_t)B * D * 4));
+    w->gemm_ws_bytes = 64u << 20;
+    w->gemm_ws = take(w->gemm_ws_bytes);
+    w->Xe = w->Mh = w->dXe = w->dMix = w->SS = w->DM = w->sc = nullptr;
+    w->cnt = nullptr; w->rowmask = nullptr;
+    if (num_evo) off += evo_plan(B, num_evo, base ? reinterpret_cast<char*>(base) + off : nullptr, &w->Xe, &w->Mh, &w->dXe,
+                                 &w->dMix, &w->SS, &w->DM, &w->cnt, &w->sc, &w->rowmask);
+    w->total = off;
+}
+
+// exchange 0 rows of this rank (warp per row segment: image xhat, own image, own text)
+__global__ void __launch_bounds__(256)
+shard_pack_rows_kernel(int B, const float* __restrict__ Xi, const float* __restrict__ own, const int64_t* __restrict__ labels,
+                       int bf, int64_t ld, void* __restrict__ rows) {
+    pdl_trigger();
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int r = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (r >= 3 * B) return;
+    const int k = r / B, b = r - k * B;
+    float4 v[4];
+    ld_row(k == 0 ? Xi + (size_t)b * D : own + ((size_t)(k - 1) * B + b) * D, lane, v);
+    char* row = reinterpret_cast<char*>(rows) + (size_t)b * ld * (bf ? 2 : 4);
+    if (bf) st_row_h(reinterpret_cast<__nv_bfloat16*>(row) + k * D, lane, v);
+    else st_row(reinterpret_cast<float*>(row) + k * D, lane, v);
+    if (k == 0 && lane == 0) {
+        int64_t* meta = reinterpret_cast<int64_t*>(row + (size_t)3 * D * (bf ? 2 : 4));
+        meta[0] = labels[b]; meta[1] = 0;
+    }
+}
+
+__global__ void __launch_bounds__(256)
+shard_labels_kernel(int Bg, const void* __restrict__ rows, int64_t row_bytes, int64_t meta_off, int64_t* __restrict__ labels) {
+    pdl_trigger();
+    pdl_wait();
+    const int j = blockIdx.x * 256 + threadIdx.x;
+    if (j < Bg) labels[j] = *reinterpret_cast<const int64_t*>(reinterpret_cast<const char*>(rows) + (size_t)j * row_bytes + meta_off);
+}
+
+// gathered per-row vectors [world][nvec][B] (+ slice stride) -> [nvec][Bg], column j = rank * B + i
+__global__ void __launch_bounds__(256)
+shard_cols_kernel(int B, int Bg, int nvec, const float* __restrict__ g, int64_t slice, float* __restrict__ out) {
+    pdl_trigger();
+    pdl_wait();
+    const int64_t e = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (e >= (int64_t)nvec * Bg) return;
+    const int v = (int)(e / Bg), j = (int)(e - (int64_t)v * Bg), w = j / B, i = j - w * B;
+    out[e] = g[(size_t)w * slice + (size_t)v * B + i];
+}
+
+// out[e] = sum over ranks of g[w * slice + e], in rank order
+template <typename T>
+__global__ void __launch_bounds__(256)
+shard_sum_kernel(int world, int64_t n, const T* __restrict__ g, int64_t slice, T* __restrict__ out) {
+    pdl_trigger();
+    pdl_wait();
+    const int64_t e = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (e >= n) return;
+    T s = g[e];
+    for (int w = 1; w < world; ++w) s += g[(size_t)w * slice + e];
+    out[e] = s;
+}
+
+// global sums of the scalar slots (exchange 1; the instance sum from exchange 2 when given) and, when losses6 is given,
+// the six loss values
+__global__ void __launch_bounds__(32)
+shard_losses_kernel(int world, const float* __restrict__ g1, int64_t slice1, const float* __restrict__ g2, int64_t slice2,
+                    int64_t Bg, float w_clip, float w_unicl, float* __restrict__ scal, float* __restrict__ losses6) {
+    pdl_trigger();
+    pdl_wait();
+    if (threadIdx.x != 0) return;
+    float v[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    for (int w = 0; w < world; ++w)
+        for (int s = 0; s < 6; ++s) v[s] += g1[(size_t)w * slice1 + s];
+    if (g2 != nullptr) {
+        v[5] = 0.f;
+        for (int w = 0; w < world; ++w) v[5] += g2[(size_t)w * slice2 + 5];
+    }
+    for (int s = 0; s < 6; ++s) scal[s] = v[s];
+    if (losses6 == nullptr) return;
+    const float n = (float)Bg;
+    const float cat = v[0] > 0.f ? v[1] / v[0] : 0.f, inst = v[5] / (3.0f * n), clip = v[2] / (2.0f * n), ce = v[4] / n;
+    const float unicl = inst + 0.5f * cat;
+    losses6[0] = ce + w_clip * clip + w_unicl * unicl;
+    losses6[1] = ce; losses6[2] = clip; losses6[3] = unicl; losses6[4] = inst; losses6[5] = cat;
+}
+
+static int shard_check(int32_t phase, const team_loss_shard* s, ShardWS& w, ShardX& x) {
+    TEAM_REQUIRE(s != nullptr, "loss_shard: null struct");
+    TEAM_REQUIRE(s->mode == TEAM_MODE_F32 || s->mode == TEAM_MODE_BF16, "loss_shard: bad mode %d", s->mode);
+    TEAM_REQUIRE(s->world >= 1 && s->world <= SHARD_MAX_WORLD && s->rank >= 0 && s->rank < s->world,
+                 "loss_shard: rank %d / world %d", s->rank, s->world);
+    const int64_t Bg = s->batch * s->world;
+    TEAM_REQUIRE(s->batch >= 1 && s->batch <= LOSS_MAX_BATCH && Bg >= 2 && Bg <= SHARD_MAX_GLOBAL,
+                 "loss_shard: batch %lld x world %d out of range (batch <= %lld, 2 <= global batch <= %lld)",
+                 (long long)s->batch, s->world, (long long)LOSS_MAX_BATCH, (long long)SHARD_MAX_GLOBAL);
+    TEAM_REQUIRE(s->num_evo >= 0 && s->num_evo <= 4096, "loss_shard: num_evo %d", s->num_evo);
+    TEAM_REQUIRE(s->num_classes >= 1 && s->num_classes < (1 << 20), "loss_shard: num_classes %lld", (long long)s->num_classes);
+    TEAM_REQUIRE(s->temperature > 0.f, "loss_shard: temperature must be positive");
+    const int P = s->num_evo ? 4 : 3;
+    TEAM_REQUIRE(phase >= 0 && phase < P, "loss_shard: phase %d of %d", phase, P);
+    TEAM_REQUIRE(s->image && s->text && s->state && s->own_rows && s->logits && s->labels && s->g_image && s->g_text &&
+                 s->g_state && s->g_own_rows && s->losses6, "loss_shard: null pointer");
+    TEAM_REQUIRE(!s->num_evo || (s->state_ids && s->evo && s->evo_mask), "loss_shard: null evolution pointer");
+    for (int p = 0; p < P - 1; ++p) {
+        if (phase == p) TEAM_REQUIRE(s->send[p] && (reinterpret_cast<uintptr_t>(s->send[p]) & 15) == 0, "loss_shard: send[%d] null or not 16-byte aligned", p);
+        if (phase > p) TEAM_REQUIRE(s->gathered[p] && (reinterpret_cast<uintptr_t>(s->gathered[p]) & 15) == 0, "loss_shard: gathered[%d] null or not 16-byte aligned", p);
+    }
+    shard_plan(s->mode, s->batch, s->world, s->num_evo, s->workspace, &w);
+    if (s->workspace == nullptr || s->workspace_bytes < w.total) {
+        set_error("loss_shard: workspace %zu < %zu bytes", s->workspace_bytes, w.total);
+        return TEAM_EWORKSPACE;
+    }
+    TEAM_REQUIRE((reinterpret_cast<uintptr_t>(s->workspace) & 255) == 0, "loss_shard: workspace must be 256-byte aligned");
+    shard_xplan(s->mode, s->batch, s->num_evo, &x);
+    return TEAM_OK;
+}
+
+}  // namespace team
+
+extern "C" int team_loss_shard_phases(int32_t num_evo) { return num_evo > 0 ? 4 : 3; }
+
+extern "C" size_t team_loss_shard_workspace_bytes(int32_t mode, int64_t batch, int32_t world, int32_t num_evo) {
+    if ((mode != TEAM_MODE_F32 && mode != TEAM_MODE_BF16) || batch < 1 || batch > LOSS_MAX_BATCH || world < 1 ||
+        world > SHARD_MAX_WORLD || batch * world < 2 || batch * world > SHARD_MAX_GLOBAL || num_evo < 0 || num_evo > 4096)
+        return 0;
+    ShardWS w;
+    shard_plan(mode, batch, world, num_evo, nullptr, &w);
+    return w.total;
+}
+
+extern "C" size_t team_loss_shard_xchg_bytes(int32_t mode, int64_t batch, int32_t num_evo, int32_t exchange) {
+    if ((mode != TEAM_MODE_F32 && mode != TEAM_MODE_BF16) || batch < 1 || batch > LOSS_MAX_BATCH || num_evo < 0 ||
+        num_evo > 4096 || exchange < 0 || exchange > 2)
+        return 0;
+    ShardX x;
+    shard_xplan(mode, batch, num_evo, &x);
+    return x.bytes[exchange];
+}
+
+extern "C" int team_loss_shard_run(int32_t phase, const team_loss_shard* s, void* stream) {
+    ShardWS w;
+    ShardX x;
+    int rc = shard_check(phase, s, w, x);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int mode = s->mode, B = (int)s->batch, W = s->world, Bg = B * W, r0 = s->rank * B, ld = (int)w.S[0].ld;
+    const bool bf = mode == TEAM_MODE_BF16, evo = s->num_evo > 0;
+    const int keys = s->num_evo * EVO_NS;
+    const float inv_tau = 1.0f / s->temperature;
+    const int64_t rld = shard_row_ld(mode);
+    // the gathered rows as GEMM operands: X_g (normalised image rows), I_g, T_g (own rows), [Bg][rld]
+    auto rows = [&](int k) {
+        char* p = const_cast<char*>(reinterpret_cast<const char*>(s->gathered[0])) + (size_t)k * D * shard_elem(mode);
+        return bf ? Mat{nullptr, reinterpret_cast<__nv_bfloat16*>(p), rld} : Mat{reinterpret_cast<float*>(p), nullptr, rld};
+    };
+    const int64_t slice1 = (int64_t)(x.bytes[1] / 4), slice2 = (int64_t)(x.bytes[2] / 4);
+    const float* g1 = reinterpret_cast<const float*>(s->gathered[1]);
+    if (phase == 0) {
+        TEAM_LAUNCH(loss_normalize_kernel, (3 * B + 7) / 8, 256, 0, st, s->batch, s->image, s->text, s->state, w.X[0], w.X[1], w.X[2],
+                    (__nv_bfloat16*)nullptr, (__nv_bfloat16*)nullptr, (__nv_bfloat16*)nullptr, w.inv[0], w.inv[1], w.inv[2], 3, 1);
+        TEAM_LAUNCH(shard_pack_rows_kernel, (3 * B + 7) / 8, 256, 0, st, B, (const float*)w.X[0], s->own_rows, s->labels, bf ? 1 : 0, rld, s->send[0]);
+    } else if (phase == 1) {
+        TEAM_LAUNCH(shard_labels_kernel, (Bg + 255) / 256, 256, 0, st, Bg, s->gathered[0], rld * shard_elem(mode),
+                    (int64_t)3 * D * shard_elem(mode), w.labels_g);
+        const Mat Xg = rows(0), Ig = rows(1), Tg = rows(2);
+        Wave wv;
+        seg(wv.add(B, Bg, 0.f, w.S[0]), false, sub(Xg, r0, 0), false, Xg, D);        // X_loc X_g^T
+        seg(wv.add(B, Bg, 0.f, w.S[1]), false, sub(Ig, r0, 0), false, Tg, D);        // I_loc T_g^T: rows of L
+        seg(wv.add(B, Bg, 0.f, w.S[2]), false, sub(Tg, r0, 0), false, Ig, D);        // T_loc I_g^T: rows of L^T
+        if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
+        float* o = reinterpret_cast<float*>(s->send[1]);
+        float* sc = o + x.x1_scal;
+        TEAM_CUDA_CHECK(cudaMemsetAsync(sc, 0, 8 * sizeof(float), st));     // slots no fold of this configuration writes stay 0
+        TEAM_LAUNCH(unicl_cat_stats_kernel, (B + 7) / 8, 256, 0, st, B, Bg, r0, ld, (const float*)w.S[0].f, (const int64_t*)w.labels_g, inv_tau,
+                    o + 2 * B, o + 3 * B, o + 4 * B, w.rloss + 2 * B, o + 5 * B);
+        TEAM_LAUNCH(clip_stats_kernel, (2 * B + 7) / 8, 256, 0, st, B, Bg, r0, ld, (const float*)w.S[1].f, (const float*)w.S[2].f, s->logit_scale, o, w.rloss);
+        TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, B, (const float*)(o + 5 * B), (const float*)(w.rloss + 2 * B), sc, 0, 0.f, (const float*)nullptr, (float*)nullptr);
+        TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, 2 * B, (const float*)w.rloss, (const float*)nullptr, sc + 2, 0, 0.f, (const float*)nullptr, (float*)nullptr);
+        TEAM_LAUNCH(ce_total_kernel, 1, 1024, 0, st, B, (int)s->num_classes, s->logits, s->labels, 0.f, 0.f, (float*)nullptr, sc + 4);
+        if (!evo) {       // the instance term is per sample: its value goes into this exchange, its gradient waits for dcat
+            TEAM_LAUNCH(unicl_instance_kernel, (B + 7) / 8, 256, 0, st, B, (const float*)w.X[0], (const float*)w.X[1], (const float*)w.X[2],
+                        (const float*)w.inv[0], (const float*)w.inv[1], (const float*)w.inv[2], (const float*)nullptr, inv_tau, 0.f,
+                        (float*)nullptr, (float*)nullptr, (float*)nullptr, w.rinst, (float*)nullptr);
+            TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, B, (const float*)w.rinst, (const float*)nullptr, sc + 5, 0, 0.f, (const float*)nullptr, (float*)nullptr);
+        } else {          // local (class, state) keyed sums and counts of the normalised state rows
+            TEAM_LAUNCH(evo_keysum_kernel, keys, 128, (size_t)((B + 31) / 32) * sizeof(unsigned int), st, B, (const float*)w.X[2], (const unsigned char*)nullptr,
+                        s->labels, s->state_ids, s->num_evo, s->evo_mask, o + x.x1_ss, reinterpret_cast<int*>(o + x.x1_cnt));
+        }
+    } else if (phase == 2) {
+        TEAM_LAUNCH(shard_cols_kernel, (6 * Bg + 255) / 256, 256, 0, st, B, Bg, 6, g1, slice1, w.cols);
+        TEAM_LAUNCH(shard_losses_kernel, 1, 32, 0, st, W, g1 + x.x1_scal, slice1, (const float*)nullptr, (int64_t)0, (int64_t)Bg,
+                    s->w_clip, s->w_unicl, w.scal, evo ? (float*)nullptr : s->losses6);
+        if (evo) {
+            TEAM_LAUNCH(shard_sum_kernel<float>, (keys * D + 255) / 256, 256, 0, st, W, (int64_t)keys * D, g1 + x.x1_ss, slice1, w.SS);
+            TEAM_LAUNCH(shard_sum_kernel<int>, (keys + 255) / 256, 256, 0, st, W, (int64_t)keys, reinterpret_cast<const int*>(g1 + x.x1_cnt), slice1, w.cnt);
+            TEAM_LAUNCH(evo_fwd_kernel, (B + 7) / 8, 256, 0, st, B, (const float*)w.X[2], s->labels, s->state_ids, s->num_evo, s->evo, s->evo_mask,
+                        (const float*)w.SS, (const int*)w.cnt, w.Xe, w.Mh, w.sc, w.rowmask);
+        }
+        const float* c = w.cols;     // [0] lse i2t, [1] lse t2i, [2] max, [3] pos, [4] all, [5] valid; each [Bg]
+        TEAM_LAUNCH(unicl_cat_grad_kernel, (B + 7) / 8, 256, 0, st, B, Bg, r0, ld, (const float*)w.S[0].f, (const int64_t*)w.labels_g, inv_tau,
+                    0.5f * s->w_unicl, c + 2 * Bg + r0, c + 3 * Bg + r0, c + 4 * Bg + r0, c + 5 * Bg + r0, c + 2 * Bg, c + 3 * Bg, c + 4 * Bg,
+                    c + 5 * Bg, (const float*)w.scal, w.G[0].f, w.G[0].h, w.G[3].f, w.G[3].h);
+        const float kc = s->logit_scale * s->w_clip / (2.0f * (float)Bg);
+        TEAM_LAUNCH(clip_grad_kernel, (B + 7) / 8, 256, 0, st, B, Bg, r0, ld, (const float*)w.S[1].f, s->logit_scale, kc, c + r0, c + Bg, w.G[1].f, w.G[1].h);
+        TEAM_LAUNCH(clip_grad_kernel, (B + 7) / 8, 256, 0, st, B, Bg, r0, ld, (const float*)w.S[2].f, s->logit_scale, kc, c + Bg + r0, c, w.G[2].f, w.G[2].h);
+        const Mat Xg = rows(0), Ig = rows(1), Tg = rows(2);
+        Wave wv;
+        seg(seg(wv.add(B, D, 0.f, Mat{w.dcat, nullptr, D}), false, w.G[0], true, Xg, Bg), false, w.G[3], true, Xg, Bg);   // dcat = G X_g + H X_g
+        seg(wv.add(B, D, 0.f, Mat{s->g_own_rows, nullptr, D}), false, w.G[1], true, Tg, Bg);             // dI = G T_g
+        seg(wv.add(B, D, 0.f, Mat{s->g_own_rows + (size_t)B * D, nullptr, D}), false, w.G[2], true, Ig, Bg);   // dT = (G^T)_loc I_g
+        if ((rc = run_wave(st, mode, wv, w.gemm_ws, w.gemm_ws_bytes))) return rc;
+        TEAM_LAUNCH(unicl_instance_kernel, (B + 7) / 8, 256, 0, st, B, (const float*)w.X[0], (const float*)w.X[1], (const float*)(evo ? w.Xe : w.X[2]),
+                    (const float*)w.inv[0], (const float*)w.inv[1], (const float*)w.inv[2], (const float*)w.dcat, inv_tau,
+                    s->w_unicl / (3.0f * (float)Bg), s->g_image, s->g_text, s->g_state, evo ? w.rinst : (float*)nullptr, evo ? w.dXe : (float*)nullptr);
+        if (evo) {
+            float* o = reinterpret_cast<float*>(s->send[2]);
+            TEAM_CUDA_CHECK(cudaMemsetAsync(o + x.x2_scal, 0, 8 * sizeof(float), st));
+            TEAM_LAUNCH(evo_bwd1_kernel, (B + 7) / 8, 256, 0, st, B, (const float*)w.Xe, (const float*)w.Mh, (const float*)w.sc, w.dXe, w.dMix);
+            TEAM_LAUNCH(evo_keysum_kernel, keys, 128, (size_t)((B + 31) / 32) * sizeof(unsigned int), st, B, (const float*)w.dMix, (const unsigned char*)w.rowmask,
+                        s->labels, s->state_ids, s->num_evo, s->evo_mask, o, (int*)nullptr);
+            TEAM_LAUNCH(loss_fold2_kernel, 1, 1024, 0, st, B, (const float*)w.rinst, (const float*)nullptr, o + x.x2_scal + 5, 0, 0.f, (const float*)nullptr, (float*)nullptr);
+        }
+    } else {              // phase 3: evolution features only
+        const float* g2 = reinterpret_cast<const float*>(s->gathered[2]);
+        TEAM_LAUNCH(shard_sum_kernel<float>, (keys * D + 255) / 256, 256, 0, st, W, (int64_t)keys * D, g2, slice2, w.DM);
+        TEAM_LAUNCH(shard_losses_kernel, 1, 32, 0, st, W, g1 + x.x1_scal, slice1, g2 + x.x2_scal, slice2, (int64_t)Bg,
+                    s->w_clip, s->w_unicl, w.scal, s->losses6);
+        TEAM_LAUNCH(evo_bwd2_kernel, (B + 7) / 8, 256, 0, st, B, (const float*)w.X[2], (const float*)w.inv[2], s->labels, s->state_ids,
+                    (const float*)w.sc, (const float*)w.DM, (const int*)w.cnt, (const float*)w.dXe, s->g_state);
+    }
     return TEAM_OK;
 }

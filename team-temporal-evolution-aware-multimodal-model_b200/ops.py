@@ -248,6 +248,85 @@ def ce_total(logits: torch.Tensor, labels: torch.Tensor, losses6: torch.Tensor, 
     return losses6
 
 
+class ShardedLosses:
+    """ClipLoss, unicl_loss (with evolution features) and the ce value over a GLOBAL batch sharded across ``world`` ranks
+    of ``batch`` samples each (``team_loss_shard_*``): the same ``losses6`` on every rank, and this rank's rows of the
+    gradient of ``total = ce + w_clip * clip + w_unicl * unicl`` (``g_image`` / ``g_text`` / ``g_state``: the head's
+    feature cotangents; ``g_own``: the ClipLoss cotangent of the own rows, ``team_head_grads.g_own_rows``).
+
+    The computation is ``phases`` calls of ``run(p)``.  Between ``run(p)`` and ``run(p + 1)`` the caller all-gathers
+    every rank's ``send[p]`` into ``gathered[p]`` in rank order (``parallel.gather_slices``, or a concatenation when the
+    ranks live in one process).  The buffers, the workspace and the bound inputs are reused by every step."""
+
+    def __init__(self, rank: int, world: int, batch: int, num_classes: int, *, evolution_features=None,
+                 mode: int = capi.MODE_F32, device=None):
+        capi.require_device()
+        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        L = capi.lib()
+        self.evo = None
+        if evolution_features is not None and len(evolution_features) > 0:
+            self.evo = evolution_features if isinstance(evolution_features, tuple) else pack_evolution_features(evolution_features, dev)
+        ne = self.evo[0].shape[0] if self.evo is not None else 0
+        nbytes = L.team_loss_shard_workspace_bytes(mode, batch, world, ne)
+        if nbytes == 0:
+            raise ValueError(f"ShardedLosses: batch {batch} x world {world} (num_evo {ne}) out of range")
+        self.rank, self.world, self.B, self.mode, self.dev = rank, world, batch, mode, dev
+        self.phases = L.team_loss_shard_phases(ne)
+        u8 = lambda n: torch.empty((n,), dtype=torch.uint8, device=dev)
+        self.workspace = u8(nbytes)
+        sizes = [L.team_loss_shard_xchg_bytes(mode, batch, ne, k) for k in range(self.phases - 1)]
+        self.send = [u8(n) for n in sizes]
+        self.gathered = [u8(world * n) for n in sizes]
+        f = lambda *s: torch.zeros(s, dtype=torch.float32, device=dev)
+        self.g_image, self.g_text, self.g_state = f(batch, capi.D), f(batch, capi.D), f(batch, capi.D)
+        self.g_own = f(2, batch, capi.D)
+        self.losses6 = f(6)
+        s = capi.LossShard()
+        s.mode, s.rank, s.world, s.num_evo, s.batch, s.num_classes = mode, rank, world, ne, batch, num_classes
+        if self.evo is not None:
+            s.evo, s.evo_mask = self.evo[0].data_ptr(), self.evo[1].data_ptr()
+        for k in range(self.phases - 1):
+            s.send[k], s.gathered[k] = self.send[k].data_ptr(), self.gathered[k].data_ptr()
+        s.g_image, s.g_text, s.g_state = self.g_image.data_ptr(), self.g_text.data_ptr(), self.g_state.data_ptr()
+        s.g_own_rows, s.losses6 = self.g_own.data_ptr(), self.losses6.data_ptr()
+        s.workspace, s.workspace_bytes = self.workspace.data_ptr(), nbytes
+        self.struct, self._bound = s, []
+
+    def bind(self, image, text, state, own_rows, logits, labels, state_ids=None, *, temperature: float = 0.07, epoch=None,
+             max_epoch=None, logit_scale: float, w_clip: float = 1.0, w_unicl: float = 0.3):
+        """The rank's inputs (kept referenced; later ``run`` calls read them in place): head outputs ``image`` / ``text`` /
+        ``state`` [B,512] fp32, ``own_rows`` [2B,512] fp32 (normalised image rows, then text rows), ``logits`` [B,C] fp32,
+        ``labels`` / ``state_ids`` [B] int64.  ``temperature`` is made dynamic by ``epoch`` / ``max_epoch`` as in
+        ``unicl_loss``."""
+        B, D = self.B, capi.D
+        want = [(image, (B, D), torch.float32), (text, (B, D), torch.float32), (state, (B, D), torch.float32),
+                (own_rows, (2 * B, D), torch.float32), (labels, (B,), torch.int64)]
+        if self.evo is not None:
+            if state_ids is None:
+                raise ValueError("ShardedLosses: evolution_features needs state_ids")
+            want.append((state_ids, (B,), torch.int64))
+        for t, shape, dt in want:
+            if t.shape != shape or t.dtype != dt or not t.is_contiguous() or t.device != self.dev:
+                raise ValueError(f"ShardedLosses: expected a contiguous {dt} {shape} tensor on {self.dev}, got {t.dtype} {tuple(t.shape)}")
+        if (logits.dim() != 2 or logits.shape[0] != B or logits.dtype != torch.float32 or not logits.is_contiguous()
+                or logits.device != self.dev):
+            raise ValueError(f"ShardedLosses: logits must be a contiguous fp32 [{B},C] tensor on {self.dev}")
+        s = self.struct
+        s.image, s.text, s.state, s.own_rows = image.data_ptr(), text.data_ptr(), state.data_ptr(), own_rows.data_ptr()
+        s.logits, s.labels, s.num_classes = logits.data_ptr(), labels.data_ptr(), logits.shape[1]
+        s.state_ids = state_ids.data_ptr() if state_ids is not None else None
+        s.temperature = dynamic_temperature(temperature, epoch, max_epoch)
+        s.logit_scale, s.w_clip, s.w_unicl = float(logit_scale), float(w_clip), float(w_unicl)
+        self._bound = [image, text, state, own_rows, logits, labels, state_ids]
+
+    def run(self, phase: int):
+        """Phase ``phase`` on the current stream (capturable)."""
+        import ctypes as C
+        if not self._bound:
+            raise RuntimeError("ShardedLosses.run before bind")
+        capi.check(capi.lib().team_loss_shard_run(phase, C.byref(self.struct), _stream_ptr()), "team_loss_shard_run")
+
+
 class FusedAdamW:
     """torch.optim.AdamW(params, lr, betas, eps, weight_decay).step() (models/proof.py:361, :445) as ONE kernel over
     all tensors (``team_adamw_step``).  ``step(grads)`` takes the gradients as a list aligned with ``params`` (e.g.

@@ -76,6 +76,16 @@ def allreduce_gradients(flat_grads: torch.Tensor, group=None, average: bool = Fa
     return work
 
 
+def gather_slices(send: torch.Tensor, gathered: torch.Tensor, group=None):
+    """One exchange of ``ops.ShardedLosses``: every rank's ``send`` slice into ``gathered`` in rank order
+    (``all_gather_into_tensor``; the collective does no arithmetic, the next loss phase folds in rank order)."""
+    _, ws = world(group)
+    if ws == 1:
+        gathered.copy_(send)
+        return
+    dist.all_gather_into_tensor(gathered, send, group=group)
+
+
 def allreduce_batch_means(text_sum: torch.Tensor, proto_sum: torch.Tensor, local_rows: int, group=None):
     """PROOF ``Proof_Net.forward`` returns batch MEANS of the text / prototype rows
     (utils/inc_net.py:458-459); under data parallelism the exact single-GPU value needs the sums
