@@ -445,6 +445,19 @@ int team_peer_allreduce_f32(void* const* bufs, void* const* flags, void* multica
  * synchronises `stream` and returns this rank's status word: 0 = all exchanges completed, otherwise
  * 1 + (phase << 8) + (peer << 16) of the first wait that timed out.  own_flags = flags[rank]. */
 int team_peer_allreduce_status(const void* own_flags, void* stream, uint32_t* status);
+/* All-gather of one slice of slice_bytes bytes per rank over NVLink peer memory: the exchanges between the phases of
+ * team_loss_shard_run inside a captured training step.  bufs[r] / flags[r] (r < world, HOST arrays of device pointers)
+ * are every rank's gathered buffer (world * slice_bytes bytes, rank-major) and flag array as mapped on THIS device
+ * (symmetric memory); flags are team_peer_allreduce_flag_bytes() bytes each, zeroed once before the first call, and
+ * must not be the arrays of an all-reduce.  Rank r's own slice must already be in slot r of bufs[rank] (bytes
+ * [rank * slice_bytes, (rank + 1) * slice_bytes)): the kernel stores it into slot r of every peer's buffer and never
+ * copies locally.  One kernel, bit-exact (no arithmetic), safe to call again on the same buffers (the kernel waits
+ * until every rank has finished reading before any slot is overwritten); every rank must make the matching call.
+ * slice_bytes % 16 == 0 (every team_loss_shard_xchg_bytes size is), world <= 8; world == 1 is a no-op.
+ * multicast: NVLS multicast mapping of the same buffers (NULL = none): each rank then sends its slice once and the
+ * switch replicates it.  Health: team_peer_allreduce_status on flags[rank]. */
+int team_peer_allgather(void* const* bufs, void* const* flags, void* multicast, int32_t rank, int32_t world,
+                        int64_t slice_bytes, void* stream);
 
 /* ------------------------------------------------------------------ temporal GCN + state distances
  * Replaces: TemporalStateGCN.forward / TemporalGCNBlock.forward   models/dynamic_modal_graph.py:239-337

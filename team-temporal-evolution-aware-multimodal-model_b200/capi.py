@@ -157,6 +157,8 @@ def _declare(lib):
         lib.team_peer_allreduce_f32.argtypes = [C.POINTER(vp), C.POINTER(vp), vp, i32, i32, i64, vp]
         lib.team_peer_allreduce_status.restype = i32
         lib.team_peer_allreduce_status.argtypes = [vp, vp, C.POINTER(C.c_uint32)]
+        lib.team_peer_allgather.restype = i32
+        lib.team_peer_allgather.argtypes = [C.POINTER(vp), C.POINTER(vp), vp, i32, i32, i64, vp]
         lib.team_adamw_step.restype = i32
         lib.team_adamw_step.argtypes = [i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(i64),
                                         C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, i64, vp]

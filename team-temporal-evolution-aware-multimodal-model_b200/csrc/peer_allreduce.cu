@@ -11,6 +11,7 @@
 // Flags carry a monotonically increasing epoch kept in the rank's own flag array, so nothing is ever reset and the
 // launch can sit inside a replayed CUDA graph.  Block b of every rank works on the same float4 indices, so the
 // barriers are per block (no grid-wide sync); the grid is small enough to be co-resident.
+// The all-gather of the data-parallel losses (team_peer_allgather, below) uses the same barriers and flag layout.
 #include <stdlib.h>
 #include "common.cuh"
 
@@ -152,6 +153,49 @@ peer_allreduce_f32_kernel(const __grid_constant__ ArArgs a) {
     ar_barrier(a, 1, epoch, true);
 }
 
+// All-gather of one slice per rank (the exchanges between the phases of team_loss_shard_run): buf[r] is rank r's
+// gathered buffer, world slices of n4 16-byte units in rank order, and this rank's slice is already in slot `rank` of
+// its own buffer (the loss phase wrote it there).  No arithmetic, so every rank ends with the same bytes.
+//   barrier A  "my slice is written and I no longer read my gathered buffer": earlier kernels of this rank did both
+//              (complete when this kernel runs), so the peers may now overwrite the other slots.  This makes reusing
+//              the buffers from step to step safe whatever runs between two calls.
+//   store      the slice into slot `rank` of every peer's buffer [with a multicast mapping: ONE multimem.st of the
+//              slice, which the switch replicates into every rank's buffer]
+//   barrier B  (release) "my slice is in your buffer"; the readers are later kernels
+__global__ void __launch_bounds__(AR_THREADS)
+peer_allgather_kernel(const __grid_constant__ ArArgs a) {
+    pdl_trigger();
+    pdl_wait();
+    __shared__ uint32_t s_epoch;
+    if (threadIdx.x == 0) {
+        uint32_t* e = a.flag[a.rank] + blockIdx.x;
+        s_epoch = *e + 1;
+        *e = s_epoch;
+    }
+    __syncthreads();
+    const uint32_t epoch = s_epoch;
+    ar_barrier(a, 0, epoch, false);
+    const int W = a.world, me = a.rank;
+    const long long n4 = a.n4, slot = n4 * me;
+    const float4* src = reinterpret_cast<const float4*>(a.buf[me]) + slot;
+    const long long stride = (long long)gridDim.x * AR_THREADS;
+    if (a.mc != nullptr) {
+        float4* mc = reinterpret_cast<float4*>(a.mc) + slot;
+        for (long long i = (long long)blockIdx.x * AR_THREADS + threadIdx.x; i < n4; i += stride) {
+            const float4 v = src[i];
+            asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1,%2,%3,%4};"
+                         ::"l"(mc + i), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+        }
+    } else
+    for (long long i = (long long)blockIdx.x * AR_THREADS + threadIdx.x; i < n4; i += stride) {
+        const float4 v = src[i];
+#pragma unroll
+        for (int r = 0; r < AR_MAX_RANKS; ++r)
+            if (r < W && r != me) (reinterpret_cast<float4*>(a.buf[r]) + slot)[i] = v;
+    }
+    ar_barrier(a, 1, epoch, true);
+}
+
 // Blocks per call: about two float4 per thread of a rank's slice, between 8 and AR_BLOCKS.  A small bucket that is
 // exchanged UNDER compute kernels should not park 64 spinning blocks on the SMs those kernels need; every rank
 // derives the same grid from the same n, and each block keeps its own epoch, so grids may differ between calls.
@@ -230,5 +274,28 @@ extern "C" int team_peer_allreduce_f32(void* const* bufs, void* const* flags, vo
     a.status = reinterpret_cast<uint32_t*>(flags[rank]) + (size_t)2 * AR_FLAG_WORDS;
     a.timeout_ns = ar_timeout_ns();
     TEAM_LAUNCH(peer_allreduce_f32_kernel, ar_grid(a.n4, a.world), AR_THREADS, 0, (cudaStream_t)stream, a);
+    return TEAM_OK;
+}
+
+extern "C" int team_peer_allgather(void* const* bufs, void* const* flags, void* multicast, int32_t rank, int32_t world,
+                                   int64_t slice_bytes, void* stream) {
+    TEAM_REQUIRE(bufs != nullptr && flags != nullptr, "peer_allgather: null pointer table");
+    TEAM_REQUIRE(world >= 1 && world <= AR_MAX_RANKS && rank >= 0 && rank < world, "peer_allgather: rank %d / world %d", rank, world);
+    TEAM_REQUIRE(slice_bytes >= 0 && slice_bytes % 16 == 0, "peer_allgather: slice of %lld bytes must be a multiple of 16", (long long)slice_bytes);
+    if (slice_bytes == 0 || world == 1) return TEAM_OK;
+    ArArgs a;
+    memset(&a, 0, sizeof(a));
+    for (int r = 0; r < world; ++r) {
+        TEAM_REQUIRE(bufs[r] != nullptr && flags[r] != nullptr && (reinterpret_cast<uintptr_t>(bufs[r]) & 15) == 0, "peer_allgather: bad pointer of rank %d", r);
+        a.buf[r] = reinterpret_cast<float*>(bufs[r]);
+        a.flag[r] = reinterpret_cast<uint32_t*>(flags[r]);
+    }
+    TEAM_REQUIRE((reinterpret_cast<uintptr_t>(multicast) & 15) == 0, "peer_allgather: misaligned multicast mapping");
+    a.mc = reinterpret_cast<float*>(multicast);
+    a.rank = rank; a.world = world; a.n4 = slice_bytes / 16;
+    a.status = reinterpret_cast<uint32_t*>(flags[rank]) + (size_t)2 * AR_FLAG_WORDS;
+    a.timeout_ns = ar_timeout_ns();
+    // the grid is sized by the slice each rank sends (every rank derives the same one from the same slice_bytes)
+    TEAM_LAUNCH(peer_allgather_kernel, ar_grid(a.n4, 1), AR_THREADS, 0, (cudaStream_t)stream, a);
     return TEAM_OK;
 }

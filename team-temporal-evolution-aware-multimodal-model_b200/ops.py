@@ -256,10 +256,14 @@ class ShardedLosses:
 
     The computation is ``phases`` calls of ``run(p)``.  Between ``run(p)`` and ``run(p + 1)`` the caller all-gathers
     every rank's ``send[p]`` into ``gathered[p]`` in rank order (``parallel.gather_slices``, or a concatenation when the
-    ranks live in one process).  The buffers, the workspace and the bound inputs are reused by every step."""
+    ranks live in one process).  The buffers, the workspace and the bound inputs are reused by every step.
+
+    ``gathered``: optional caller-owned exchange buffers, one contiguous uint8 tensor of ``world *
+    xchg_bytes(p)`` bytes per exchange (``parallel.PeerAllGather.gathered``); ``send[p]`` is then the rank's slot of
+    ``gathered[p]``, so the phases write their slices where the peer all-gather expects them."""
 
     def __init__(self, rank: int, world: int, batch: int, num_classes: int, *, evolution_features=None,
-                 mode: int = capi.MODE_F32, device=None):
+                 mode: int = capi.MODE_F32, device=None, gathered=None):
         capi.require_device()
         dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         L = capi.lib()
@@ -275,8 +279,19 @@ class ShardedLosses:
         u8 = lambda n: torch.empty((n,), dtype=torch.uint8, device=dev)
         self.workspace = u8(nbytes)
         sizes = [L.team_loss_shard_xchg_bytes(mode, batch, ne, k) for k in range(self.phases - 1)]
-        self.send = [u8(n) for n in sizes]
-        self.gathered = [u8(world * n) for n in sizes]
+        self.xchg_bytes = sizes
+        if gathered is None:
+            self.send = [u8(n) for n in sizes]
+            self.gathered = [u8(world * n) for n in sizes]
+        else:
+            gathered = list(gathered)
+            if len(gathered) != len(sizes) or any(
+                    g.dtype != torch.uint8 or g.numel() != world * n or not g.is_contiguous() or g.device != dev
+                    or g.data_ptr() % 16 for g, n in zip(gathered, sizes)):
+                raise ValueError(f"ShardedLosses: gathered must be {len(sizes)} contiguous 16-byte aligned uint8 tensors "
+                                 f"on {dev} of {[world * n for n in sizes]} bytes")
+            self.gathered = gathered
+            self.send = [g[rank * n:(rank + 1) * n] for g, n in zip(gathered, sizes)]
         f = lambda *s: torch.zeros(s, dtype=torch.float32, device=dev)
         self.g_image, self.g_text, self.g_state = f(batch, capi.D), f(batch, capi.D), f(batch, capi.D)
         self.g_own = f(2, batch, capi.D)

@@ -100,7 +100,30 @@ def allreduce_batch_means(text_sum: torch.Tensor, proto_sum: torch.Tensor, local
     return text_sum / g, proto_sum / g
 
 
-class PeerAllReduce:
+class _PeerExchange:
+    """Health of a peer-memory exchange: ``_lib``, ``_hf`` (the rendezvoused flag array), ``rank`` and ``_what`` are set
+    by the subclass."""
+
+    def status(self, stream=None) -> int:
+        """Synchronises ``stream`` and returns this rank's exchange status: 0 = every exchange so far completed;
+        otherwise ``1 + (phase << 8) + (peer << 16)`` of the first wait that ran past the deadline
+        (``TEAM_PEER_TIMEOUT_S``, default 1800 s) - the buffer then does NOT hold the exchanged data."""
+        import ctypes as C
+        from . import capi
+        st = (stream or torch.cuda.current_stream()).cuda_stream
+        out = C.c_uint32(0)
+        capi.check(self._lib.team_peer_allreduce_status(int(self._hf.buffer_ptrs[self.rank]), st, C.byref(out)),
+                   "team_peer_allreduce_status")
+        return int(out.value)
+
+    def check(self, stream=None):
+        s = self.status(stream)
+        if s:
+            raise RuntimeError(f"{self._what} on rank {self.rank}: peer {(s >> 16) & 0xff} did not arrive at barrier "
+                               f"{(s >> 8) & 0xff} before the deadline (TEAM_PEER_TIMEOUT_S)")
+
+
+class PeerAllReduce(_PeerExchange):
     """In-place sum over the ranks of ONE fp32 buffer per GPU by a single kernel over NVLink peer memory
     (``team_peer_allreduce_f32``: two-shot, rank-ordered sum, graph-capturable) instead of an NCCL ring/tree,
     whose latency dominates at the size of the head's gradient buffer (7.4 MB).
@@ -108,6 +131,8 @@ class PeerAllReduce:
     ``buffer`` is allocated in torch symmetric memory and mapped by every rank; hand it to
     ``HeadStepRunner(grad_buffer=...)`` so the backward writes the gradients straight into it.  torch.distributed
     (NCCL) is only used for the rendezvous that exchanges the memory handles."""
+
+    _what = "peer all-reduce"
 
     def __init__(self, numel: int, device, group=None, multicast: bool = True):
         import ctypes as C
@@ -152,24 +177,6 @@ class PeerAllReduce:
         c.rank, c.world, c.n_total, c.split_at = self.rank, self.world, self.numel, int(split_at)
         return c
 
-    def status(self, stream=None) -> int:
-        """Synchronises ``stream`` and returns this rank's exchange status: 0 = every exchange so far completed;
-        otherwise ``1 + (phase << 8) + (peer << 16)`` of the first wait that ran past the deadline
-        (``TEAM_PEER_TIMEOUT_S``, default 1800 s) - the buffer is then NOT the sum over the ranks."""
-        import ctypes as C
-        from . import capi
-        st = (stream or torch.cuda.current_stream()).cuda_stream
-        out = C.c_uint32(0)
-        capi.check(self._lib.team_peer_allreduce_status(int(self._hf.buffer_ptrs[self.rank]), st, C.byref(out)),
-                   "team_peer_allreduce_status")
-        return int(out.value)
-
-    def check(self, stream=None):
-        s = self.status(stream)
-        if s:
-            raise RuntimeError(f"peer all-reduce on rank {self.rank}: peer {(s >> 16) & 0xff} did not arrive at barrier "
-                               f"{(s >> 8) & 0xff} before the deadline (TEAM_PEER_TIMEOUT_S)")
-
     def __call__(self, stream=None):
         """Enqueue the all-reduce of ``buffer`` on ``stream`` (default: the current stream); capturable."""
         from . import capi
@@ -177,3 +184,58 @@ class PeerAllReduce:
         capi.check(self._lib.team_peer_allreduce_f32(self._bufs, self._flgs, self.multicast_ptr or None, self.rank, self.world,
                                                         self.numel, st),
                    "team_peer_allreduce_f32")
+
+
+class PeerAllGather(_PeerExchange):
+    """All-gathers of fixed-size byte slices, one per rank in rank order, by a single kernel over NVLink peer memory
+    (``team_peer_allgather``: bit-exact, graph-capturable): the exchanges between the phases of ``ops.ShardedLosses``
+    inside a captured training step, where an eager NCCL call cannot sit.
+
+    ``slice_bytes[p]`` is the size of one rank's slice of exchange ``p`` (a multiple of 16).  ``gathered[p]`` (uint8,
+    ``world * slice_bytes[p]`` bytes, torch symmetric memory) is the rank's gathered buffer and ``send[p]`` its slot
+    ``rank`` of it: whatever the caller writes there is what every rank finds in slot ``rank`` after ``self(p)``.
+    Hand ``gathered`` to ``ops.ShardedLosses(gathered=...)`` so the loss phases write their slices in place.
+    torch.distributed (NCCL) is only used for the rendezvous that exchanges the memory handles."""
+
+    _what = "peer all-gather"
+
+    def __init__(self, slice_bytes, device, group=None, multicast: bool = True):
+        import ctypes as C
+        import torch.distributed._symmetric_memory as symm
+        from . import capi
+        if not (dist.is_available() and dist.is_initialized()):
+            raise RuntimeError("PeerAllGather needs an initialised process group")
+        self.group = group if group is not None else dist.group.WORLD
+        self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
+        if self.world > 8:
+            raise ValueError("PeerAllGather: one NVSwitch box (<= 8 ranks)")
+        self.slice_bytes = [int(n) for n in slice_bytes]
+        if any(n <= 0 or n % 16 for n in self.slice_bytes):
+            raise ValueError(f"PeerAllGather: slice sizes {self.slice_bytes} must be positive multiples of 16 bytes")
+        self._lib = capi.lib()
+        self.gathered = [symm.empty(self.world * n, dtype=torch.uint8, device=device) for n in self.slice_bytes]
+        self.send = [g[self.rank * n:(self.rank + 1) * n] for g, n in zip(self.gathered, self.slice_bytes)]
+        self._flags = symm.empty(self._lib.team_peer_allreduce_flag_bytes() // 4, dtype=torch.int32, device=device)
+        for g in self.gathered:
+            g.zero_()
+        self._flags.zero_()
+        self._hg = [symm.rendezvous(g, self.group) for g in self.gathered]
+        self._hf = symm.rendezvous(self._flags, self.group)
+        torch.cuda.synchronize(device)
+        dist.barrier(self.group)                     # every rank has zeroed its flags before anyone signals
+        vp8 = C.c_void_p * self.world
+        self._bufs = [vp8(*[int(p) for p in h.buffer_ptrs]) for h in self._hg]
+        self._flgs = vp8(*[int(p) for p in self._hf.buffer_ptrs])
+        # the all-reduce's policy: multicast from 4 ranks up, and only when every buffer of every rank has the mapping
+        mc = [int(getattr(h, "multicast_ptr", 0) or 0) if (multicast and self.world >= 4) else 0 for h in self._hg]
+        ok = torch.tensor([1 if all(mc) else 0], device=device)
+        dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=self.group)      # all ranks take the same path
+        self.multicast_ptrs = mc if int(ok.item()) else [0] * len(mc)
+
+    def __call__(self, p: int, stream=None):
+        """Enqueue exchange ``p`` on ``stream`` (default: the current stream); capturable.  ``send[p]`` must be final."""
+        from . import capi
+        st = (stream or torch.cuda.current_stream()).cuda_stream
+        capi.check(self._lib.team_peer_allgather(self._bufs[p], self._flgs, self.multicast_ptrs[p] or None, self.rank,
+                                                 self.world, self.slice_bytes[p], st),
+                   "team_peer_allgather")

@@ -10,6 +10,8 @@ launch of the step - 50-odd library kernels - is captured once per epoch (the le
 and unicl's dynamic temperature change per epoch, :111-116, :363) and replayed per batch.  The Adam step count lives
 on the device (`team_adamw_step_graph`).  Not captured (and not trained here): `convnet.logit_scale` - the captured
 ClipLoss launch bakes its value in; pass the current value when an epoch's graph is captured.
+`DataParallelTrainStep` is the same loop body on N GPUs of one box over a global batch (losses over the whole batch,
+gradient summed over the ranks inside the graph).
 """
 from __future__ import annotations
 
@@ -38,8 +40,7 @@ class TrainStep:
         dev = pack.flat[0].device
         self.dev = dev
         self.text_cls = text_cls.to(device=dev, dtype=torch.float32).contiguous()
-        self.runner = head.HeadStepRunner(pack, img_prototypes, batch, int(self.text_cls.shape[0]), mode,
-                                          dropout_p=dropout_p, seed=seed)
+        self.runner = self._make_runner(pack, img_prototypes, batch, int(self.text_cls.shape[0]), mode, dropout_p, seed)
         self.dropout_base = self.runner.offset
         gv = self.runner.grad_views
         P = pack.T * pack.ppt
@@ -73,6 +74,9 @@ class TrainStep:
         self._graphs: Dict[int, torch.cuda.CUDAGraph] = {}
         self._stream = torch.cuda.Stream(device=dev)
         self._side = torch.cuda.Stream(device=dev)
+
+    def _make_runner(self, pack, img_prototypes, batch, n_cls, mode, dropout_p, seed):
+        return head.HeadStepRunner(pack, img_prototypes, batch, n_cls, mode, dropout_p=dropout_p, seed=seed)
 
     def lr_at(self, epoch: int) -> float:
         """CosineAnnealingLR(T_max=tuned_epoch, eta_min=min_lr) stepped once per epoch (models/proof.py:363, :447)."""
@@ -144,3 +148,133 @@ class TrainStep:
             self._capture(epoch)
         self._graphs[epoch].replay()
         return self.losses
+
+
+class DataParallelTrainStep(TrainStep):
+    """``TrainStep`` over a GLOBAL batch of ``world * batch`` samples, one rank per GPU: every rank loads its own
+    ``batch`` samples (contiguous shards in rank order) and replays one CUDA graph per epoch holding
+
+        head forward -> loss phase 0 -> all-gather 0 -> phase 1 -> all-gather 1 -> ... -> last phase
+        -> head backward (its parameter gradients summed over the ranks inside it) -> AdamW step
+
+    The loss phases (``ops.ShardedLosses``) give every rank the same ``losses6`` and the gradient of the global-batch
+    total for its own rows, so the rank sum of the backwards is the gradient one GPU computes on the whole batch: it is
+    applied as is (no averaging), by every rank, and the parameters stay bit-identical across ranks without a
+    broadcast.  The all-gathers run on ``parallel.PeerAllGather`` and the gradient sum on ``parallel.PeerAllReduce``
+    (both peer-memory kernels, capturable); by default both are built from the process group (``group``).
+
+    Every exchange is a matching call on all ranks, and capturing an epoch's graph first runs the step once eagerly:
+    all ranks must call ``step(epoch)`` the same number of times with the same epochs in the same order.
+
+    The step is also written as stages (``bind``, ``stage_forward``, ``stage_loss``, ``stage_exchange``,
+    ``stage_backward``, ``stage_update``).  With explicit ``rank`` / ``world`` and ``build_exchanges=False`` no exchange
+    object is built, and a caller that holds all ranks in one process drives the stages itself: it concatenates the
+    ranks' ``sl.send[p]`` into every ``sl.gathered[p]`` and sums the ranks' ``runner.flat_grads`` in rank order.
+
+    Not supported: ``dropout_p`` > 0 (the masks are keyed by the LOCAL sample index, so every rank would draw rank 0's
+    masks), more than 8 ranks, and batches beyond the ``team_loss_shard`` limits (batch <= 16384, world * batch <=
+    65536)."""
+
+    def __init__(self, params: Dict[str, torch.Tensor], img_prototypes: torch.Tensor, batch: int, text_cls: torch.Tensor,
+                 mode: int = head.MODE_BF16, init_lr: float = 0.004, min_lr: float = 1e-8, weight_decay: float = 0.05,
+                 tuned_epoch: int = 20, logit_scale: float = math.exp(2.6592600369327783),
+                 evolution_features=None, dropout_p: float = 0.0, seed: Optional[int] = None, *,
+                 rank: Optional[int] = None, world: Optional[int] = None, group=None, gather=None, peer=None,
+                 build_exchanges: bool = True):
+        from . import parallel
+        r0, w0 = parallel.world(group)
+        rank = r0 if rank is None else int(rank)
+        world = w0 if world is None else int(world)
+        if dropout_p != 0.0:
+            raise ValueError("DataParallelTrainStep: dropout_p > 0 is not supported (the dropout masks are keyed by the "
+                             "local sample index, so every rank would draw rank 0's masks)")
+        if not 1 <= world <= 8 or not 0 <= rank < world:
+            raise ValueError(f"DataParallelTrainStep: rank {rank} / world {world} (one NVSwitch box: at most 8 ranks)")
+        if not 1 <= batch <= 16384 or not 2 <= world * batch <= 65536:
+            raise ValueError(f"DataParallelTrainStep: {batch} samples per rank x {world} ranks out of range "
+                             "(batch <= 16384, 2 <= world * batch <= 65536)")
+        for obj in (gather, peer):
+            if obj is not None and (obj.rank, obj.world) != (rank, world):
+                raise ValueError(f"DataParallelTrainStep: exchange of rank {obj.rank} / world {obj.world} for rank {rank} / world {world}")
+        self.rank, self.world, self.group = rank, world, group
+        self._build = build_exchanges and world > 1
+        self.peer = peer
+        super().__init__(params, img_prototypes, batch, text_cls, mode=mode, init_lr=init_lr, min_lr=min_lr,
+                         weight_decay=weight_decay, tuned_epoch=tuned_epoch, logit_scale=logit_scale,
+                         evolution_features=evolution_features, seed=seed)
+        L = capi.lib()
+        ne = self.evo[0].shape[0] if self.evo is not None else 0
+        sizes = [L.team_loss_shard_xchg_bytes(mode, batch, ne, k) for k in range(L.team_loss_shard_phases(ne) - 1)]
+        if gather is None and self._build:
+            gather = parallel.PeerAllGather(sizes, self.dev, group)
+        self.gather = gather
+        # without an all-gather object the step still owns rank-major gathered buffers, so send[p] is the rank's slot:
+        # at world 1 the exchange is then nothing at all
+        gathered = gather.gathered if gather is not None else [torch.empty((world * n,), dtype=torch.uint8, device=self.dev)
+                                                               for n in sizes]
+        self.sl = ops.ShardedLosses(rank, world, batch, int(self.text_cls.shape[0]), evolution_features=self.evo, mode=mode,
+                                    device=self.dev, gathered=gathered)
+        self.losses6 = self.sl.losses6          # total, ce, clip, unicl total, unicl instance, unicl category
+        self.losses = self.losses6[:5]
+        self.g_own = self.sl.g_own
+
+    def _make_runner(self, pack, img_prototypes, batch, n_cls, mode, dropout_p, seed):
+        from . import parallel
+        if self.peer is None and self._build:
+            self.peer = parallel.PeerAllReduce(head.HeadStepRunner.grad_numel(pack), pack.flat[0].device, self.group)
+        return head.HeadStepRunner(pack, img_prototypes, batch, n_cls, mode, peer=self.peer)
+
+    def bind(self, epoch: int):
+        """Point the loss phases at the head's outputs and this epoch's temperature / logit scale (host only: the values
+        are passed by value when the phases are enqueued, so a captured graph keeps them)."""
+        r = self.runner
+        self.sl.bind(r.outs[0], r.outs[1], r.outs[2], r.own_rows(), r.logits, self.labels, self.state, epoch=epoch,
+                     max_epoch=self.tuned_epoch, logit_scale=self.logit_scale, w_clip=1.0, w_unicl=0.3)
+
+    def stage_forward(self):
+        self.runner.forward(self.image, self.text, self.state, self.text_cls)      # cls logits + the four feature outputs
+
+    def stage_loss(self, p: int):
+        self.sl.run(p)
+
+    def stage_exchange(self, p: int):
+        """All-gather ``sl.send[p]`` of every rank into ``sl.gathered[p]`` (nothing to do at world 1)."""
+        if self.world == 1:
+            return
+        if self.gather is None:
+            raise RuntimeError("DataParallelTrainStep built without exchanges: the caller performs them")
+        self.gather(p)
+
+    def stage_backward(self):
+        # the losses never touch the prototype output; with a PeerAllReduce the backward sums the gradients over the ranks
+        self.runner.backward(self.image, self.text, self.state, [self.sl.g_image, self.sl.g_text, self.sl.g_state, None],
+                             g_own_rows=self.sl.g_own)
+
+    def stage_update(self, epoch: int):
+        self.runner.advance_offset()
+        self.opt.lr = self.lr_at(epoch)
+        self.opt.step_graph([g for _, g in self.pairs])
+
+    def _body(self, epoch: int):
+        self.bind(epoch)
+        self.stage_forward()
+        n = self.sl.phases
+        for p in range(n):
+            self.stage_loss(p)
+            if p < n - 1:
+                self.stage_exchange(p)
+        self.stage_backward()
+        self.stage_update(epoch)
+
+    def step(self, epoch: int = 0):
+        """One optimisation step on the loaded shard of the global batch; returns the device tensor [total, ce, clip, unicl,
+        unicl_instance] of the GLOBAL batch (the same on every rank).  Every rank must make the same calls."""
+        if self.world > 1 and (self.gather is None or self.peer is None):
+            raise RuntimeError("DataParallelTrainStep built without exchanges: drive the stages instead of step()")
+        return super().step(epoch)
+
+    def check(self):
+        """Raise if an exchange of this rank waited past its deadline (``TEAM_PEER_TIMEOUT_S``); synchronises."""
+        for x in (self.gather, self.peer):
+            if x is not None:
+                x.check()
